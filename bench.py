@@ -2,6 +2,7 @@
 """bench.py -- GCUPS of the score-only Smith-Waterman/Gotoh hot path on B200 (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|...] [--no-extra]
+                  [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  The headline workload is BASELINE config 2:
 one 100 000 x 100 000 pair of seeded random ACGT (seed 2), parameters 1/-1/1/1, one pair per GPU (weak scaling, no
@@ -21,8 +22,14 @@ and, unless --no-extra, two sub-records measured in the same run on the same N G
   batch      BASELINE config 4: 10 M read/window pairs generated in HBM by the seeded device generator, sharded
              pair-wise over the N GPUs (strong scaling, no communication), a sample checked against the oracle and a
              64-bit checksum over all scores that is the same for every N
+Every timed loop, the sub-records' and the end-to-end host-call figures' included, runs --steps times (after --warmup
+untimed steps; at least 3 for pairs and batches, 1 for the ring); the e2e figures are per call.
 --workload cfg1|n1m|ring400k|ring1m|cfg3|cfg4|cfg5 makes that workload the line itself.
 --impl reference runs only the reference's CPU path, as the reference arm.
+--dump-outputs DIR writes, after the timed steps, the scores the timed path returned in its last step: one
+DIR/<workload>_scores.npy per record (float64 for single pairs, float32 for batches, exact for every score these
+workloads reach), with a .rank<r> suffix when several ranks run.  Inputs are seeded, so two builds of the project
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -127,6 +134,18 @@ class ClockSampler(threading.Thread):
         s = sorted(self.samples)
         return {"sm_mhz": s[len(s) // 2] if s else None, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons),
                 "samples": len(s)}
+
+
+def dump_outputs(args, env, name, values, dtype):
+    """--dump-outputs: the scores of the last timed step of one record as DIR/<name>_scores[.rank<r>].npy."""
+    if not args.dump_outputs:
+        return
+    out = np.asarray(values, dtype=dtype)
+    if not np.array_equal(out, np.asarray(values)):
+        raise SystemExit(f"bench.py: {name} scores are not exact in {np.dtype(dtype).name}")
+    d = Path(args.dump_outputs)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / f"{name}_scores{'' if env.world == 1 else f'.rank{env.rank}'}.npy", out)
 
 
 def peak_gcups(f_mhz, vwidth, gpus=1):
@@ -284,6 +303,7 @@ def pair_record(env, args, name):
         check(s, "device")
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    dump_outputs(args, env, name, s, np.float64)
     dev_ms = sum(e0.elapsed_time(e1) for e0, e1 in ev)
     # end to end through the host-buffer call of the reference harness (TestFileWithGPU.cpp:92):
     # H2D of both sequences + encode + wavefront kernel + D2H of the result, wall clock per call
@@ -364,6 +384,7 @@ def ring_record(env, args, name, steps, warmup):
     e1.record(stream)
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    dump_outputs(args, env, name, [scores[-1]], np.float64)
     # end to end: every step copies both sequences from pinned host memory and reads the score back
     a_p, b_p = torch.from_numpy(a_h.copy()).pin_memory(), torch.from_numpy(b_h.copy()).pin_memory()
     dist.barrier()
@@ -478,6 +499,7 @@ def batch_record(env, args, name, steps, warmup):
     dev_ms = e0.elapsed_time(e1)
     if checksum() != chk:
         raise SystemExit("bench.py: batch checksum changed between passes")
+    dump_outputs(args, env, name, scores.cpu().numpy(), np.float32)    # cfg4: 10 M pairs, 40 MB
     # end to end from HOST bytes: H2D of the sequences, pack, kernel, D2H of the scores, through the C ABI host call
     ne = min(npairs, 2500000 if not banded else 250000)
     r_e, w_e = seq1[:ne].cpu().pin_memory().numpy().reshape(-1), seq2[:ne].cpu().pin_memory().numpy().reshape(-1)
@@ -494,8 +516,9 @@ def batch_record(env, args, name, steps, warmup):
     out = host_call() if ne else np.zeros(0, dtype=np.int32)
     env.barrier()
     t1 = time.perf_counter()
-    out = host_call() if ne else out
-    e2e_s = time.perf_counter() - t1
+    for _ in range(steps):
+        out = host_call() if ne else out
+    e2e_s = (time.perf_counter() - t1) / steps      # per call
     if out.tolist() != scores[:ne].cpu().numpy().tolist():
         raise SystemExit("bench.py: host batch call disagrees with the device-resident pass")
     # the same call with the host batch already in the resident 2-bit format (a quarter of the PCIe bytes, no pack kernel)
@@ -514,8 +537,9 @@ def batch_record(env, args, name, steps, warmup):
         packed_call()
         env.barrier()
         t1 = time.perf_counter()
-        outp = packed_call()
-        e2e_packed_s = time.perf_counter() - t1
+        for _ in range(steps):
+            outp = packed_call()
+        e2e_packed_s = (time.perf_counter() - t1) / steps      # per call
         if outp.tolist() != out[:np_pk].tolist():
             raise SystemExit("bench.py: packed host batch call disagrees with the byte call")
     dev_ms, e2e_ms, k_ms, e2e_packed_ms = env.max_over_ranks([dev_ms, e2e_s * 1e3, float(np.mean(kms)), e2e_packed_s * 1e3])
@@ -584,8 +608,8 @@ def run_ours(args):
         line = pair_record(env, args, name)
         if name == "cfg2" and not args.no_extra:
             # the two multi-GPU designs of BASELINE configs 3 and 4 on the same N GPUs, in the same run
-            ring = ring_record(env, args, "cfg3", 2, 1)
-            batch = batch_record(env, args, "cfg4", 3, 3)
+            ring = ring_record(env, args, "cfg3", args.steps, args.warmup)
+            batch = batch_record(env, args, "cfg4", args.steps, args.warmup)
             if env.rank == 0:
                 line["ring"] = ring
                 line["batch"] = batch
@@ -607,7 +631,13 @@ def main():
     ap.add_argument("--one-sided", action="store_true", help="ring workloads: never sweep from both ends")
     ap.add_argument("--no-linear", action="store_true",
                     help="keep the general affine kernel although GAP_INIT == GAP_EXT (default: use the exact E/F-free kernel)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the scores the timed path returned in its last step as DIR/<workload>_scores.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has nothing to dump")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -121,5 +121,42 @@ def main(big: bool):
     print(f"parameterised fixtures: {len(pcases)} cases, lazy != main in {ndiff}")
 
 
+def fresh_inputs():
+    """The 25 seeded pairs of tests/test_oracle.py::test_oracle_equals_live_reference_on_fresh_inputs."""
+    for k in range(25):
+        n, m = 1 + int(rng.mix64(41, 1, k) % 700), 1 + int(rng.mix64(41, 2, k) % 700)
+        a, b = rng.random_acgt(41, 2 * k, n), rng.random_acgt(41, 2 * k + 1, m)
+        if k % 4 == 0:
+            b = rng.mutate(a, 41, 900 + k, 0.07, 0.03)
+        yield a, b
+
+
+HARNESS_SEED, HARNESS_LENGTHS, HARNESS_TESTS = 8, (1, 50, 500, 1000, 3000), 10
+
+
+def harness_inputs():
+    """The pairs harness/test_runner_b200 scores with seed 8 at these lengths (its random_sequence = rng.random_acgt)."""
+    for n in HARNESS_LENGTHS:
+        for it in range(HARNESS_TESTS):
+            yield rng.random_acgt(HARNESS_SEED, 2 * it, n), rng.random_acgt(HARNESS_SEED, 2 * it + 1, n)
+
+
+def live():
+    """(5) ref_scores_live.json: the scores of the reference's three CPU functions (SmithWatermanScore, LazySmith,
+    ParallelLazySmith_threads) on the inputs that tests/test_oracle.py and tests/test_gpu_dropin.py otherwise compare
+    with the reference live.  Needs oracle/_ref/libref.so."""
+    assert O.ref_available(), "needs oracle/_ref/libref.so"
+    fns = ("ref_SmithWatermanScore", "ref_LazySmith", "ref_ParallelLazySmith_threads")
+    out = {"functions": list(fns),
+           "fresh": [[O.ref_call(f, a, b) for f in fns] for a, b in fresh_inputs()],
+           "harness": {"seed": HARNESS_SEED, "lengths": list(HARNESS_LENGTHS), "tests": HARNESS_TESTS,
+                       "scores": [[O.ref_call(f, a, b) for f in fns] for a, b in harness_inputs()]}}
+    (HERE / "ref_scores_live.json").write_text(json.dumps(out) + "\n")
+    print(f"live-comparison fixtures: {len(out['fresh'])} fresh pairs, {len(out['harness']['scores'])} harness pairs")
+
+
 if __name__ == "__main__":
-    main(big="--big" in sys.argv)
+    if "--live" in sys.argv:
+        live()
+    else:
+        main(big="--big" in sys.argv)

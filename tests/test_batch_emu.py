@@ -18,14 +18,15 @@ pytestmark = pytest.mark.skipif(shutil.which("nvcc") is None, reason="nvcc not a
 
 
 @pytest.fixture(scope="module")
-def emu():
+def emu(tmp_path_factory):
     src = EMU_DIR / "batch_emu.cu"
     hdrs = list((EMU_DIR.parent.parent / "concurrentproject_b200" / "csrc").glob("swb_*.cuh"))
     if not EMU.exists() or EMU.stat().st_mtime < max(p.stat().st_mtime for p in [src] + hdrs):
         subprocess.run(["nvcc", "-O1", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-o", str(EMU), str(src),
                         "-lpthread"], check=True, cwd=EMU_DIR)
+    work = tmp_path_factory.mktemp("batch_emu")       # per run: concurrent runs and other users do not collide
 
-    def run(s1, s2, kind, R, mode, G, p=O.DEFAULT, band_lo=-32, tmp=Path("/tmp")):
+    def run(s1, s2, kind, R, mode, G, p=O.DEFAULT, band_lo=-32, tmp=work):
         f = tmp / "swb_batch_emu.bin"
         with open(f, "wb") as out:
             out.write(struct.pack("<i", len(s1)))

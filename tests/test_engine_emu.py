@@ -20,14 +20,15 @@ pytestmark = pytest.mark.skipif(shutil.which("nvcc") is None, reason="nvcc not a
 
 
 @pytest.fixture(scope="module")
-def emu():
+def emu(tmp_path_factory):
     src = EMU_DIR / "engine_emu.cu"
     hdrs = list((EMU_DIR.parent.parent / "concurrentproject_b200" / "csrc").glob("swb_*.cuh"))
     if not EMU.exists() or EMU.stat().st_mtime < max(p.stat().st_mtime for p in [src] + hdrs):
         subprocess.run(["nvcc", "-O1", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-o", str(EMU),
                         str(src), "-lpthread"], check=True, cwd=EMU_DIR)
+    work = tmp_path_factory.mktemp("engine_emu")      # per run: concurrent runs and other users do not collide
 
-    def run(q, t, R, mode, slack, W, G, p=O.DEFAULT, link_len=4096, epoch=5, tmp=Path("/tmp"), final_row=False, short=None, hs=False):
+    def run(q, t, R, mode, slack, W, G, p=O.DEFAULT, link_len=4096, epoch=5, tmp=work, final_row=False, short=None, hs=False):
         qf, tf, ff = tmp / "swb_emu_q.bin", tmp / "swb_emu_t.bin", tmp / "swb_emu_final.bin"
         qf.write_bytes(bytes(q)); tf.write_bytes(bytes(t))
         ma, mi, gi, ge = p
