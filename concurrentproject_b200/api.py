@@ -184,6 +184,24 @@ class Context:
             raise SwbError(rc, "swb200_score_end_device")
         return out.value, ie.value, je.value
 
+    def align_device(self, d_seq1: int, n: int, d_seq2: int, m: int, params: Sequence[int] = DEFAULT_PARAMS, *,
+                     stream: int = 0):
+        """align for sequences resident in HBM (swb200_align_device): (score, span, cigar) as align returns them."""
+        out, need = C.c_int(0), C.c_longlong(0)
+        span = (C.c_longlong * 4)()
+        p = _params(params)
+        cap = 64
+        while True:
+            buf = C.create_string_buffer(cap)
+            rc = _lib.load().swb200_align_device(self.handle, C.c_void_p(d_seq1), n, C.c_void_p(d_seq2), m, C.byref(p),
+                                                 C.c_void_p(stream), C.byref(out), span, buf, cap, C.byref(need))
+            if rc == -2 and need.value + 1 > cap:            # buffer too small: the call says how much it needs
+                cap = need.value + 1
+                continue
+            if rc != 0:
+                raise SwbError(rc, "swb200_align_device")
+            return out.value, tuple(int(x) for x in span), buf.value.decode()
+
     def last_run(self) -> dict:
         return last_run(self)
 
@@ -289,6 +307,17 @@ class PackedBatch:
                                                    C.c_void_p(d_scores))
         if rc != 0:
             raise SwbError(rc, "swb200_batch_score_banded")
+
+    def align(self, d_scores: int, d_spans: int, d_ops: int, ops_stride: int, d_ops_count: int,
+              params: Sequence[int] = DEFAULT_PARAMS, *, stream: int = 0) -> None:
+        """Score, span and alignment operations of every pair (swb200_batch_align; the batch must be packed with
+        keep_order=False).  Device outputs: int32 scores[n], int32 spans[n, 4], uint32 ops[n, ops_stride] (count << 4 | op,
+        BAM numbering), int32 ops_count[n] (-(count) where ops_stride was too small)."""
+        p = _params(params)
+        rc = _lib.load().swb200_batch_align(self.handle, C.byref(p), None, C.c_void_p(stream), C.c_void_p(d_scores),
+                                            C.c_void_p(d_spans), C.c_void_p(d_ops), ops_stride, C.c_void_p(d_ops_count))
+        if rc != 0:
+            raise SwbError(rc, "swb200_batch_align")
 
     def close(self):
         if self.handle:
@@ -423,3 +452,53 @@ def score_banded_batch_packed(w1: np.ndarray, stride1: int, w2: np.ndarray, stri
     if rc != 0:
         raise SwbError(rc, "swb200_score_banded_batch_packed")
     return out
+
+
+# ---- batch alignment (swb200_align_batch) ----------------------------------------------------------------------------
+OPS_STRIDE = 96          # operations per pair in the first attempt: a planted 150-base read needs ~10; on 1 M cfg4 pairs 28 %
+                         # (unrelated reads, long gap-rich local alignments) need more and are redone by align_batch
+_OP_CHARS = {1: "I", 2: "D", 7: "=", 8: "X"}
+
+
+def cigar_string(ops) -> str:
+    """The extended CIGAR of a row of operations (count << 4 | op, BAM numbering), in align's format."""
+    return "".join(f"{int(w) >> 4}{_OP_CHARS[int(w) & 15]}" for w in ops)
+
+
+def align_batch_ops(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray, flat2: np.ndarray, off2: np.ndarray, len2: np.ndarray,
+                    params: Sequence[int] = DEFAULT_PARAMS, ops_stride: int = OPS_STRIDE):
+    """swb200_align_batch on flattened HOST arrays: (scores int32[n], spans int32[n, 4], ops uint32[n, ops_stride],
+    ops_count int32[n]); ops_count[k] < 0 where pair k needed more than ops_stride operations."""
+    n = len(len1)
+    scores = np.zeros(n, dtype=np.int32)
+    spans = np.zeros((n, 4), dtype=np.int32)
+    ops = np.zeros((n, ops_stride), dtype=np.uint32)
+    cnt = np.zeros(n, dtype=np.int32)
+    p = _params(params)
+    LL, I = C.POINTER(C.c_longlong), C.POINTER(C.c_int)
+    rc = _lib.load().swb200_align_batch(_ptr(flat1), off1.ctypes.data_as(LL), len1.ctypes.data_as(I), _ptr(flat2),
+                                        off2.ctypes.data_as(LL), len2.ctypes.data_as(I), n, C.byref(p), None,
+                                        scores.ctypes.data_as(I), spans.ctypes.data_as(I),
+                                        ops.ctypes.data_as(C.POINTER(C.c_uint)), ops_stride, cnt.ctypes.data_as(I))
+    if rc != 0:
+        raise SwbError(rc, "swb200_align_batch")
+    return scores, spans, ops, cnt
+
+
+def align_batch(seqs1, seqs2, params: Sequence[int] = DEFAULT_PARAMS, *, ops_stride: int = OPS_STRIDE):
+    """(scores int32[n], spans int32[n, 4], cigars list[str]): align(seqs1[k], seqs2[k]) for every pair, in one batch call
+    (swb200_align_batch; the limits of score_batch).  Pairs whose alignment needs more than ops_stride operations are
+    aligned again in a second batch with room for len1 + len2 operations, which always suffices."""
+    if len(seqs1) != len(seqs2):
+        raise ValueError("seqs1 and seqs2 differ in length")
+    f1, o1, l1 = _flatten(seqs1)
+    f2, o2, l2 = _flatten(seqs2)
+    scores, spans, ops, cnt = align_batch_ops(f1, o1, l1, f2, o2, l2, params, ops_stride)
+    cigars = [cigar_string(ops[k, :c]) if c >= 0 else None for k, c in enumerate(cnt.tolist())]
+    redo = np.flatnonzero(cnt < 0)
+    if len(redo):
+        stride = int((l1[redo].astype(np.int64) + l2[redo]).max())
+        _, _, ops2, cnt2 = align_batch_ops(f1, o1[redo].copy(), l1[redo].copy(), f2, o2[redo].copy(), l2[redo].copy(), params, stride)
+        for r, k in enumerate(redo.tolist()):
+            cigars[k] = cigar_string(ops2[r, :cnt2[r]])
+    return scores, spans, cigars

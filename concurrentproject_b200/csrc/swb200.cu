@@ -11,6 +11,7 @@
 #include "swb_chain.cuh"
 #include "swb_batch.cuh"
 #include "swb_banded.cuh"
+#include "swb_align_batch.cuh"
 
 #include <cstdio>
 #include <cstdlib>
@@ -271,6 +272,15 @@ struct swb200_ctx {
   uint64_t* hb_tw = nullptr; size_t hb_tw_cap = 0;
   int* hb_ql = nullptr; size_t hb_ql_cap = 0;
   int* hb_tl = nullptr; size_t hb_tl_cap = 0;
+  // batch alignment (swb200_align_batch / swb200_batch_align), grow-only
+  int2* ab_col = nullptr; size_t ab_col_cap = 0;          // per-thread column buffers
+  uint64_t* ab_slot = nullptr; size_t ab_slot_cap = 0;    // per-thread direction slots
+  uint64_t* ab_pool = nullptr; size_t ab_pool_cap = 0;    // shared direction pool (allocated only when a rectangle needs it)
+  int* ab_list = nullptr; size_t ab_list_cap = 0;         // two pending lists
+  unsigned long long* ab_misc = nullptr; size_t ab_misc_cap = 0;   // [0] err | npending << 32, [1] pool words used, [2] cells
+  int* hb_spans = nullptr; size_t hb_spans_cap = 0;       // host batch alignment: outputs before the copy back
+  uint32_t* hb_ops = nullptr; size_t hb_ops_cap = 0;
+  int* hb_opsn = nullptr; size_t hb_opsn_cap = 0;
 };
 
 namespace swb {
@@ -291,6 +301,7 @@ struct swb200_batch {
   uint64_t* t_words = nullptr;
   int* q_len = nullptr;
   int* t_len = nullptr;
+  int* len1 = nullptr;         // keep_order = 0: the caller's seq1 lengths (which pairs were swapped; swb200_batch_align)
   long long cells = 0;
 };
 
@@ -1027,6 +1038,8 @@ void swb200_ctx_destroy(swb200_ctx* c) {
   cudaFree(c->d_dirs); cudaFree(c->d_ops); cudaFree(c->d_prof); cudaFree(c->d_progress); cudaFree(c->d_cand); cudaFree(c->d_rev); cudaFree(c->d_result); cudaFree(c->d_lut);
   cudaFree(c->hb_seq1); cudaFree(c->hb_seq2); cudaFree(c->hb_off1); cudaFree(c->hb_off2); cudaFree(c->hb_len1); cudaFree(c->hb_len2);
   cudaFree(c->hb_scores); cudaFree(c->hb_qw); cudaFree(c->hb_tw); cudaFree(c->hb_ql); cudaFree(c->hb_tl);
+  cudaFree(c->ab_col); cudaFree(c->ab_slot); cudaFree(c->ab_pool); cudaFree(c->ab_list); cudaFree(c->ab_misc);
+  cudaFree(c->hb_spans); cudaFree(c->hb_ops); cudaFree(c->hb_opsn);
   if (c->h_result) cudaFreeHost(c->h_result);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
@@ -1332,6 +1345,7 @@ static int batch_pack_impl(swb200_ctx* c, const unsigned char* d_seq1, const lon
     SWB_CUDA(cudaMalloc(&b->t_words, np * b->t_stride * sizeof(uint64_t)));
     SWB_CUDA(cudaMalloc(&b->q_len, np * sizeof(int)));
     SWB_CUDA(cudaMalloc(&b->t_len, np * sizeof(int)));
+    if (!keep_order) SWB_CUDA(cudaMalloc(&b->len1, np * sizeof(int)));
   }
   SWB_CUDA(cudaMemsetAsync(c->d_result, 0, 12 * sizeof(int), s));    // [0] score, [1] status, [3..8] timeout post-mortem, [11] protocol-checker mismatches
   if (npairs > 0) {
@@ -1340,6 +1354,7 @@ static int batch_pack_impl(swb200_ctx* c, const unsigned char* d_seq1, const lon
     swb::launch_pack_batch(d_seq1, d_off1, d_len1, d_seq2, d_off2, d_len2, npairs, b->q_stride, b->t_stride, b->q_words,
                            b->t_words, b->q_len, b->t_len, b->keep_order, c->d_result, blocks, s);
     SWB_CUDA(cudaGetLastError());
+    if (b->len1) SWB_CUDA(cudaMemcpyAsync(b->len1, d_len1, (size_t)npairs * sizeof(int), cudaMemcpyDeviceToDevice, s));
   }
   SWB_CUDA(cudaMemcpyAsync(c->h_result, c->d_result, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
   SWB_CUDA(cudaStreamSynchronize(s));
@@ -1511,7 +1526,7 @@ void swb200_batch_free(swb200_batch* b) {
   if (!b) return;
   DeviceGuard guard;
   cudaSetDevice(b->ctx->device);
-  if (!b->pooled) { cudaFree(b->q_words); cudaFree(b->t_words); cudaFree(b->q_len); cudaFree(b->t_len); }
+  if (!b->pooled) { cudaFree(b->q_words); cudaFree(b->t_words); cudaFree(b->q_len); cudaFree(b->t_len); cudaFree(b->len1); }
   delete b;
 }
 
@@ -2325,6 +2340,243 @@ int swb200_set_devices(int count) {
 int swb200_get_devices(void) {
   std::lock_guard<std::mutex> pl(g_pool.mu);
   return std::max<int>(1, (int)g_pool.ctx.size());
+}
+
+}  // extern "C"
+
+// ---- batch alignment: score, span and CIGAR for every pair (swb_align_batch.cuh) ----------------------------------
+namespace {
+
+constexpr long long kAlignSlotWords = 2048;        // direction slot per thread: 2048 x 16 cells (a 150-base read's span: ~1 500)
+constexpr long long kAlignPoolWords = 32LL << 20;  // shared pool for larger rectangles: 256 MB, or the largest rectangle if more
+
+// The limits of swb200_score_batch, checked on the host before any device is touched.
+int check_align_batch_limits(const swb200_params& p, int max_short) {
+  if (max_short > 1024)
+    return fail(SWB200_ERR_ARG, "batch alignment needs min(len1,len2) <= 1024 per pair; use swb200_align for long pairs");
+  if ((long long)p.match * max_short > 32767 - p.match - 1)
+    return fail(SWB200_ERR_RANGE, "match * min(len) is outside the batch limits; use swb200_align for such pairs");
+  return SWB200_OK;
+}
+
+// Passes 1-3 and the walk over a packed range (shorter sequence first, len1 = the caller's seq1 lengths), everything on
+// stream s of c's device.  Synchronises once per trace round (the pending count decides whether another round runs).
+int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, const swb200_params& p, cudaStream_t s,
+                        int* d_scores, int* d_spans, uint32_t* d_ops, int ops_stride, int* d_ops_count, swb200_run_info* info) {
+  if (v.npairs == 0) return SWB200_OK;
+  const long long blocks = std::max(1LL, std::min<long long>((v.npairs + 255) / 256, 2LL * c->sms));
+  const long long nt = blocks * 256;
+  int rc;
+  if ((rc = grow(c->ab_col, c->ab_col_cap, (size_t)(v.max_short + 1) * nt, false, s)) ||
+      (rc = grow(c->ab_slot, c->ab_slot_cap, (size_t)(kAlignSlotWords * nt), false, s)) ||
+      (rc = grow(c->ab_list, c->ab_list_cap, 2 * (size_t)v.npairs, false, s)) ||
+      (rc = grow(c->ab_misc, c->ab_misc_cap, 4, false, s))) return rc;
+  SWB_CUDA(cudaMemsetAsync(c->ab_misc, 0, 3 * sizeof(unsigned long long), s));
+  swb::AlignBatchParams P{};
+  P.q_words = v.q_words; P.t_words = v.t_words; P.q_len = v.q_len; P.t_len = v.t_len; P.len1 = d_len1;
+  P.q_stride = v.q_stride; P.t_stride = v.t_stride; P.npairs = v.npairs;
+  P.match = p.match; P.mismatch = p.mismatch; P.gap_init = p.gap_init; P.gap_ext = p.gap_ext;
+  P.scores = d_scores; P.spans = d_spans; P.col = c->ab_col; P.nthreads = nt;
+  P.slot = c->ab_slot; P.slot_words = kAlignSlotWords; P.pool = c->ab_pool; P.pool_words = (long long)c->ab_pool_cap;
+  P.pool_used = c->ab_misc + 1;
+  P.todo = nullptr; P.ntodo = v.npairs;
+  P.pending = c->ab_list; P.npending = reinterpret_cast<int*>(c->ab_misc) + 1;
+  P.ops = d_ops; P.ops_stride = ops_stride; P.ops_count = d_ops_count;
+  P.err = reinterpret_cast<int*>(c->ab_misc); P.cells = c->ab_misc + 2;
+  swb::launch_align_span(P, (int)blocks, s);
+  swb::launch_align_trace(P, (int)blocks, s);
+  SWB_CUDA(cudaGetLastError());
+  info->engine_launches += 2;
+  for (int cur = 0;;) {
+    unsigned long long h[3] = {0, 0, 0};
+    SWB_CUDA(cudaMemcpyAsync(h, c->ab_misc, sizeof h, cudaMemcpyDeviceToHost, s));
+    SWB_CUDA(cudaStreamSynchronize(s));
+    const int err = (int)(uint32_t)h[0], npend = (int)(h[0] >> 32);
+    if (err & swb::kAlignErrStart) return fail(SWB200_ERR_CUDA, "internal: anchored pass does not reproduce the score");
+    if (err & swb::kAlignErrTrace) return fail(SWB200_ERR_CUDA, "internal: the traceback pass does not reproduce the score");
+    if (err) return fail(SWB200_ERR_CUDA, "internal: the alignment does not re-score to the score");
+    if (npend == 0) { info->cells += (long long)h[2]; return SWB200_OK; }
+    // rectangles larger than a slot: the pool, emptied for every round; its first taker always fits
+    const size_t need = (size_t)std::max(kAlignPoolWords, swb::align_dir_words(v.max_long, v.max_short));
+    if ((rc = grow(c->ab_pool, c->ab_pool_cap, need, false, s))) return rc;
+    P.pool = c->ab_pool; P.pool_words = (long long)c->ab_pool_cap;
+    P.todo = c->ab_list + (size_t)cur * v.npairs; P.ntodo = npend;
+    cur ^= 1;
+    P.pending = c->ab_list + (size_t)cur * v.npairs;
+    SWB_CUDA(cudaMemsetAsync(c->ab_misc, 0, 2 * sizeof(unsigned long long), s));
+    swb::launch_align_trace(P, (int)std::max(1LL, std::min<long long>(blocks, (npend + 255) / 256)), s);
+    SWB_CUDA(cudaGetLastError());
+    info->engine_launches += 1;
+  }
+}
+
+}  // namespace
+
+// One context's share of a host batch alignment (arguments checked by the caller).  Copy and pack in chunks as
+// score_batch_host_ctx does, then the passes over the whole range, then the outputs back.
+static int align_batch_host_ctx(swb200_ctx* c, const unsigned char* seq1_all, const long long* off1, const int* len1,
+                                const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                                const swb200_params& pv, int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride,
+                                int* ops_count) {
+  if (npairs == 0) return SWB200_OK;
+  long long bytes1 = 0, bytes2 = 0, base1 = LLONG_MAX, base2 = LLONG_MAX;
+  int max_short = 0, max_long = 0;
+  for (long long k = 0; k < npairs; ++k) {
+    const int a = len1[k], b = len2[k];
+    bytes1 = std::max(bytes1, off1[k] + a); bytes2 = std::max(bytes2, off2[k] + b);
+    base1 = std::min(base1, off1[k]); base2 = std::min(base2, off2[k]);
+    max_short = std::max(max_short, std::min(a, b)); max_long = std::max(max_long, std::max(a, b));
+  }
+  base1 &= ~15LL; base2 &= ~15LL;
+  bytes1 -= base1; bytes2 -= base2;
+  std::lock_guard<std::mutex> lk(c->mu);
+  DeviceGuard guard;
+  SWB_CUDA(cudaSetDevice(c->device));
+  cudaStream_t sc = c->own_stream, sk = c->aux_stream;
+  const size_t np = (size_t)npairs;
+  const long long q_stride = std::max(1, (max_short + 31) / 32);
+  const long long t_stride = std::max(1, (max_long + 31) / 32) + 2;
+  int rc;
+  if ((rc = grow(c->hb_seq1, c->hb_seq1_cap, (size_t)bytes1 + 16, false, sc)) || (rc = grow(c->hb_seq2, c->hb_seq2_cap, (size_t)bytes2 + 16, false, sc)) ||
+      (rc = grow(c->hb_off1, c->hb_off1_cap, np, false, sc)) || (rc = grow(c->hb_off2, c->hb_off2_cap, np, false, sc)) ||
+      (rc = grow(c->hb_len1, c->hb_len1_cap, np, false, sc)) || (rc = grow(c->hb_len2, c->hb_len2_cap, np, false, sc)) ||
+      (rc = grow(c->hb_scores, c->hb_scores_cap, np, false, sc)) || (rc = grow(c->hb_spans, c->hb_spans_cap, 4 * np, false, sc)) ||
+      (rc = grow(c->hb_ops, c->hb_ops_cap, np * (size_t)ops_stride, false, sc)) || (rc = grow(c->hb_opsn, c->hb_opsn_cap, np, false, sc)) ||
+      (rc = grow(c->hb_qw, c->hb_qw_cap, np * q_stride, false, sc)) || (rc = grow(c->hb_tw, c->hb_tw_cap, np * t_stride, false, sc)) ||
+      (rc = grow(c->hb_ql, c->hb_ql_cap, np, false, sc)) || (rc = grow(c->hb_tl, c->hb_tl_cap, np, false, sc))) return rc;
+  c->info = swb200_run_info{};
+  SWB_CUDA(cudaMemsetAsync(c->d_result, 0, 10 * sizeof(int), sc));
+  SWB_CUDA(cudaMemcpyAsync(c->hb_off1, off1, np * sizeof(long long), cudaMemcpyHostToDevice, sc));
+  SWB_CUDA(cudaMemcpyAsync(c->hb_off2, off2, np * sizeof(long long), cudaMemcpyHostToDevice, sc));
+  SWB_CUDA(cudaMemcpyAsync(c->hb_len1, len1, np * sizeof(int), cudaMemcpyHostToDevice, sc));
+  SWB_CUDA(cudaMemcpyAsync(c->hb_len2, len2, np * sizeof(int), cudaMemcpyHostToDevice, sc));
+  // chunks of ~48 MB of sequence: own_stream copies chunk k+1 while aux_stream packs chunk k
+  size_t ci = 0;
+  bool first = true;
+  const long long forced = settings().batch_chunk_bytes;
+  const long long target = forced > 0 ? forced : 48LL << 20, min_pairs = forced > 0 ? 1 : 1024;
+  long long k0 = 0, acc = 0, lo1 = LLONG_MAX, hi1 = 0, lo2 = LLONG_MAX, hi2 = 0;
+  for (long long k = 0; k < npairs; ++k) {
+    lo1 = std::min(lo1, off1[k]); hi1 = std::max(hi1, off1[k] + len1[k]);
+    lo2 = std::min(lo2, off2[k]); hi2 = std::max(hi2, off2[k] + len2[k]);
+    acc += (long long)len1[k] + len2[k];
+    if (!((acc >= target && k + 1 - k0 >= min_pairs) || k + 1 == npairs)) continue;
+    while (c->chunk_events.size() < ci + 1) {
+      cudaEvent_t e;
+      SWB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+      c->chunk_events.push_back(e);
+    }
+    if (hi1 > lo1) SWB_CUDA(cudaMemcpyAsync(c->hb_seq1 + (lo1 - base1), seq1_all + lo1, (size_t)(hi1 - lo1), cudaMemcpyHostToDevice, sc));
+    if (hi2 > lo2) SWB_CUDA(cudaMemcpyAsync(c->hb_seq2 + (lo2 - base2), seq2_all + lo2, (size_t)(hi2 - lo2), cudaMemcpyHostToDevice, sc));
+    SWB_CUDA(cudaEventRecord(c->chunk_events[ci], sc));
+    SWB_CUDA(cudaStreamWaitEvent(sk, c->chunk_events[ci], 0));
+    ci += 1;
+    if (first) { SWB_CUDA(cudaEventRecord(c->ev0, sk)); first = false; }
+    const long long nk = k + 1 - k0;
+    const int blocks = (int)std::min<long long>((nk * (q_stride + t_stride) + 255) / 256, 64LL * c->sms);
+    swb::launch_pack_batch(c->hb_seq1 - base1, c->hb_off1 + k0, c->hb_len1 + k0, c->hb_seq2 - base2, c->hb_off2 + k0, c->hb_len2 + k0, nk,
+                           q_stride, t_stride, c->hb_qw + k0 * q_stride, c->hb_tw + k0 * t_stride, c->hb_ql + k0, c->hb_tl + k0, 0,
+                           c->d_result, blocks, sk);
+    SWB_CUDA(cudaGetLastError());
+    c->info.aux_launches += 1;
+    k0 = k + 1; acc = 0; lo1 = LLONG_MAX; hi1 = 0; lo2 = LLONG_MAX; hi2 = 0;
+  }
+  SWB_CUDA(cudaMemcpyAsync(c->h_result, c->d_result, 2 * sizeof(int), cudaMemcpyDeviceToHost, sk));
+  SWB_CUDA(cudaStreamSynchronize(sk));
+  SWB_CUDA(cudaStreamSynchronize(sc));
+  if (c->h_result[1] & swb::STATUS_BAD_SYMBOL) return fail(SWB200_ERR_ALPHABET, "batch input contains bytes other than A,C,G,T");
+  const BatchView v{c->hb_qw, c->hb_tw, c->hb_ql, c->hb_tl, q_stride, t_stride, npairs, max_short, max_long};
+  SWB_CUDA(cudaMemsetAsync(c->hb_ops, 0, np * (size_t)ops_stride * sizeof(uint32_t), sk));   // overflowed pairs come back as zeros
+  if ((rc = align_packed_locked(c, v, c->hb_len1, pv, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info))) return rc;
+  SWB_CUDA(cudaEventRecord(c->ev1, sk));
+  SWB_CUDA(cudaMemcpyAsync(scores_out, c->hb_scores, np * sizeof(int), cudaMemcpyDeviceToHost, sk));
+  SWB_CUDA(cudaMemcpyAsync(spans_out, c->hb_spans, 4 * np * sizeof(int), cudaMemcpyDeviceToHost, sk));
+  SWB_CUDA(cudaMemcpyAsync(ops_count, c->hb_opsn, np * sizeof(int), cudaMemcpyDeviceToHost, sk));
+  SWB_CUDA(cudaMemcpyAsync(ops_out, c->hb_ops, np * (size_t)ops_stride * sizeof(uint32_t), cudaMemcpyDeviceToHost, sk));
+  SWB_CUDA(cudaStreamSynchronize(sk));
+  float ms = 0;
+  SWB_CUDA(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+  c->info.engine_ms = ms;          // first pack to the last trace round
+  c->info.lanes = 32; c->info.config = 300; c->info.rows = swb::kAlignStrip;
+  return SWB200_OK;
+}
+
+extern "C" {
+
+int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, const int* len1, const unsigned char* seq2_all,
+                       const long long* off2, const int* len2, long long npairs, const swb200_params* p, const swb200_options* opt,
+                       int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride, int* ops_count) {
+  (void)opt;
+  if (npairs < 0 || ops_stride < 1 ||
+      (npairs > 0 && (!seq1_all || !seq2_all || !off1 || !off2 || !len1 || !len2 || !scores_out || !spans_out || !ops_out || !ops_count)))
+    return fail(SWB200_ERR_ARG, "bad batch arguments");
+  const swb200_params pv = p ? *p : swb200_params{1, -1, 1, 1};
+  int rc;
+  {
+    long long neg = 0;
+    int mxmin = 0;
+    for (long long k = 0; k < npairs; ++k) {
+      neg |= (long long)(len1[k] | len2[k]) | off1[k] | off2[k];
+      mxmin = std::max(mxmin, std::min(len1[k], len2[k]));
+    }
+    if (neg < 0) return fail(SWB200_ERR_ARG, "negative length or offset");
+    if ((rc = check_params(pv)) || (rc = check_align_batch_limits(pv, mxmin))) return rc;
+  }
+  if (npairs == 0) return SWB200_OK;
+  {
+    std::unique_lock<std::mutex> pl(g_pool.mu);
+    const int G = (int)g_pool.ctx.size();
+    if (G > 1 && npairs >= 2LL * G) {
+      // contiguous ranges of pairs, one per GPU, as swb200_score_batch
+      const long long per = (npairs + G - 1) / G;
+      rc = pool_parallel(G, [&](int g) -> int {
+        const long long k0 = std::min<long long>(npairs, (long long)g * per), k1 = std::min<long long>(npairs, k0 + per);
+        return align_batch_host_ctx(g_pool.ctx[(size_t)g], seq1_all, off1 + k0, len1 + k0, seq2_all, off2 + k0, len2 + k0, k1 - k0, pv,
+                                    scores_out + k0, spans_out + 4 * k0, ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
+      });
+      if (rc) return rc;
+      g_pool.info = g_pool.ctx[0]->info;
+      g_pool.info.cells = 0; g_pool.info.engine_ms = 0; g_pool.info.engine_launches = 0; g_pool.info.aux_launches = 0;
+      for (int g = 0; g < G; ++g) {
+        const swb200_run_info& gi = g_pool.ctx[(size_t)g]->info;
+        g_pool.info.cells += gi.cells; g_pool.info.engine_ms = std::max(g_pool.info.engine_ms, gi.engine_ms);
+        g_pool.info.engine_launches += gi.engine_launches; g_pool.info.aux_launches += gi.aux_launches;
+      }
+      g_pool.info_valid = true;
+      return SWB200_OK;
+    }
+    g_pool.info_valid = false;
+  }
+  swb200_ctx* c = nullptr;
+  if ((rc = default_ctx(&c))) return rc;
+  return align_batch_host_ctx(c, seq1_all, off1, len1, seq2_all, off2, len2, npairs, pv, scores_out, spans_out, ops_out, ops_stride, ops_count);
+}
+
+int swb200_batch_align(swb200_batch* b, const swb200_params* pp, const swb200_options* opt, void* stream, int* d_scores,
+                       int* d_spans, unsigned int* d_ops, int ops_stride, int* d_ops_count) {
+  (void)opt;
+  if (!b || ops_stride < 1 || (b->npairs > 0 && (!d_scores || !d_spans || !d_ops || !d_ops_count)))
+    return fail(SWB200_ERR_ARG, "bad batch arguments");
+  if (b->keep_order || !b->len1) return fail(SWB200_ERR_ARG, "batch was packed in caller order (banded); re-pack with keep_order=0");
+  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
+  int rc;
+  if ((rc = check_params(p)) || (rc = check_align_batch_limits(p, b->max_short))) return rc;
+  swb200_ctx* c = b->ctx;
+  std::lock_guard<std::mutex> lk(c->mu);
+  DeviceGuard guard;
+  SWB_CUDA(cudaSetDevice(c->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  c->info = swb200_run_info{};
+  if (b->npairs == 0) return SWB200_OK;
+  SWB_CUDA(cudaEventRecord(c->ev0, s));
+  if ((rc = align_packed_locked(c, whole_batch(b), b->len1, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info))) return rc;
+  SWB_CUDA(cudaEventRecord(c->ev1, s));
+  SWB_CUDA(cudaStreamSynchronize(s));
+  float ms = 0;
+  SWB_CUDA(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+  c->info.engine_ms = ms;
+  c->info.lanes = 32; c->info.config = 300; c->info.rows = swb::kAlignStrip;
+  return SWB200_OK;
 }
 
 }  // extern "C"

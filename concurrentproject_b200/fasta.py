@@ -221,6 +221,81 @@ def score_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
     return scores
 
 
+def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarray,
+                  params: Sequence[int] = api.DEFAULT_PARAMS, *, min_bucket: int = 512, device: int = 0,
+                  ops_stride: int = api.OPS_STRIDE):
+    """Align pair k = (a[ia[k]], b[ib[k]]): (scores int32[n], spans int32[n, 4], cigars list[str]) in pair order, each
+    as api.align returns it.  The buckets of score_records: batch buckets are packed in place and aligned by
+    swb200_batch_align (pairs that need more than ops_stride operations once more with room for len1 + len2); the
+    rest (bytes other than A,C,G,T, a shorter side over 1024) pair by pair through swb200_align_device."""
+    import torch
+    ia = np.asarray(ia, dtype=np.int64)
+    ib = np.asarray(ib, dtype=np.int64)
+    if ia.shape != ib.shape:
+        raise ValueError("index arrays differ in length")
+    n = len(ia)
+    scores = np.zeros(n, dtype=np.int32)
+    spans = np.zeros((n, 4), dtype=np.int32)
+    cigars: List[str] = [""] * n
+    if n == 0:
+        return scores, spans, cigars
+    if not torch.cuda.is_available():
+        raise RuntimeError("concurrentproject_b200.fasta needs a CUDA device; there is no CPU alignment path")
+    dev = torch.device("cuda", device)
+    ctx = api.Context(device)
+    try:
+        fa, ok_a = _device_records(a, torch, dev)
+        fb, ok_b = (fa, ok_a) if b is a else _device_records(b, torch, dev)
+        l1, l2 = a.lengths[ia].astype(np.int32), b.lengths[ib].astype(np.int32)
+        o1, o2 = a.offsets[ia].astype(np.int64), b.offsets[ib].astype(np.int64)
+        buckets = plan_buckets(l1, l2, ok_a[ia] & ok_b[ib], min_bucket, match=int(params[0]))
+        stream = torch.cuda.current_stream(dev).cuda_stream
+
+        def run(ids, stride):
+            bl1, bl2 = l1[ids], l2[ids]
+            d_o1 = torch.from_numpy(o1[ids]).to(dev); d_o2 = torch.from_numpy(o2[ids]).to(dev)
+            d_l1 = torch.from_numpy(bl1).to(dev); d_l2 = torch.from_numpy(bl2).to(dev)
+            d_sc = torch.empty(len(ids), dtype=torch.int32, device=dev)
+            d_sp = torch.empty((len(ids), 4), dtype=torch.int32, device=dev)
+            d_ops = torch.empty((len(ids), stride), dtype=torch.int32, device=dev)
+            d_cnt = torch.empty(len(ids), dtype=torch.int32, device=dev)
+            short, long_ = np.minimum(bl1, bl2), np.maximum(bl1, bl2)
+            cells = int((bl1.astype(np.int64) * bl2).sum())
+            pb = api.PackedBatch(ctx, fa.data_ptr(), d_o1.data_ptr(), d_l1.data_ptr(), fb.data_ptr(), d_o2.data_ptr(),
+                                 d_l2.data_ptr(), len(ids), int(short.max()), int(long_.max()), cells, stream=stream)
+            try:
+                pb.align(d_sc.data_ptr(), d_sp.data_ptr(), d_ops.data_ptr(), stride, d_cnt.data_ptr(), params, stream=stream)
+            finally:
+                pb.close()
+            return d_sc.cpu().numpy(), d_sp.cpu().numpy(), d_ops.cpu().numpy().view(np.uint32), d_cnt.cpu().numpy()
+
+        for bk in buckets:
+            ids = bk.index
+            if bk.kind == "batch":
+                sc, sp, ops, cnt = run(ids, ops_stride)
+                scores[ids] = sc
+                spans[ids] = sp
+                for r, pid in enumerate(ids.tolist()):
+                    if cnt[r] >= 0:
+                        cigars[pid] = api.cigar_string(ops[r, :cnt[r]])
+                redo = ids[cnt < 0]
+                if len(redo):
+                    _, _, ops2, cnt2 = run(redo, int((l1[redo].astype(np.int64) + l2[redo]).max()))
+                    for r, pid in enumerate(redo.tolist()):
+                        cigars[pid] = api.cigar_string(ops2[r, :cnt2[r]])
+            else:
+                for pid in ids.tolist():
+                    i1, i2 = int(ia[pid]), int(ib[pid])
+                    if a.lengths[i1] == 0 or b.lengths[i2] == 0:
+                        continue                                   # an empty sequence scores 0: span (0,0,0,0), no CIGAR
+                    s_, span, cig = ctx.align_device(fa.data_ptr() + int(a.offsets[i1]), int(a.lengths[i1]),
+                                                     fb.data_ptr() + int(b.offsets[i2]), int(b.lengths[i2]), params, stream=stream)
+                    scores[pid], spans[pid], cigars[pid] = s_, span, cig
+    finally:
+        ctx.close()
+    return scores, spans, cigars
+
+
 def _as_records(seqs) -> FastaRecords:
     if isinstance(seqs, FastaRecords):
         return seqs
@@ -243,3 +318,13 @@ def search(query, database, params: Sequence[int] = api.DEFAULT_PARAMS, *, min_b
     db = _as_records(database)
     return score_records(q, np.zeros(len(db), dtype=np.int64), db, np.arange(len(db), dtype=np.int64), params,
                          min_bucket=min_bucket)
+
+
+def align_pairs(seqs1, seqs2, params: Sequence[int] = api.DEFAULT_PARAMS, *, min_bucket: int = 512):
+    """(scores, spans, cigars) of (seqs1[k], seqs2[k]) for ragged lists of byte strings (or two FastaRecords of equal size),
+    each as api.align returns it (align_records)."""
+    a, b = _as_records(seqs1), _as_records(seqs2)
+    if len(a) != len(b):
+        raise ValueError("seqs1 and seqs2 differ in length")
+    ids = np.arange(len(a), dtype=np.int64)
+    return align_records(a, ids, b, ids, params, min_bucket=min_bucket)

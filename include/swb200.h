@@ -228,6 +228,30 @@ SWB200_API int swb200_batch_score(swb200_batch* batch, const swb200_params* p, c
                                   void* stream, int* d_scores);
 SWB200_API void swb200_batch_free(swb200_batch* batch);
 
+/* ---- batch alignment: score, span and CIGAR for every pair of a batch -------------------------------------------------
+ * For every pair k the same score, span {i_start, j_start, i_end, j_end} and alignment that swb200_align(seq1[k], seq2[k])
+ * returns for that pair alone (same tie rules), one thread per pair on the device: end cell, start cell, then the anchored
+ * recurrence over the span rectangle with 4 bits of traceback direction per cell and the walk back through them.  Limits
+ * and errors are those of swb200_score_batch (bytes A,C,G,T: SWB200_ERR_ALPHABET; min(len1,len2) <= 1024: SWB200_ERR_ARG;
+ * match*min(len) <= 32766 - match: SWB200_ERR_RANGE); pairs outside them go through swb200_align.  Score 0 (and an
+ * empty sequence) gives span (0,0,0,0) and no operations.
+ * Operations: count << 4 | op with op 7 '=', 8 'X', 1 'I' (a base of seq1 against a gap), 2 'D' (a base of seq2 against a
+ * gap) -- BAM's numbering -- first operation first.  Pair k's operations go to ops_out[k*ops_stride ...], ops_count[k] of
+ * them; a pair that needs more than ops_stride gets ops_count[k] = -(its count), nothing is written for it, and the call
+ * still succeeds (len1 + len2 operations always suffice; the host call returns that pair's slot zero-filled).  When gap_ext > gap_init the recurrence never extends a gap,
+ * so two neighbouring gap characters are two gaps and are reported as two operations ("1I1I"); otherwise the operations
+ * are exactly swb200_align's CIGAR.  Every alignment is re-scored on the device with the costs of main.cpp:28-33,57-58
+ * before the call returns; a mismatch fails the call with SWB200_ERR_CUDA ("internal: ...").
+ * The host call copies and packs in chunks and, after swb200_set_devices(G), gives each GPU a contiguous range of pairs
+ * (results identical for every G).  spans_out: 4 ints per pair.  opt is reserved (NULL). */
+SWB200_API int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                                  const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                                  const swb200_params* p, const swb200_options* opt, int* scores_out, int* spans_out,
+                                  unsigned int* ops_out, int ops_stride, int* ops_count);
+/* The same for a device-resident batch packed with keep_order = 0; every output pointer is a DEVICE pointer. */
+SWB200_API int swb200_batch_align(swb200_batch* batch, const swb200_params* p, const swb200_options* opt, void* stream,
+                                  int* d_scores, int* d_spans, unsigned int* d_ops, int ops_stride, int* d_ops_count);
+
 /* ---- banded batches (long reads): cell (i,j), i = row in seq2, j = column in seq1, is scored iff
  * band_lo <= j - i <= band_hi; everything outside the band is H=E=F=0 and excluded from the max.  The reference
  * has no banded mode; semantics = main.cpp:57-63 restricted to the band (oracle: oracle_gotoh_banded).
