@@ -220,16 +220,7 @@ def score_batch(seqs1, seqs2, params: Sequence[int] = DEFAULT_PARAMS, *, rows: i
     """Scores of many independent HOST pairs in one kernel (swb200_score_batch).  seqs1[k] vs seqs2[k]."""
     if len(seqs1) != len(seqs2):
         raise ValueError("seqs1 and seqs2 differ in length")
-    f1, o1, l1 = _flatten(seqs1)
-    f2, o2, l2 = _flatten(seqs2)
-    out = np.zeros(len(seqs1), dtype=np.int32)
-    p, o = _params(params), _options(rows=rows, no_linear=no_linear)
-    LL, I = C.POINTER(C.c_longlong), C.POINTER(C.c_int)
-    rc = _lib.load().swb200_score_batch(_ptr(f1), o1.ctypes.data_as(LL), l1.ctypes.data_as(I), _ptr(f2), o2.ctypes.data_as(LL),
-                                        l2.ctypes.data_as(I), len(seqs1), C.byref(p), C.byref(o), out.ctypes.data_as(I))
-    if rc != 0:
-        raise SwbError(rc, "swb200_score_batch")
-    return out
+    return score_batch_flat(*_flatten(seqs1), *_flatten(seqs2), params, rows=rows, no_linear=no_linear)
 
 
 def score_batch_flat(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray, flat2: np.ndarray, off2: np.ndarray,
@@ -252,25 +243,16 @@ def score_banded_batch(seqs1, seqs2, band_lo: int = -32, band_hi: int = 31, para
     """Banded scores of many HOST pairs: cell (i, j) counts iff band_lo <= j - i <= band_hi (64 diagonals)."""
     if len(seqs1) != len(seqs2):
         raise ValueError("seqs1 and seqs2 differ in length")
-    f1, o1, l1 = _flatten(seqs1)
-    f2, o2, l2 = _flatten(seqs2)
-    out = np.zeros(len(seqs1), dtype=np.int32)
-    p, o = _params(params), _options(no_linear=no_linear, config=config)      # config 16: the 16-threads-per-pair layout
-    LL, I = C.POINTER(C.c_longlong), C.POINTER(C.c_int)
-    rc = _lib.load().swb200_score_banded_batch(_ptr(f1), o1.ctypes.data_as(LL), l1.ctypes.data_as(I), _ptr(f2),
-                                               o2.ctypes.data_as(LL), l2.ctypes.data_as(I), len(seqs1), band_lo, band_hi,
-                                               C.byref(p), C.byref(o), out.ctypes.data_as(I))
-    if rc != 0:
-        raise SwbError(rc, "swb200_score_banded_batch")
-    return out
+    return score_banded_batch_flat(*_flatten(seqs1), *_flatten(seqs2), band_lo, band_hi, params, no_linear=no_linear,
+                                   config=config)
 
 
 def score_banded_batch_flat(flat1, off1, len1, flat2, off2, len2, band_lo: int = -32, band_hi: int = 31,
-                            params: Sequence[int] = DEFAULT_PARAMS, *, no_linear: bool = False) -> np.ndarray:
+                            params: Sequence[int] = DEFAULT_PARAMS, *, no_linear: bool = False, config: int = 0) -> np.ndarray:
     """swb200_score_banded_batch on already flattened HOST arrays."""
     n = len(len1)
     out = np.zeros(n, dtype=np.int32)
-    p, o = _params(params), _options(no_linear=no_linear)
+    p, o = _params(params), _options(no_linear=no_linear, config=config)      # config 16: the 16-threads-per-pair layout
     LL, I = C.POINTER(C.c_longlong), C.POINTER(C.c_int)
     rc = _lib.load().swb200_score_banded_batch(_ptr(flat1), off1.ctypes.data_as(LL), len1.ctypes.data_as(I), _ptr(flat2),
                                                off2.ctypes.data_as(LL), len2.ctypes.data_as(I), n, band_lo, band_hi, C.byref(p),

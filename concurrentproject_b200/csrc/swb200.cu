@@ -23,6 +23,7 @@
 #include <string>
 #include <vector>
 #include <algorithm>
+#include <functional>
 
 namespace {
 
@@ -296,7 +297,6 @@ struct swb200_batch {
   long long npairs = 0, q_stride = 0, t_stride = 0;
   int max_short = 0, max_long = 0;
   int keep_order = 0;          // 1: q = seq1, t = seq2 exactly as given (banded scoring needs j-i)
-  bool pooled = false;         // storage belongs to the context's staging pool
   uint64_t* q_words = nullptr;
   uint64_t* t_words = nullptr;
   int* q_len = nullptr;
@@ -355,6 +355,10 @@ int check_params(const swb200_params& p) {
     return fail(SWB200_ERR_ARG, "scoring parameters outside the documented limits");
   return SWB200_OK;
 }
+
+// NULL parameters / options: MATCH, MISMATCH, GAP_INIT, GAP_EXT of main.cpp:20-23, and every option at its default
+swb200_params params_or_default(const swb200_params* p) { return p ? *p : swb200_params{1, -1, 1, 1}; }
+swb200_options options_or_default(const swb200_options* o) { return o ? *o : swb200_options{}; }
 
 // Re-based 16-bit lanes are exact as long as the values one warp holds at one time, plus what they can drift
 // between two re-base decisions, stay far inside 16 bits: neighbouring cells differ by at most match + gap per
@@ -831,8 +835,8 @@ int run_once(swb200_ctx* c, const uint8_t* d_seq1, long long n, const uint8_t* d
 int score_device_locked(swb200_ctx* c, const uint8_t* d_seq1, long long n, const uint8_t* d_seq2, long long m,
                         const swb200_params* pp, const swb200_options* oo, cudaStream_t s, int* score_out,
                         long long* end_out = nullptr, bool anchored = false, bool record_dirs = false) {
-  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
-  swb200_options o = oo ? *oo : swb200_options{};
+  const swb200_params p = params_or_default(pp);
+  swb200_options o = options_or_default(oo);
   if (end_out || record_dirs) { o.orient = 2; o.lanes = 0; o.two_sided = -1; o.rebase = -1; if (o.rows > 16) o.rows = 16; }
   int rc;
   if ((rc = check_params(p))) return rc;
@@ -946,11 +950,6 @@ static bool pool_last_run(swb200_run_info* info);
 // host pair call: 1 = not a case for the device pool (score it on one GPU), otherwise the call's return code
 static int score_pair_on_pool(const unsigned char* seq1, long long n, const unsigned char* seq2, long long m,
                               const swb200_params* p, const swb200_options* opt, int* score_out);
-// host batch calls: one GPU, or contiguous ranges of pairs over the devices chosen with swb200_set_devices
-static int score_batch_host(const unsigned char* seq1_all, const long long* off1, const int* len1,
-                            const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
-                            const swb200_params* p, const swb200_options* opt, int banded, int band_lo, int band_hi,
-                            int* scores_out);
 
 // ---------------------------------------------------------------------------------------------
 //  exported C ABI
@@ -981,8 +980,8 @@ int swb200_configure(const char* key, const char* value) {
 int swb200_plan(long long n, long long m, const swb200_params* pp, const swb200_options* oo, int lanes, int sms,
                 int allow_two_sided, int out[4], double* est_cycles) {
   if (!out || n < 1 || m < 1 || sms < 1) return fail(SWB200_ERR_ARG, "bad plan arguments");
-  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
-  const swb200_options o = oo ? *oo : swb200_options{};
+  const swb200_params p = params_or_default(pp);
+  const swb200_options o = options_or_default(oo);
   const Plan pl = make_plan(n, m, p, o, lanes, sms, allow_two_sided != 0, /*allow_chain=*/allow_two_sided != 0);
   out[0] = pl.mode; out[1] = pl.R; out[2] = pl.config; out[3] = pl.two_sided ? 1 : 0;
   if (est_cycles) {
@@ -1185,7 +1184,7 @@ static int align_locked(swb200_ctx* c, const uint8_t* d_seq1, long long n, const
   cigar->clear();
   int rc = score_span_locked(c, d_seq1, n, d_seq2, m, pp, s, score_out, span4);
   if (rc || *score_out <= 0) return rc;
-  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
+  const swb200_params p = params_or_default(pp);
   const long long is = span4[0], js = span4[1], ie = span4[2], je = span4[3];
   const long long rows = ie - is + 1, cols = je - js + 1;
   const swb200_run_info before = c->info;
@@ -1306,22 +1305,22 @@ int swb200_last_run(swb200_ctx* c, swb200_run_info* info) {
 }
 
 // ---- batches of independent pairs --------------------------------------------------------------------
-static int batch_pack_impl(swb200_ctx* c, const unsigned char* d_seq1, const long long* d_off1, const int* d_len1,
-                           const unsigned char* d_seq2, const long long* d_off2, const int* d_len2, long long npairs,
-                           int max_short, int max_long, long long total_cells, int keep_order, bool pooled, void* stream,
-                           swb200_batch** out);
+// Word strides of the resident 2-bit layout (32 symbols per 64-bit word) for sequences of up to max_q / max_t symbols: at
+// least one word; +2 on the T side because the kernels prefetch one word past the end; +2 on the Q side of a batch kept
+// in caller order (keep_order: the banded kernel streams both sequences).
+struct Strides { long long q, t; };
+static Strides batch_strides_for(int max_q, int max_t, bool keep_order) {
+  return Strides{std::max(1, (max_q + 31) / 32) + (keep_order ? 2 : 0), std::max(1, (max_t + 31) / 32) + 2};
+}
+static bool fits_strides(int q, int t, const Strides& s, bool keep_order) {
+  const Strides need = batch_strides_for(q, t, keep_order);
+  return q >= 0 && t >= 0 && need.q <= s.q && need.t <= s.t;
+}
+
 int swb200_batch_pack_device(swb200_ctx* c, const unsigned char* d_seq1, const long long* d_off1, const int* d_len1,
                              const unsigned char* d_seq2, const long long* d_off2, const int* d_len2, long long npairs,
                              int max_short, int max_long, long long total_cells, int keep_order, void* stream,
                              swb200_batch** out) {
-  return batch_pack_impl(c, d_seq1, d_off1, d_len1, d_seq2, d_off2, d_len2, npairs, max_short, max_long, total_cells,
-                         keep_order, false, stream, out);
-}
-
-static int batch_pack_impl(swb200_ctx* c, const unsigned char* d_seq1, const long long* d_off1, const int* d_len1,
-                           const unsigned char* d_seq2, const long long* d_off2, const int* d_len2, long long npairs,
-                           int max_short, int max_long, long long total_cells, int keep_order, bool pooled, void* stream,
-                           swb200_batch** out) {
   if (!c || !out || npairs < 0 || max_short < 0 || max_long < 0 || (!keep_order && max_long < max_short))
     return fail(SWB200_ERR_ARG, "bad batch arguments");
   std::lock_guard<std::mutex> lk(c->mu);
@@ -1331,22 +1330,14 @@ static int batch_pack_impl(swb200_ctx* c, const unsigned char* d_seq1, const lon
   std::unique_ptr<swb200_batch, BatchDeleter> b(new swb200_batch());   // freed on every early return
   b->ctx = c; b->npairs = npairs; b->max_short = max_short; b->max_long = max_long; b->cells = total_cells;
   b->keep_order = keep_order ? 1 : 0;
-  b->q_stride = std::max(1, (max_short + 31) / 32) + (keep_order ? 2 : 0);
-  b->t_stride = std::max(1, (max_long + 31) / 32) + 2;      // +2: the kernel prefetches one word past the end
+  const Strides st = batch_strides_for(max_short, max_long, keep_order);
+  b->q_stride = st.q; b->t_stride = st.t;
   const size_t np = (size_t)std::max<long long>(npairs, 1);
-  b->pooled = pooled;
-  if (pooled) {
-    int rc;
-    if ((rc = grow(c->hb_qw, c->hb_qw_cap, np * b->q_stride, false, s)) || (rc = grow(c->hb_tw, c->hb_tw_cap, np * b->t_stride, false, s)) ||
-        (rc = grow(c->hb_ql, c->hb_ql_cap, np, false, s)) || (rc = grow(c->hb_tl, c->hb_tl_cap, np, false, s))) return rc;
-    b->q_words = c->hb_qw; b->t_words = c->hb_tw; b->q_len = c->hb_ql; b->t_len = c->hb_tl;
-  } else {
-    SWB_CUDA(cudaMalloc(&b->q_words, np * b->q_stride * sizeof(uint64_t)));
-    SWB_CUDA(cudaMalloc(&b->t_words, np * b->t_stride * sizeof(uint64_t)));
-    SWB_CUDA(cudaMalloc(&b->q_len, np * sizeof(int)));
-    SWB_CUDA(cudaMalloc(&b->t_len, np * sizeof(int)));
-    if (!keep_order) SWB_CUDA(cudaMalloc(&b->len1, np * sizeof(int)));
-  }
+  SWB_CUDA(cudaMalloc(&b->q_words, np * b->q_stride * sizeof(uint64_t)));
+  SWB_CUDA(cudaMalloc(&b->t_words, np * b->t_stride * sizeof(uint64_t)));
+  SWB_CUDA(cudaMalloc(&b->q_len, np * sizeof(int)));
+  SWB_CUDA(cudaMalloc(&b->t_len, np * sizeof(int)));
+  if (!keep_order) SWB_CUDA(cudaMalloc(&b->len1, np * sizeof(int)));
   SWB_CUDA(cudaMemsetAsync(c->d_result, 0, 12 * sizeof(int), s));    // [0] score, [1] status, [3..8] timeout post-mortem, [11] protocol-checker mismatches
   if (npairs > 0) {
     const long long total = npairs * (b->q_stride + b->t_stride);
@@ -1371,11 +1362,11 @@ struct BatchView {
   int max_short, max_long;      // of the WHOLE batch: every range of one batch runs the same kernel
 };
 
-static int check_batch_score(const BatchView& v, const swb200_params& p, int keep_order) {
+static int check_batch_score(const swb200_params& p, int keep_order, int max_short) {
   if (keep_order) return fail(SWB200_ERR_ARG, "batch was packed in caller order (banded); re-pack with keep_order=0");
-  if (v.max_short > 1024)
+  if (max_short > 1024)
     return fail(SWB200_ERR_ARG, "batch kernel needs min(len1,len2) <= 1024 per pair; use swb200_score for long pairs");
-  if ((long long)p.match * v.max_short > 32767 - p.match - 1)
+  if ((long long)p.match * max_short > 32767 - p.match - 1)
     return fail(SWB200_ERR_RANGE, "match * min(len) does not fit the 16-bit lanes of the batch kernel");
   return SWB200_OK;
 }
@@ -1411,10 +1402,10 @@ static int launch_batch_score(swb200_ctx* c, const BatchView& v, const swb200_pa
   return SWB200_OK;
 }
 
-static int check_banded_score(const BatchView& v, const swb200_params& p, int keep_order, int band_lo, int band_hi) {
+static int check_banded_score(const swb200_params& p, int keep_order, int band_lo, int band_hi, int max1, int max2) {
   if (!keep_order) return fail(SWB200_ERR_ARG, "banded scoring needs a batch packed with keep_order=1");
   if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
-  if ((long long)p.match * std::min(v.max_short, v.max_long) > 32767 - p.match - 1)
+  if ((long long)p.match * std::min(max1, max2) > 32767 - p.match - 1)
     return fail(SWB200_ERR_RANGE, "match * min(len) does not fit the 16-bit lanes of the banded kernel");
   return SWB200_OK;
 }
@@ -1468,25 +1459,21 @@ static BatchView whole_batch(const swb200_batch* b) {
   return BatchView{b->q_words, b->t_words, b->q_len, b->t_len, b->q_stride, b->t_stride, b->npairs, b->max_short, b->max_long};
 }
 
-int swb200_batch_score(swb200_batch* b, const swb200_params* pp, const swb200_options* oo, void* stream,
-                       int* d_scores) {
-  if (!b || !d_scores) return fail(SWB200_ERR_ARG, "bad batch arguments");
+// The device-batch calls after their argument checks: b's context locked and its device current, the run info reset to
+// `cells`, nothing more for an empty batch, else work(c, s) between the two timing events on the caller's stream.
+static int run_device_batch(swb200_batch* b, long long cells, void* stream,
+                            const std::function<int(swb200_ctx*, cudaStream_t)>& work) {
   swb200_ctx* c = b->ctx;
   std::lock_guard<std::mutex> lk(c->mu);
-  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
-  const swb200_options o = oo ? *oo : swb200_options{};
-  int rc;
-  if ((rc = check_params(p))) return rc;
-  const BatchView v = whole_batch(b);
-  if ((rc = check_batch_score(v, p, b->keep_order))) return rc;
   DeviceGuard guard;
   SWB_CUDA(cudaSetDevice(c->device));
-  cudaStream_t s = (cudaStream_t)stream;
+  const cudaStream_t s = (cudaStream_t)stream;
   c->info = swb200_run_info{};
-  c->info.cells = b->cells;
+  c->info.cells = cells;
   if (b->npairs == 0) return SWB200_OK;
   SWB_CUDA(cudaEventRecord(c->ev0, s));
-  if ((rc = launch_batch_score(c, v, p, o, s, d_scores, &c->info))) return rc;
+  int rc;
+  if ((rc = work(c, s))) return rc;
   SWB_CUDA(cudaEventRecord(c->ev1, s));
   SWB_CUDA(cudaStreamSynchronize(s));
   float ms = 0;
@@ -1495,153 +1482,177 @@ int swb200_batch_score(swb200_batch* b, const swb200_params* pp, const swb200_op
   return SWB200_OK;
 }
 
+int swb200_batch_score(swb200_batch* b, const swb200_params* pp, const swb200_options* oo, void* stream,
+                       int* d_scores) {
+  if (!b || !d_scores) return fail(SWB200_ERR_ARG, "bad batch arguments");
+  const swb200_params p = params_or_default(pp);
+  const swb200_options o = options_or_default(oo);
+  int rc;
+  if ((rc = check_params(p)) || (rc = check_batch_score(p, b->keep_order, b->max_short))) return rc;
+  return run_device_batch(b, b->cells, stream, [&](swb200_ctx* c, cudaStream_t s) {
+    return launch_batch_score(c, whole_batch(b), p, o, s, d_scores, &c->info);
+  });
+}
+
 int swb200_batch_score_banded(swb200_batch* b, int band_lo, int band_hi, const swb200_params* pp, const swb200_options* oo,
                               void* stream, int* d_scores) {
   if (!b || !d_scores) return fail(SWB200_ERR_ARG, "bad batch arguments");
-  swb200_ctx* c = b->ctx;
-  std::lock_guard<std::mutex> lk(c->mu);
-  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
-  const swb200_options o = oo ? *oo : swb200_options{};
+  const swb200_params p = params_or_default(pp);
+  const swb200_options o = options_or_default(oo);
   int rc;
-  if ((rc = check_params(p))) return rc;
-  const BatchView v = whole_batch(b);
-  if ((rc = check_banded_score(v, p, b->keep_order, band_lo, band_hi))) return rc;
-  DeviceGuard guard;
-  SWB_CUDA(cudaSetDevice(c->device));
-  cudaStream_t s = (cudaStream_t)stream;
-  c->info = swb200_run_info{};
-  c->info.cells = b->cells;
-  if (b->npairs == 0) return SWB200_OK;
-  SWB_CUDA(cudaEventRecord(c->ev0, s));
-  if ((rc = launch_banded_score(c, v, band_lo, p, o, s, d_scores, &c->info))) return rc;
-  SWB_CUDA(cudaEventRecord(c->ev1, s));
-  SWB_CUDA(cudaStreamSynchronize(s));
-  float ms = 0;
-  SWB_CUDA(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-  c->info.engine_ms = ms;
-  return SWB200_OK;
+  if ((rc = check_params(p)) || (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
+  return run_device_batch(b, b->cells, stream, [&](swb200_ctx* c, cudaStream_t s) {
+    return launch_banded_score(c, whole_batch(b), band_lo, p, o, s, d_scores, &c->info);
+  });
 }
 
 void swb200_batch_free(swb200_batch* b) {
   if (!b) return;
   DeviceGuard guard;
   cudaSetDevice(b->ctx->device);
-  if (!b->pooled) { cudaFree(b->q_words); cudaFree(b->t_words); cudaFree(b->q_len); cudaFree(b->t_len); cudaFree(b->len1); }
+  cudaFree(b->q_words); cudaFree(b->t_words); cudaFree(b->q_len); cudaFree(b->t_len); cudaFree(b->len1);
   delete b;
 }
 
-// One context's share of a host batch call (the whole batch on one GPU; a contiguous range of pairs when the batch is
-// sharded over several GPUs: off1/len1/... then point at the range's first pair, offsets stay absolute).
-static int score_batch_host_ctx(swb200_ctx* c, const unsigned char* seq1_all, const long long* off1, const int* len1,
-                                const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
-                                const swb200_params* p, const swb200_options* opt, int banded, int band_lo, int band_hi,
-                                int* scores_out) {
-  if (npairs < 0 || (npairs > 0 && (!seq1_all || !seq2_all || !off1 || !off2 || !len1 || !len2 || !scores_out)))
-    return fail(SWB200_ERR_ARG, "bad batch arguments");
-  if (npairs == 0) return SWB200_OK;
-  int rc;
-  long long bytes1 = 0, bytes2 = 0, cells = 0, base1 = LLONG_MAX, base2 = LLONG_MAX;
-  int max_short = 0, max_long = 0;
-  {
-    // branch-free (this pass runs before the first copy can start: 1 ns per pair instead of 2-3)
-    long long neg = 0;
-    int mx1 = 0, mx2 = 0, mxmin = 0;
-    for (long long k = 0; k < npairs; ++k) {
-      const int a = len1[k], b = len2[k];
-      const long long o1 = off1[k], o2 = off2[k];
-      neg |= (long long)(a | b) | o1 | o2;                       // sign bit set iff any of the four is negative
-      bytes1 = std::max(bytes1, o1 + a);
-      bytes2 = std::max(bytes2, o2 + b);
-      base1 = std::min(base1, o1);
-      base2 = std::min(base2, o2);
-      mx1 = std::max(mx1, a); mx2 = std::max(mx2, b); mxmin = std::max(mxmin, std::min(a, b));
-      cells += (long long)a * b;
-    }
-    if (neg < 0) return fail(SWB200_ERR_ARG, "negative length or offset");
-    if (banded) { max_short = mx1; max_long = mx2; }
-    else { max_short = mxmin; max_long = std::max(mx1, mx2); }
+// An ASCII host batch, or a contiguous range of one: pointers at its first pair, offsets absolute.
+struct HostPairs {
+  const unsigned char* seq1; const long long* off1; const int* len1;
+  const unsigned char* seq2; const long long* off2; const int* len2;
+  HostPairs from(long long k0) const { return HostPairs{seq1, off1 + k0, len1 + k0, seq2, off2 + k0, len2 + k0}; }
+};
+
+// What the host calls learn from pairs [k0, k1) of an ASCII batch before they touch a device.
+struct PairScan {
+  long long neg = 0;                                            // sign bit set iff a length or an offset is negative
+  int max1 = 0, max2 = 0, max_min = 0;                          // longest seq1, longest seq2, longest shorter sequence
+  long long cells = 0;
+  long long lo1 = LLONG_MAX, hi1 = 0, lo2 = LLONG_MAX, hi2 = 0;   // lowest offset and highest end on each side
+  // the batch shape: a banded batch (keep_order) keeps seq1 / seq2 in place, the others put the shorter sequence first
+  int max_short(bool keep_order) const { return keep_order ? max1 : max_min; }
+  int max_long(bool keep_order) const { return keep_order ? max2 : std::max(max1, max2); }
+  void merge(const PairScan& o) {
+    neg |= o.neg; max1 = std::max(max1, o.max1); max2 = std::max(max2, o.max2); max_min = std::max(max_min, o.max_min);
+    cells += o.cells;
+    lo1 = std::min(lo1, o.lo1); hi1 = std::max(hi1, o.hi1); lo2 = std::min(lo2, o.lo2); hi2 = std::max(hi2, o.hi2);
   }
-  base1 &= ~15LL; base2 &= ~15LL;          // staged bytes keep their position relative to the range's lowest offset
-  bytes1 -= base1; bytes2 -= base2;
-  // Pipeline: the pairs are cut into chunks of ~48 MB of sequence; own_stream copies chunk k+1 from the host while
-  // aux_stream packs and scores chunk k (the staging pool is sized for the whole range, so chunks need no double
-  // buffering: every byte keeps its relative position).  With pinned host buffers the call runs at PCIe speed.
-  const swb200_params pv = p ? *p : swb200_params{1, -1, 1, 1};
-  const swb200_options ov = opt ? *opt : swb200_options{};
-  if ((rc = check_params(pv))) return rc;
+};
+
+// Branch-free (this pass runs before the first copy can start: 1 ns per pair instead of 2-3).
+static PairScan scan_pairs(const HostPairs& h, long long k0, long long k1) {
+  long long neg = 0, cells = 0, lo1 = LLONG_MAX, hi1 = 0, lo2 = LLONG_MAX, hi2 = 0;
+  int mx1 = 0, mx2 = 0, mxmin = 0;
+  for (long long k = k0; k < k1; ++k) {
+    const int a = h.len1[k], b = h.len2[k];
+    const long long o1 = h.off1[k], o2 = h.off2[k];
+    neg |= (long long)(a | b) | o1 | o2;
+    hi1 = std::max(hi1, o1 + a);
+    hi2 = std::max(hi2, o2 + b);
+    lo1 = std::min(lo1, o1);
+    lo2 = std::min(lo2, o2);
+    mx1 = std::max(mx1, a); mx2 = std::max(mx2, b); mxmin = std::max(mxmin, std::min(a, b));
+    cells += (long long)a * b;
+  }
+  return PairScan{neg, mx1, mx2, mxmin, cells, lo1, hi1, lo2, hi2};
+}
+
+static int check_score_pairs(const PairScan& s, const swb200_params& p, int banded, int band_lo, int band_hi) {
+  if (s.neg < 0) return fail(SWB200_ERR_ARG, "negative length or offset");
+  int rc;
+  if ((rc = check_params(p))) return rc;
+  return banded ? check_banded_score(p, 1, band_lo, band_hi, s.max1, s.max2) : check_batch_score(p, 0, s.max_min);
+}
+
+// chunk_events of the host pipelines, grow-only: one per chunk of a call
+static int chunk_events_at_least(swb200_ctx* c, size_t n) {
+  while (c->chunk_events.size() < n) {
+    cudaEvent_t e;
+    SWB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    c->chunk_events.push_back(e);
+  }
+  return SWB200_OK;
+}
+
+// Copy/pack pipeline of the ASCII host calls for one context's range h of npairs pairs (c locked, its device current;
+// part: the range's scan, whole: the whole batch's).  The pairs are cut into chunks of ~48 MB of sequence; own_stream
+// copies chunk k+1 from the host while aux_stream packs chunk k and runs each_chunk (if any) on it.  The staging pool is
+// sized for the whole range, so chunks need no double buffering: every byte keeps its position relative to the range's
+// lowest offset.  With pinned host buffers the call runs at PCIe speed.  ev0 is recorded at the first pack; *staged is
+// the packed range.
+static int stage_and_pack_locked(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part,
+                                 const PairScan& whole, bool keep_order, BatchView* staged,
+                                 const std::function<int(const BatchView& chunk, long long k0)>& each_chunk) {
+  cudaStream_t sc = c->own_stream, sk = c->aux_stream;
+  const size_t np = (size_t)npairs;
+  const long long base1 = part.lo1 & ~15LL, base2 = part.lo2 & ~15LL;
+  const int max_short = whole.max_short(keep_order), max_long = whole.max_long(keep_order);
+  const Strides st = batch_strides_for(max_short, max_long, keep_order);
+  int rc;
+  if ((rc = grow(c->hb_seq1, c->hb_seq1_cap, (size_t)(part.hi1 - base1) + 16, false, sc)) ||
+      (rc = grow(c->hb_seq2, c->hb_seq2_cap, (size_t)(part.hi2 - base2) + 16, false, sc)) ||
+      (rc = grow(c->hb_off1, c->hb_off1_cap, np, false, sc)) || (rc = grow(c->hb_off2, c->hb_off2_cap, np, false, sc)) ||
+      (rc = grow(c->hb_len1, c->hb_len1_cap, np, false, sc)) || (rc = grow(c->hb_len2, c->hb_len2_cap, np, false, sc)) ||
+      (rc = grow(c->hb_scores, c->hb_scores_cap, np, false, sc)) ||
+      (rc = grow(c->hb_qw, c->hb_qw_cap, np * st.q, false, sc)) || (rc = grow(c->hb_tw, c->hb_tw_cap, np * st.t, false, sc)) ||
+      (rc = grow(c->hb_ql, c->hb_ql_cap, np, false, sc)) || (rc = grow(c->hb_tl, c->hb_tl_cap, np, false, sc))) return rc;
+  *staged = BatchView{c->hb_qw, c->hb_tw, c->hb_ql, c->hb_tl, st.q, st.t, npairs, max_short, max_long};
+  SWB_CUDA(cudaMemsetAsync(c->d_result, 0, 10 * sizeof(int), sc));
+  SWB_CUDA(cudaMemcpyAsync(c->hb_off1, h.off1, np * sizeof(long long), cudaMemcpyHostToDevice, sc));
+  SWB_CUDA(cudaMemcpyAsync(c->hb_off2, h.off2, np * sizeof(long long), cudaMemcpyHostToDevice, sc));
+  SWB_CUDA(cudaMemcpyAsync(c->hb_len1, h.len1, np * sizeof(int), cudaMemcpyHostToDevice, sc));
+  SWB_CUDA(cudaMemcpyAsync(c->hb_len2, h.len2, np * sizeof(int), cudaMemcpyHostToDevice, sc));
+  size_t ci = 0;
+  long long k0 = 0, acc = 0, lo1 = LLONG_MAX, hi1 = 0, lo2 = LLONG_MAX, hi2 = 0;
+  auto issue = [&](long long k1) -> int {
+    int r;
+    if ((r = chunk_events_at_least(c, ci + 1))) return r;
+    if (hi1 > lo1) SWB_CUDA(cudaMemcpyAsync(c->hb_seq1 + (lo1 - base1), h.seq1 + lo1, (size_t)(hi1 - lo1), cudaMemcpyHostToDevice, sc));
+    if (hi2 > lo2) SWB_CUDA(cudaMemcpyAsync(c->hb_seq2 + (lo2 - base2), h.seq2 + lo2, (size_t)(hi2 - lo2), cudaMemcpyHostToDevice, sc));
+    SWB_CUDA(cudaEventRecord(c->chunk_events[ci], sc));
+    SWB_CUDA(cudaStreamWaitEvent(sk, c->chunk_events[ci], 0));
+    if (ci++ == 0) SWB_CUDA(cudaEventRecord(c->ev0, sk));
+    const long long nk = k1 - k0;
+    const int blocks = (int)std::min<long long>((nk * (st.q + st.t) + 255) / 256, 64LL * c->sms);
+    // the pack kernel adds the absolute offsets: hand it the staging pointers shifted back by the range's base
+    swb::launch_pack_batch(c->hb_seq1 - base1, c->hb_off1 + k0, c->hb_len1 + k0, c->hb_seq2 - base2, c->hb_off2 + k0,
+                           c->hb_len2 + k0, nk, st.q, st.t, c->hb_qw + k0 * st.q, c->hb_tw + k0 * st.t, c->hb_ql + k0,
+                           c->hb_tl + k0, keep_order ? 1 : 0, c->d_result, blocks, sk);
+    SWB_CUDA(cudaGetLastError());
+    c->info.aux_launches += 1;
+    if (!each_chunk) return SWB200_OK;
+    return each_chunk(BatchView{c->hb_qw + k0 * st.q, c->hb_tw + k0 * st.t, c->hb_ql + k0, c->hb_tl + k0, st.q, st.t, nk,
+                                max_short, max_long}, k0);
+  };
+  // a chunk is issued the moment the scan over the pairs has found its end, so the GPU works while the host is still
+  // cutting the later chunks
+  const long long forced = settings().batch_chunk_bytes;           // tests: force many small chunks
+  const long long target = forced > 0 ? forced : 48LL << 20, min_pairs = forced > 0 ? 1 : 1024;
+  for (long long k = 0; k < npairs; ++k) {
+    lo1 = std::min(lo1, h.off1[k]); hi1 = std::max(hi1, h.off1[k] + h.len1[k]);
+    lo2 = std::min(lo2, h.off2[k]); hi2 = std::max(hi2, h.off2[k] + h.len2[k]);
+    acc += (long long)h.len1[k] + h.len2[k];
+    if (!((acc >= target && k + 1 - k0 >= min_pairs) || k + 1 == npairs)) continue;
+    if ((rc = issue(k + 1))) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sk); return rc; }
+    k0 = k + 1; acc = 0; lo1 = LLONG_MAX; hi1 = 0; lo2 = LLONG_MAX; hi2 = 0;
+  }
+  return SWB200_OK;
+}
+
+// One context's share of a host ASCII score batch (arguments checked by the caller): every chunk is scored as soon as it
+// is packed, while the next one is copied.
+static int score_ascii_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part, const PairScan& whole,
+                           const swb200_params& p, const swb200_options& o, int banded, int band_lo, int* scores_out) {
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
   SWB_CUDA(cudaSetDevice(c->device));
   cudaStream_t sc = c->own_stream, sk = c->aux_stream;
-  const size_t np = (size_t)npairs;
-  const long long q_stride = std::max(1, (max_short + 31) / 32) + (banded ? 2 : 0);
-  const long long t_stride = std::max(1, (max_long + 31) / 32) + 2;      // +2: the kernel prefetches one word past the end
-  if ((rc = grow(c->hb_seq1, c->hb_seq1_cap, (size_t)bytes1 + 16, false, sc)) || (rc = grow(c->hb_seq2, c->hb_seq2_cap, (size_t)bytes2 + 16, false, sc)) ||
-      (rc = grow(c->hb_off1, c->hb_off1_cap, np, false, sc)) || (rc = grow(c->hb_off2, c->hb_off2_cap, np, false, sc)) ||
-      (rc = grow(c->hb_len1, c->hb_len1_cap, np, false, sc)) || (rc = grow(c->hb_len2, c->hb_len2_cap, np, false, sc)) ||
-      (rc = grow(c->hb_scores, c->hb_scores_cap, np, false, sc)) ||
-      (rc = grow(c->hb_qw, c->hb_qw_cap, np * q_stride, false, sc)) || (rc = grow(c->hb_tw, c->hb_tw_cap, np * t_stride, false, sc)) ||
-      (rc = grow(c->hb_ql, c->hb_ql_cap, np, false, sc)) || (rc = grow(c->hb_tl, c->hb_tl_cap, np, false, sc))) return rc;
-  const BatchView all{c->hb_qw, c->hb_tw, c->hb_ql, c->hb_tl, q_stride, t_stride, npairs, max_short, max_long};
-  if ((rc = banded ? check_banded_score(all, pv, 1, band_lo, band_hi) : check_batch_score(all, pv, 0))) return rc;
-
-  // A chunk is issued (copies on own_stream, pack + score on aux_stream) the moment the scan over the pairs has found its
-  // end, so the GPU works while the host is still cutting the later chunks.
-  struct Chunk { long long k0, k1, lo1, hi1, lo2, hi2; };
   c->info = swb200_run_info{};
-  c->info.cells = cells;
-  SWB_CUDA(cudaMemsetAsync(c->d_result, 0, 10 * sizeof(int), sc));
-  SWB_CUDA(cudaMemcpyAsync(c->hb_off1, off1, npairs * sizeof(long long), cudaMemcpyHostToDevice, sc));
-  SWB_CUDA(cudaMemcpyAsync(c->hb_off2, off2, npairs * sizeof(long long), cudaMemcpyHostToDevice, sc));
-  SWB_CUDA(cudaMemcpyAsync(c->hb_len1, len1, npairs * sizeof(int), cudaMemcpyHostToDevice, sc));
-  SWB_CUDA(cudaMemcpyAsync(c->hb_len2, len2, npairs * sizeof(int), cudaMemcpyHostToDevice, sc));
-  bool first = true;
-  size_t ci = 0;
-  auto issue = [&](const Chunk& ch) -> int {
-    while (c->chunk_events.size() < ci + 1) {
-      cudaEvent_t e;
-      SWB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      c->chunk_events.push_back(e);
-    }
-    if (ch.hi1 > ch.lo1) SWB_CUDA(cudaMemcpyAsync(c->hb_seq1 + (ch.lo1 - base1), seq1_all + ch.lo1, (size_t)(ch.hi1 - ch.lo1), cudaMemcpyHostToDevice, sc));
-    if (ch.hi2 > ch.lo2) SWB_CUDA(cudaMemcpyAsync(c->hb_seq2 + (ch.lo2 - base2), seq2_all + ch.lo2, (size_t)(ch.hi2 - ch.lo2), cudaMemcpyHostToDevice, sc));
-    SWB_CUDA(cudaEventRecord(c->chunk_events[ci], sc));
-    SWB_CUDA(cudaStreamWaitEvent(sk, c->chunk_events[ci], 0));
-    ci += 1;
-    if (first) { SWB_CUDA(cudaEventRecord(c->ev0, sk)); first = false; }
-    const long long nk = ch.k1 - ch.k0;
-    const long long total = nk * (q_stride + t_stride);
-    const int blocks = (int)std::min<long long>((total + 255) / 256, 64LL * c->sms);
-    // the pack kernel adds the absolute offsets: hand it the staging pointers shifted back by the range's base
-    swb::launch_pack_batch(c->hb_seq1 - base1, c->hb_off1 + ch.k0, c->hb_len1 + ch.k0, c->hb_seq2 - base2, c->hb_off2 + ch.k0, c->hb_len2 + ch.k0, nk,
-                           q_stride, t_stride, c->hb_qw + ch.k0 * q_stride, c->hb_tw + ch.k0 * t_stride, c->hb_ql + ch.k0,
-                           c->hb_tl + ch.k0, banded ? 1 : 0, c->d_result, blocks, sk);
-    SWB_CUDA(cudaGetLastError());
-    c->info.aux_launches += 1;
-    const BatchView v{c->hb_qw + ch.k0 * q_stride, c->hb_tw + ch.k0 * t_stride, c->hb_ql + ch.k0, c->hb_tl + ch.k0,
-                      q_stride, t_stride, nk, max_short, max_long};
-    return banded ? launch_banded_score(c, v, band_lo, pv, ov, sk, c->hb_scores + ch.k0, &c->info)
-                  : launch_batch_score(c, v, pv, ov, sk, c->hb_scores + ch.k0, &c->info);
-  };
-  {
-    const long long forced = settings().batch_chunk_bytes;
-    const bool ov_chunk = forced > 0;                                // tests: force many small chunks
-    const long long target = ov_chunk ? forced : 48LL << 20;
-    const long long min_pairs = ov_chunk ? 1 : 1024;
-    Chunk cur{0, 0, LLONG_MAX, 0, LLONG_MAX, 0};
-    long long acc = 0;
-    for (long long k = 0; k < npairs; ++k) {
-      cur.lo1 = std::min(cur.lo1, off1[k]); cur.hi1 = std::max(cur.hi1, off1[k] + len1[k]);
-      cur.lo2 = std::min(cur.lo2, off2[k]); cur.hi2 = std::max(cur.hi2, off2[k] + len2[k]);
-      acc += (long long)len1[k] + len2[k];
-      if ((acc >= target && k + 1 - cur.k0 >= min_pairs) || k + 1 == npairs) {
-        cur.k1 = k + 1;
-        if ((rc = issue(cur))) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sk); return rc; }
-        cur = Chunk{k + 1, 0, LLONG_MAX, 0, LLONG_MAX, 0};
-        acc = 0;
-      }
-    }
-  }
+  c->info.cells = part.cells;
+  BatchView staged;
+  int rc = stage_and_pack_locked(c, h, npairs, part, whole, banded != 0, &staged, [&](const BatchView& v, long long k0) {
+    return banded ? launch_banded_score(c, v, band_lo, p, o, sk, c->hb_scores + k0, &c->info)
+                  : launch_batch_score(c, v, p, o, sk, c->hb_scores + k0, &c->info);
+  });
+  if (rc) return rc;
   SWB_CUDA(cudaEventRecord(c->ev1, sk));
   SWB_CUDA(cudaMemcpyAsync(scores_out, c->hb_scores, npairs * sizeof(int), cudaMemcpyDeviceToHost, sk));
   SWB_CUDA(cudaMemcpyAsync(c->h_result, c->d_result, 2 * sizeof(int), cudaMemcpyDeviceToHost, sk));
@@ -1654,20 +1665,6 @@ static int score_batch_host_ctx(swb200_ctx* c, const unsigned char* seq1_all, co
   return SWB200_OK;
 }
 
-int swb200_score_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
-                       const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
-                       const swb200_params* p, const swb200_options* opt, int* scores_out) {
-  return score_batch_host(seq1_all, off1, len1, seq2_all, off2, len2, npairs, p, opt, 0, 0, 0, scores_out);
-}
-
-int swb200_score_banded_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
-                              const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
-                              int band_lo, int band_hi, const swb200_params* p, const swb200_options* opt,
-                              int* scores_out) {
-  if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
-  return score_batch_host(seq1_all, off1, len1, seq2_all, off2, len2, npairs, p, opt, 1, band_lo, band_hi, scores_out);
-}
-
 int swb200_score_banded(const unsigned char* seq1, int n, const unsigned char* seq2, int m, int band_lo, int band_hi,
                         const swb200_params* p, int* score_out) {
   if (n < 0 || m < 0 || !score_out || (n > 0 && !seq1) || (m > 0 && !seq2)) return fail(SWB200_ERR_ARG, "bad sequence arguments");
@@ -1675,10 +1672,13 @@ int swb200_score_banded(const unsigned char* seq1, int n, const unsigned char* s
   *score_out = 0;
   if (n == 0 || m == 0) { if (p) { int rc = check_params(*p); if (rc) return rc; } return SWB200_OK; }
   const long long off = 0;
+  const HostPairs in{seq1, &off, &n, seq2, &off, &m};
+  const PairScan s = scan_pairs(in, 0, 1);
+  const swb200_params pv = params_or_default(p);
   swb200_ctx* c = nullptr;
-  int rc = default_ctx(&c);
-  if (rc) return rc;
-  return score_batch_host_ctx(c, seq1, &off, &n, seq2, &off, &m, 1, p, nullptr, 1, band_lo, band_hi, score_out);
+  int rc;
+  if ((rc = check_score_pairs(s, pv, 1, band_lo, band_hi)) || (rc = default_ctx(&c))) return rc;
+  return score_ascii_ctx(c, in, 1, s, s, pv, swb200_options{}, 1, band_lo, score_out);
 }
 
 // ---- one pair over a ring of GPUs (one swb200_ring per GPU / per process) -------------------------
@@ -1779,8 +1779,8 @@ int swb200_ring_score_device(swb200_ring* r, const unsigned char* d_seq1, long l
   if (!r->next) return fail(SWB200_ERR_ARG, "ring is not connected");
   swb200_ctx* c = r->ctx;
   std::lock_guard<std::mutex> lk(c->mu);
-  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
-  swb200_options o = oo ? *oo : swb200_options{};
+  const swb200_params p = params_or_default(pp);
+  swb200_options o = options_or_default(oo);
   int rc;
   if ((rc = check_params(p))) return rc;
   if (n < 1 || m < 1) return fail(SWB200_ERR_ARG, "ring scoring needs non-empty sequences");
@@ -1908,8 +1908,8 @@ int pool_score_pair(const unsigned char* seq1, long long n, const unsigned char*
                     const swb200_options* oo, int* score_out, bool* handled) {
   *handled = true;
   const int G = (int)g_pool.ctx.size();
-  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
-  const swb200_options o = oo ? *oo : swb200_options{};
+  const swb200_params p = params_or_default(pp);
+  const swb200_options o = options_or_default(oo);
   int rc;
   if ((rc = check_params(p))) return rc;
   const bool stream_is_shorter = o.orient == 0;
@@ -1979,6 +1979,49 @@ int pool_score_pair(const unsigned char* seq1, long long n, const unsigned char*
   return fail(SWB200_ERR_RANGE, "no lane width could score this pair");
 }
 
+// The host batch calls: the whole batch on one GPU, or contiguous ranges of pairs, one per device chosen with
+// swb200_set_devices (SURVEY.md 8e: pair_id / ceil(P / G); no data-path communication).  scan(k0, k1) reads a range's
+// host inputs, each range on its own host thread (a serial pass over 10 M pairs costs milliseconds before the first copy
+// can start); check(whole) validates the merged scan before any device is touched; run(ctx, k0, k1, part, whole) is one
+// context's share, given its range's scan and the whole batch's.
+template <class ScanFn, class CheckFn, class RunFn>
+int run_host_batch(long long npairs, ScanFn scan, CheckFn check, RunFn run) {
+  using Scan = decltype(scan(0LL, 0LL));
+  std::unique_lock<std::mutex> pl(g_pool.mu);
+  g_pool.info_valid = false;
+  int G = (int)g_pool.ctx.size();
+  int rc;
+  if (G < 2 || npairs < 2LL * G) {
+    pl.unlock();
+    const Scan whole = scan(0, npairs);
+    swb200_ctx* c = nullptr;
+    if ((rc = check(whole)) || (rc = default_ctx(&c))) return rc;
+    return run(c, 0, npairs, whole, whole);
+  }
+  const long long per = (npairs + G - 1) / G;
+  auto first = [&](int g) { return std::min<long long>(npairs, (long long)g * per); };
+  std::vector<Scan> part((size_t)G);
+  if ((rc = pool_parallel(G, [&](int g) { part[(size_t)g] = scan(first(g), first(g + 1)); return SWB200_OK; }))) return rc;
+  Scan whole = part[0];
+  for (int g = 1; g < G; ++g) whole.merge(part[(size_t)g]);
+  if ((rc = check(whole))) return rc;
+  if ((rc = pool_parallel(G, [&](int g) {
+         return first(g) == first(g + 1) ? SWB200_OK : run(g_pool.ctx[(size_t)g], first(g), first(g + 1), part[(size_t)g], whole);
+       }))) return rc;
+  // what the call ran: cells and launches summed over the GPUs (a device left without pairs ran nothing), the longest
+  // device time, everything else as device 0 ran it
+  swb200_run_info& info = g_pool.info;
+  info = g_pool.ctx[0]->info;
+  info.cells = 0; info.engine_launches = 0; info.aux_launches = 0; info.engine_ms = 0;
+  for (int g = 0; g < G && first(g) < npairs; ++g) {
+    const swb200_run_info& gi = g_pool.ctx[(size_t)g]->info;
+    info.cells += gi.cells; info.engine_launches += gi.engine_launches; info.aux_launches += gi.aux_launches;
+    info.engine_ms = std::max(info.engine_ms, gi.engine_ms);
+  }
+  g_pool.info_valid = true;
+  return SWB200_OK;
+}
+
 }  // namespace
 
 static int score_pair_on_pool(const unsigned char* seq1, long long n, const unsigned char* seq2, long long m,
@@ -1994,44 +2037,30 @@ static int score_pair_on_pool(const unsigned char* seq1, long long n, const unsi
   return handled ? SWB200_OK : 1;
 }
 
-static int score_batch_host(const unsigned char* seq1_all, const long long* off1, const int* len1,
-                            const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
-                            const swb200_params* p, const swb200_options* opt, int banded, int band_lo, int band_hi,
-                            int* scores_out) {
-  {
-    std::unique_lock<std::mutex> pl(g_pool.mu);
-    const int G = (int)g_pool.ctx.size();
-    if (G > 1 && npairs >= 2LL * G) {
-      // contiguous ranges of pairs, one per GPU (SURVEY.md 8e: pair_id / ceil(P / G)); no data-path communication
-      const long long per = (npairs + G - 1) / G;
-      int rc = pool_parallel(G, [&](int g) -> int {
-        const long long k0 = std::min<long long>(npairs, (long long)g * per), k1 = std::min<long long>(npairs, k0 + per);
-        return score_batch_host_ctx(g_pool.ctx[(size_t)g], seq1_all, off1 + k0, len1 + k0, seq2_all, off2 + k0, len2 + k0, k1 - k0, p, opt,
-                                    banded, band_lo, band_hi, scores_out + k0);
+// swb200_score_batch / swb200_score_banded_batch
+static int score_batch_host(const HostPairs& in, long long npairs, const swb200_params* pp, const swb200_options* oo,
+                            int banded, int band_lo, int band_hi, int* scores_out) {
+  if (npairs < 0 || (npairs > 0 && (!in.seq1 || !in.seq2 || !in.off1 || !in.off2 || !in.len1 || !in.len2 || !scores_out)))
+    return fail(SWB200_ERR_ARG, "bad batch arguments");
+  if (npairs == 0) return SWB200_OK;
+  const swb200_params p = params_or_default(pp);
+  const swb200_options o = options_or_default(oo);
+  return run_host_batch(
+      npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); },
+      [&](const PairScan& whole) { return check_score_pairs(whole, p, banded, band_lo, band_hi); },
+      [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
+        return score_ascii_ctx(c, in.from(k0), k1 - k0, part, whole, p, o, banded, band_lo, scores_out + k0);
       });
-      if (rc) return rc;
-      g_pool.info = g_pool.ctx[0]->info;
-      g_pool.info.cells = 0; g_pool.info.engine_ms = 0; g_pool.info.engine_launches = 0; g_pool.info.aux_launches = 0;
-      for (int g = 0; g < G; ++g) {
-        const swb200_run_info& gi = g_pool.ctx[(size_t)g]->info;
-        g_pool.info.cells += gi.cells; g_pool.info.engine_ms = std::max(g_pool.info.engine_ms, gi.engine_ms);
-        g_pool.info.engine_launches += gi.engine_launches; g_pool.info.aux_launches += gi.aux_launches;
-      }
-      g_pool.info_valid = true;
-      return SWB200_OK;
-    }
-    g_pool.info_valid = false;
-  }
-  swb200_ctx* c = nullptr;
-  int rc = default_ctx(&c);
-  if (rc) return rc;
-  return score_batch_host_ctx(c, seq1_all, off1, len1, seq2_all, off2, len2, npairs, p, opt, banded, band_lo, band_hi, scores_out);
 }
 
 // ---- host batches that are ALREADY in the resident 2-bit format: a quarter of the bytes over PCIe, no pack kernel ----
 // One branch-free pass over the lengths of a packed host batch (a loop with early returns cost 1-2 ns per pair, 2-4 ms
-// per million pairs BEFORE the first copy started): maxima, sum of cells, and whether any pair breaks the rules.
-struct LenScan { int max_q = 0, max_t = 0; long long cells = 0; bool bad = false; };
+// per million pairs BEFORE the first copy started): maxima, sum of cells, and whether any pair breaks the rules
+// (a negative length; with `ordered`, a q longer than its t).
+struct LenScan {
+  int max_q = 0, max_t = 0; long long cells = 0; bool bad = false;
+  void merge(const LenScan& o) { max_q = std::max(max_q, o.max_q); max_t = std::max(max_t, o.max_t); cells += o.cells; bad |= o.bad; }
+};
 static LenScan scan_lens(const int* q_len, const int* t_len, long long k0, long long k1, bool ordered) {
   LenScan r;
   int bad = 0;
@@ -2047,25 +2076,21 @@ static LenScan scan_lens(const int* q_len, const int* t_len, long long k0, long 
   return r;
 }
 
+// One context's share of a packed host batch (arguments checked by the caller): chunks of 24 MB (banded: whole waves of
+// ~48 MB) copied on own_stream while aux_stream scores the chunk before.
 static int score_batch_packed_ctx(swb200_ctx* c, const unsigned long long* q_words, long long q_stride,
                                   const unsigned long long* t_words, long long t_stride, const int* q_len, const int* t_len,
-                                  long long npairs, int max_short, int max_long, const swb200_params* p, const swb200_options* opt,
-                                  int* scores_out, int banded = 0, int band_lo = 0, int band_hi = 0, long long cells_known = -1) {
-  if (npairs == 0) return SWB200_OK;
-  const swb200_params pv = p ? *p : swb200_params{1, -1, 1, 1};
-  const swb200_options ov = opt ? *opt : swb200_options{};
-  int rc;
-  if ((rc = check_params(pv))) return rc;
+                                  long long npairs, int max_short, int max_long, long long cells, const swb200_params& pv,
+                                  const swb200_options& ov, int banded, int band_lo, int* scores_out) {
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
   SWB_CUDA(cudaSetDevice(c->device));
   cudaStream_t sc = c->own_stream, sk = c->aux_stream;
   const size_t np = (size_t)npairs;
+  int rc;
   if ((rc = grow(c->hb_scores, c->hb_scores_cap, np, false, sc)) || (rc = grow(c->hb_qw, c->hb_qw_cap, np * q_stride, false, sc)) ||
       (rc = grow(c->hb_tw, c->hb_tw_cap, np * t_stride, false, sc)) || (rc = grow(c->hb_ql, c->hb_ql_cap, np, false, sc)) ||
       (rc = grow(c->hb_tl, c->hb_tl_cap, np, false, sc))) return rc;
-  const BatchView all{c->hb_qw, c->hb_tw, c->hb_ql, c->hb_tl, q_stride, t_stride, npairs, max_short, max_long};
-  if ((rc = banded ? check_banded_score(all, pv, 1, band_lo, band_hi) : check_batch_score(all, pv, 0))) return rc;
   const long long forced = settings().batch_chunk_bytes;
   const long long target = forced > 0 ? forced : (banded ? 48LL << 20 : 24LL << 20);   // measured: bench/batch_e2e.py, bench/banded_e2e.py
   const long long per_pair = (q_stride + t_stride) * 8 + 8;
@@ -2077,14 +2102,9 @@ static int score_batch_packed_ctx(swb200_ctx* c, const unsigned long long* q_wor
     chunk_pairs = wave * std::max<long long>(1, (target + wave * per_pair / 2) / (wave * per_pair));
   }
   const size_t nchunks = (size_t)((npairs + chunk_pairs - 1) / chunk_pairs);
-  while (c->chunk_events.size() < nchunks + 1) {
-    cudaEvent_t e;
-    SWB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    c->chunk_events.push_back(e);
-  }
+  if ((rc = chunk_events_at_least(c, nchunks + 1))) return rc;
   c->info = swb200_run_info{};
-  if (cells_known >= 0) c->info.cells = cells_known;
-  else for (long long k = 0; k < npairs; ++k) c->info.cells += (long long)q_len[k] * t_len[k];
+  c->info.cells = cells;
   bool first = true;
   for (size_t ci = 0; ci < nchunks; ++ci) {
     const long long k0 = (long long)ci * chunk_pairs, nk = std::min(chunk_pairs, npairs - k0);
@@ -2110,12 +2130,54 @@ static int score_batch_packed_ctx(swb200_ctx* c, const unsigned long long* q_wor
   return SWB200_OK;
 }
 
+// swb200_score_batch_packed / swb200_score_banded_batch_packed (banded: q = seq1 and t = seq2, in caller order)
+static int score_packed_host(const unsigned long long* q_words, long long q_stride, const unsigned long long* t_words,
+                             long long t_stride, const int* q_len, const int* t_len, long long npairs, int banded, int band_lo,
+                             int band_hi, const swb200_params* pp, const swb200_options* oo, int* scores_out) {
+  const Strides st{q_stride, t_stride}, least = batch_strides_for(0, 0, banded != 0);
+  if (npairs < 0 || q_stride < least.q || t_stride < least.t ||
+      (npairs > 0 && (!q_words || !t_words || !q_len || !t_len || !scores_out)))
+    return fail(SWB200_ERR_ARG, "bad batch arguments");
+  if (npairs == 0) return SWB200_OK;
+  const swb200_params p = params_or_default(pp);
+  const swb200_options o = options_or_default(oo);
+  return run_host_batch(
+      npairs, [&](long long k0, long long k1) { return scan_lens(q_len, t_len, k0, k1, !banded); },
+      [&](const LenScan& whole) {
+        if (whole.bad || !fits_strides(whole.max_q, whole.max_t, st, banded != 0))
+          return fail(SWB200_ERR_ARG, banded ? "pair lengths do not fit the strides"
+                                             : "pair lengths do not fit the strides (q must be the shorter sequence)");
+        int rc;
+        if ((rc = check_params(p))) return rc;
+        return banded ? check_banded_score(p, 1, band_lo, band_hi, whole.max_q, whole.max_t) : check_batch_score(p, 0, whole.max_q);
+      },
+      [&](swb200_ctx* c, long long k0, long long k1, const LenScan& part, const LenScan& whole) {
+        return score_batch_packed_ctx(c, q_words + k0 * q_stride, q_stride, t_words + k0 * t_stride, t_stride, q_len + k0,
+                                      t_len + k0, k1 - k0, whole.max_q, whole.max_t, part.cells, p, o, banded, band_lo,
+                                      scores_out + k0);
+      });
+}
+
 extern "C" {
+
+int swb200_score_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                       const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                       const swb200_params* p, const swb200_options* opt, int* scores_out) {
+  return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, 0, 0, 0, scores_out);
+}
+
+int swb200_score_banded_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                              const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                              int band_lo, int band_hi, const swb200_params* p, const swb200_options* opt,
+                              int* scores_out) {
+  if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
+  return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, 1, band_lo, band_hi, scores_out);
+}
 
 int swb200_batch_strides(int max_short, int max_long, long long* q_stride, long long* t_stride) {
   if (max_short < 0 || max_long < max_short || !q_stride || !t_stride) return fail(SWB200_ERR_ARG, "bad batch shape");
-  *q_stride = std::max(1, (max_short + 31) / 32);
-  *t_stride = std::max(1, (max_long + 31) / 32) + 2;      // +2: the kernel prefetches one word past the end
+  const Strides st = batch_strides_for(max_short, max_long, false);
+  *q_stride = st.q; *t_stride = st.t;
   return SWB200_OK;
 }
 
@@ -2139,7 +2201,7 @@ static int pack_host_range(const unsigned char* seq1_all, const long long* off1,
     const unsigned char* q = swap ? seq2_all + off2[k] : seq1_all + off1[k];
     const unsigned char* t = swap ? seq1_all + off1[k] : seq2_all + off2[k];
     const int lq = swap ? len2[k] : len1[k], lt = swap ? len1[k] : len2[k];
-    if (lq < 0 || lt < 0 || (lq + 31) / 32 + (keep_order ? 2 : 0) > q_stride || (lt + 31) / 32 + 2 > t_stride) return 1;
+    if (!fits_strides(lq, lt, Strides{q_stride, t_stride}, keep_order)) return 1;
     for (int side = 0; side < 2; ++side) {
       const unsigned char* src = side ? t : q;
       const int len = side ? lt : lq;
@@ -2210,8 +2272,8 @@ int swb200_pack_batch_host(const unsigned char* seq1_all, const long long* off1,
 // ---- banded batches in the resident format: seq1 (columns) and seq2 (rows) keep their roles ----
 int swb200_banded_strides(int max_len1, int max_len2, long long* stride1, long long* stride2) {
   if (max_len1 < 0 || max_len2 < 0 || !stride1 || !stride2) return fail(SWB200_ERR_ARG, "bad batch shape");
-  *stride1 = std::max(1, (max_len1 + 31) / 32) + 2;
-  *stride2 = std::max(1, (max_len2 + 31) / 32) + 2;
+  const Strides st = batch_strides_for(max_len1, max_len2, true);
+  *stride1 = st.q; *stride2 = st.t;
   return SWB200_OK;
 }
 
@@ -2226,87 +2288,13 @@ int swb200_pack_banded_host(const unsigned char* seq1_all, const long long* off1
 int swb200_score_banded_batch_packed(const unsigned long long* words1, long long stride1, const unsigned long long* words2,
                                      long long stride2, const int* len1, const int* len2, long long npairs, int band_lo,
                                      int band_hi, const swb200_params* p, const swb200_options* opt, int* scores_out) {
-  if (npairs < 0 || stride1 < 3 || stride2 < 3 || (npairs > 0 && (!words1 || !words2 || !len1 || !len2 || !scores_out)))
-    return fail(SWB200_ERR_ARG, "bad batch arguments");
-  if (npairs == 0) return SWB200_OK;
-  int max1 = 0, max2 = 0;
-  for (long long k = 0; k < npairs; ++k) {
-    if (len1[k] < 0 || len2[k] < 0 || (len1[k] + 31) / 32 + 2 > stride1 || (len2[k] + 31) / 32 + 2 > stride2)
-      return fail(SWB200_ERR_ARG, "pair lengths do not fit the strides");
-    max1 = std::max(max1, len1[k]); max2 = std::max(max2, len2[k]);
-  }
-  {
-    std::unique_lock<std::mutex> pl(g_pool.mu);
-    const int G = (int)g_pool.ctx.size();
-    if (G > 1 && npairs >= 2LL * G) {
-      const long long per = (npairs + G - 1) / G;
-      int rc = pool_parallel(G, [&](int g) -> int {
-        const long long k0 = std::min<long long>(npairs, (long long)g * per), k1 = std::min<long long>(npairs, k0 + per);
-        return score_batch_packed_ctx(g_pool.ctx[(size_t)g], words1 + k0 * stride1, stride1, words2 + k0 * stride2, stride2, len1 + k0,
-                                      len2 + k0, k1 - k0, max1, max2, p, opt, scores_out + k0, 1, band_lo, band_hi);
-      });
-      if (rc) return rc;
-      g_pool.info = g_pool.ctx[0]->info;
-      g_pool.info.cells = 0; g_pool.info.engine_ms = 0;
-      for (int g = 0; g < G; ++g) { g_pool.info.cells += g_pool.ctx[(size_t)g]->info.cells; g_pool.info.engine_ms = std::max(g_pool.info.engine_ms, g_pool.ctx[(size_t)g]->info.engine_ms); }
-      g_pool.info_valid = true;
-      return SWB200_OK;
-    }
-    g_pool.info_valid = false;
-  }
-  swb200_ctx* c = nullptr;
-  int rc = default_ctx(&c);
-  if (rc) return rc;
-  return score_batch_packed_ctx(c, words1, stride1, words2, stride2, len1, len2, npairs, max1, max2, p, opt, scores_out, 1, band_lo, band_hi);
+  return score_packed_host(words1, stride1, words2, stride2, len1, len2, npairs, 1, band_lo, band_hi, p, opt, scores_out);
 }
 
 int swb200_score_batch_packed(const unsigned long long* q_words, long long q_stride, const unsigned long long* t_words,
                               long long t_stride, const int* q_len, const int* t_len, long long npairs,
                               const swb200_params* p, const swb200_options* opt, int* scores_out) {
-  if (npairs < 0 || q_stride < 1 || t_stride < 3 || (npairs > 0 && (!q_words || !t_words || !q_len || !t_len || !scores_out)))
-    return fail(SWB200_ERR_ARG, "bad batch arguments");
-  if (npairs == 0) return SWB200_OK;
-  auto lens_ok = [&](const LenScan& sc) {
-    return !sc.bad && (sc.max_q + 31) / 32 <= q_stride && (sc.max_t + 31) / 32 + 2 <= t_stride;
-  };
-  const char* const lens_msg = "pair lengths do not fit the strides (q must be the shorter sequence)";
-  {
-    std::unique_lock<std::mutex> pl(g_pool.mu);
-    const int G = (int)g_pool.ctx.size();
-    if (G > 1 && npairs >= 2LL * G) {
-      const long long per = (npairs + G - 1) / G;
-      std::vector<LenScan> scans((size_t)G);
-      int rc = pool_parallel(G, [&](int g) -> int {                      // every shard's lengths scanned by its own thread
-        const long long k0 = std::min<long long>(npairs, (long long)g * per), k1 = std::min<long long>(npairs, k0 + per);
-        scans[(size_t)g] = scan_lens(q_len, t_len, k0, k1, true);
-        return SWB200_OK;
-      });
-      if (rc) return rc;
-      int max_short = 0, max_long = 0;
-      for (const LenScan& sc : scans) {
-        if (!lens_ok(sc)) return fail(SWB200_ERR_ARG, lens_msg);
-        max_short = std::max(max_short, sc.max_q); max_long = std::max(max_long, sc.max_t);
-      }
-      rc = pool_parallel(G, [&](int g) -> int {
-        const long long k0 = std::min<long long>(npairs, (long long)g * per), k1 = std::min<long long>(npairs, k0 + per);
-        return score_batch_packed_ctx(g_pool.ctx[(size_t)g], q_words + k0 * q_stride, q_stride, t_words + k0 * t_stride, t_stride, q_len + k0,
-                                      t_len + k0, k1 - k0, max_short, max_long, p, opt, scores_out + k0, 0, 0, 0, scans[(size_t)g].cells);
-      });
-      if (rc) return rc;
-      g_pool.info = g_pool.ctx[0]->info;
-      g_pool.info.cells = 0; g_pool.info.engine_ms = 0;
-      for (int g = 0; g < G; ++g) { g_pool.info.cells += g_pool.ctx[(size_t)g]->info.cells; g_pool.info.engine_ms = std::max(g_pool.info.engine_ms, g_pool.ctx[(size_t)g]->info.engine_ms); }
-      g_pool.info_valid = true;
-      return SWB200_OK;
-    }
-    g_pool.info_valid = false;
-  }
-  const LenScan sc = scan_lens(q_len, t_len, 0, npairs, true);
-  if (!lens_ok(sc)) return fail(SWB200_ERR_ARG, lens_msg);
-  swb200_ctx* c = nullptr;
-  int rc = default_ctx(&c);
-  if (rc) return rc;
-  return score_batch_packed_ctx(c, q_words, q_stride, t_words, t_stride, q_len, t_len, npairs, sc.max_q, sc.max_t, p, opt, scores_out, 0, 0, 0, sc.cells);
+  return score_packed_host(q_words, q_stride, t_words, t_stride, q_len, t_len, npairs, 0, 0, 0, p, opt, scores_out);
 }
 
 }  // extern "C"
@@ -2395,7 +2383,11 @@ int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, co
     if (err & swb::kAlignErrStart) return fail(SWB200_ERR_CUDA, "internal: anchored pass does not reproduce the score");
     if (err & swb::kAlignErrTrace) return fail(SWB200_ERR_CUDA, "internal: the traceback pass does not reproduce the score");
     if (err) return fail(SWB200_ERR_CUDA, "internal: the alignment does not re-score to the score");
-    if (npend == 0) { info->cells += (long long)h[2]; return SWB200_OK; }
+    if (npend == 0) {
+      info->cells += (long long)h[2];
+      info->lanes = 32; info->config = 300; info->rows = swb::kAlignStrip;
+      return SWB200_OK;
+    }
     // rectangles larger than a slot: the pool, emptied for every round; its first taker always fits
     const size_t need = (size_t)std::max(kAlignPoolWords, swb::align_dir_words(v.max_long, v.max_short));
     if ((rc = grow(c->ab_pool, c->ab_pool_cap, need, false, s))) return rc;
@@ -2412,82 +2404,28 @@ int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, co
 
 }  // namespace
 
-// One context's share of a host batch alignment (arguments checked by the caller).  Copy and pack in chunks as
-// score_batch_host_ctx does, then the passes over the whole range, then the outputs back.
-static int align_batch_host_ctx(swb200_ctx* c, const unsigned char* seq1_all, const long long* off1, const int* len1,
-                                const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
-                                const swb200_params& pv, int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride,
+// One context's share of a host batch alignment (arguments checked by the caller): the copy/pack pipeline of the score
+// calls, then the passes over the whole range, then the outputs back.
+static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part, const PairScan& whole,
+                                const swb200_params& p, int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride,
                                 int* ops_count) {
-  if (npairs == 0) return SWB200_OK;
-  long long bytes1 = 0, bytes2 = 0, base1 = LLONG_MAX, base2 = LLONG_MAX;
-  int max_short = 0, max_long = 0;
-  for (long long k = 0; k < npairs; ++k) {
-    const int a = len1[k], b = len2[k];
-    bytes1 = std::max(bytes1, off1[k] + a); bytes2 = std::max(bytes2, off2[k] + b);
-    base1 = std::min(base1, off1[k]); base2 = std::min(base2, off2[k]);
-    max_short = std::max(max_short, std::min(a, b)); max_long = std::max(max_long, std::max(a, b));
-  }
-  base1 &= ~15LL; base2 &= ~15LL;
-  bytes1 -= base1; bytes2 -= base2;
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
   SWB_CUDA(cudaSetDevice(c->device));
   cudaStream_t sc = c->own_stream, sk = c->aux_stream;
   const size_t np = (size_t)npairs;
-  const long long q_stride = std::max(1, (max_short + 31) / 32);
-  const long long t_stride = std::max(1, (max_long + 31) / 32) + 2;
   int rc;
-  if ((rc = grow(c->hb_seq1, c->hb_seq1_cap, (size_t)bytes1 + 16, false, sc)) || (rc = grow(c->hb_seq2, c->hb_seq2_cap, (size_t)bytes2 + 16, false, sc)) ||
-      (rc = grow(c->hb_off1, c->hb_off1_cap, np, false, sc)) || (rc = grow(c->hb_off2, c->hb_off2_cap, np, false, sc)) ||
-      (rc = grow(c->hb_len1, c->hb_len1_cap, np, false, sc)) || (rc = grow(c->hb_len2, c->hb_len2_cap, np, false, sc)) ||
-      (rc = grow(c->hb_scores, c->hb_scores_cap, np, false, sc)) || (rc = grow(c->hb_spans, c->hb_spans_cap, 4 * np, false, sc)) ||
-      (rc = grow(c->hb_ops, c->hb_ops_cap, np * (size_t)ops_stride, false, sc)) || (rc = grow(c->hb_opsn, c->hb_opsn_cap, np, false, sc)) ||
-      (rc = grow(c->hb_qw, c->hb_qw_cap, np * q_stride, false, sc)) || (rc = grow(c->hb_tw, c->hb_tw_cap, np * t_stride, false, sc)) ||
-      (rc = grow(c->hb_ql, c->hb_ql_cap, np, false, sc)) || (rc = grow(c->hb_tl, c->hb_tl_cap, np, false, sc))) return rc;
+  if ((rc = grow(c->hb_spans, c->hb_spans_cap, 4 * np, false, sc)) ||
+      (rc = grow(c->hb_ops, c->hb_ops_cap, np * (size_t)ops_stride, false, sc)) || (rc = grow(c->hb_opsn, c->hb_opsn_cap, np, false, sc))) return rc;
   c->info = swb200_run_info{};
-  SWB_CUDA(cudaMemsetAsync(c->d_result, 0, 10 * sizeof(int), sc));
-  SWB_CUDA(cudaMemcpyAsync(c->hb_off1, off1, np * sizeof(long long), cudaMemcpyHostToDevice, sc));
-  SWB_CUDA(cudaMemcpyAsync(c->hb_off2, off2, np * sizeof(long long), cudaMemcpyHostToDevice, sc));
-  SWB_CUDA(cudaMemcpyAsync(c->hb_len1, len1, np * sizeof(int), cudaMemcpyHostToDevice, sc));
-  SWB_CUDA(cudaMemcpyAsync(c->hb_len2, len2, np * sizeof(int), cudaMemcpyHostToDevice, sc));
-  // chunks of ~48 MB of sequence: own_stream copies chunk k+1 while aux_stream packs chunk k
-  size_t ci = 0;
-  bool first = true;
-  const long long forced = settings().batch_chunk_bytes;
-  const long long target = forced > 0 ? forced : 48LL << 20, min_pairs = forced > 0 ? 1 : 1024;
-  long long k0 = 0, acc = 0, lo1 = LLONG_MAX, hi1 = 0, lo2 = LLONG_MAX, hi2 = 0;
-  for (long long k = 0; k < npairs; ++k) {
-    lo1 = std::min(lo1, off1[k]); hi1 = std::max(hi1, off1[k] + len1[k]);
-    lo2 = std::min(lo2, off2[k]); hi2 = std::max(hi2, off2[k] + len2[k]);
-    acc += (long long)len1[k] + len2[k];
-    if (!((acc >= target && k + 1 - k0 >= min_pairs) || k + 1 == npairs)) continue;
-    while (c->chunk_events.size() < ci + 1) {
-      cudaEvent_t e;
-      SWB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      c->chunk_events.push_back(e);
-    }
-    if (hi1 > lo1) SWB_CUDA(cudaMemcpyAsync(c->hb_seq1 + (lo1 - base1), seq1_all + lo1, (size_t)(hi1 - lo1), cudaMemcpyHostToDevice, sc));
-    if (hi2 > lo2) SWB_CUDA(cudaMemcpyAsync(c->hb_seq2 + (lo2 - base2), seq2_all + lo2, (size_t)(hi2 - lo2), cudaMemcpyHostToDevice, sc));
-    SWB_CUDA(cudaEventRecord(c->chunk_events[ci], sc));
-    SWB_CUDA(cudaStreamWaitEvent(sk, c->chunk_events[ci], 0));
-    ci += 1;
-    if (first) { SWB_CUDA(cudaEventRecord(c->ev0, sk)); first = false; }
-    const long long nk = k + 1 - k0;
-    const int blocks = (int)std::min<long long>((nk * (q_stride + t_stride) + 255) / 256, 64LL * c->sms);
-    swb::launch_pack_batch(c->hb_seq1 - base1, c->hb_off1 + k0, c->hb_len1 + k0, c->hb_seq2 - base2, c->hb_off2 + k0, c->hb_len2 + k0, nk,
-                           q_stride, t_stride, c->hb_qw + k0 * q_stride, c->hb_tw + k0 * t_stride, c->hb_ql + k0, c->hb_tl + k0, 0,
-                           c->d_result, blocks, sk);
-    SWB_CUDA(cudaGetLastError());
-    c->info.aux_launches += 1;
-    k0 = k + 1; acc = 0; lo1 = LLONG_MAX; hi1 = 0; lo2 = LLONG_MAX; hi2 = 0;
-  }
+  BatchView v;
+  if ((rc = stage_and_pack_locked(c, h, npairs, part, whole, false, &v, nullptr))) return rc;
   SWB_CUDA(cudaMemcpyAsync(c->h_result, c->d_result, 2 * sizeof(int), cudaMemcpyDeviceToHost, sk));
   SWB_CUDA(cudaStreamSynchronize(sk));
   SWB_CUDA(cudaStreamSynchronize(sc));
   if (c->h_result[1] & swb::STATUS_BAD_SYMBOL) return fail(SWB200_ERR_ALPHABET, "batch input contains bytes other than A,C,G,T");
-  const BatchView v{c->hb_qw, c->hb_tw, c->hb_ql, c->hb_tl, q_stride, t_stride, npairs, max_short, max_long};
   SWB_CUDA(cudaMemsetAsync(c->hb_ops, 0, np * (size_t)ops_stride * sizeof(uint32_t), sk));   // overflowed pairs come back as zeros
-  if ((rc = align_packed_locked(c, v, c->hb_len1, pv, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info))) return rc;
+  if ((rc = align_packed_locked(c, v, c->hb_len1, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info))) return rc;
   SWB_CUDA(cudaEventRecord(c->ev1, sk));
   SWB_CUDA(cudaMemcpyAsync(scores_out, c->hb_scores, np * sizeof(int), cudaMemcpyDeviceToHost, sk));
   SWB_CUDA(cudaMemcpyAsync(spans_out, c->hb_spans, 4 * np * sizeof(int), cudaMemcpyDeviceToHost, sk));
@@ -2497,59 +2435,33 @@ static int align_batch_host_ctx(swb200_ctx* c, const unsigned char* seq1_all, co
   float ms = 0;
   SWB_CUDA(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
   c->info.engine_ms = ms;          // first pack to the last trace round
-  c->info.lanes = 32; c->info.config = 300; c->info.rows = swb::kAlignStrip;
   return SWB200_OK;
 }
 
 extern "C" {
 
 int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, const int* len1, const unsigned char* seq2_all,
-                       const long long* off2, const int* len2, long long npairs, const swb200_params* p, const swb200_options* opt,
+                       const long long* off2, const int* len2, long long npairs, const swb200_params* pp, const swb200_options* opt,
                        int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride, int* ops_count) {
   (void)opt;
   if (npairs < 0 || ops_stride < 1 ||
       (npairs > 0 && (!seq1_all || !seq2_all || !off1 || !off2 || !len1 || !len2 || !scores_out || !spans_out || !ops_out || !ops_count)))
     return fail(SWB200_ERR_ARG, "bad batch arguments");
-  const swb200_params pv = p ? *p : swb200_params{1, -1, 1, 1};
-  int rc;
-  {
-    long long neg = 0;
-    int mxmin = 0;
-    for (long long k = 0; k < npairs; ++k) {
-      neg |= (long long)(len1[k] | len2[k]) | off1[k] | off2[k];
-      mxmin = std::max(mxmin, std::min(len1[k], len2[k]));
-    }
-    if (neg < 0) return fail(SWB200_ERR_ARG, "negative length or offset");
-    if ((rc = check_params(pv)) || (rc = check_align_batch_limits(pv, mxmin))) return rc;
-  }
-  if (npairs == 0) return SWB200_OK;
-  {
-    std::unique_lock<std::mutex> pl(g_pool.mu);
-    const int G = (int)g_pool.ctx.size();
-    if (G > 1 && npairs >= 2LL * G) {
-      // contiguous ranges of pairs, one per GPU, as swb200_score_batch
-      const long long per = (npairs + G - 1) / G;
-      rc = pool_parallel(G, [&](int g) -> int {
-        const long long k0 = std::min<long long>(npairs, (long long)g * per), k1 = std::min<long long>(npairs, k0 + per);
-        return align_batch_host_ctx(g_pool.ctx[(size_t)g], seq1_all, off1 + k0, len1 + k0, seq2_all, off2 + k0, len2 + k0, k1 - k0, pv,
-                                    scores_out + k0, spans_out + 4 * k0, ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
+  const swb200_params p = params_or_default(pp);
+  const HostPairs in{seq1_all, off1, len1, seq2_all, off2, len2};
+  auto check = [&](const PairScan& whole) {
+    if (whole.neg < 0) return fail(SWB200_ERR_ARG, "negative length or offset");
+    int rc;
+    if ((rc = check_params(p))) return rc;
+    return check_align_batch_limits(p, whole.max_min);
+  };
+  if (npairs == 0) return check(PairScan{});
+  return run_host_batch(
+      npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
+      [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, scores_out + k0, spans_out + 4 * k0,
+                                    ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
       });
-      if (rc) return rc;
-      g_pool.info = g_pool.ctx[0]->info;
-      g_pool.info.cells = 0; g_pool.info.engine_ms = 0; g_pool.info.engine_launches = 0; g_pool.info.aux_launches = 0;
-      for (int g = 0; g < G; ++g) {
-        const swb200_run_info& gi = g_pool.ctx[(size_t)g]->info;
-        g_pool.info.cells += gi.cells; g_pool.info.engine_ms = std::max(g_pool.info.engine_ms, gi.engine_ms);
-        g_pool.info.engine_launches += gi.engine_launches; g_pool.info.aux_launches += gi.aux_launches;
-      }
-      g_pool.info_valid = true;
-      return SWB200_OK;
-    }
-    g_pool.info_valid = false;
-  }
-  swb200_ctx* c = nullptr;
-  if ((rc = default_ctx(&c))) return rc;
-  return align_batch_host_ctx(c, seq1_all, off1, len1, seq2_all, off2, len2, npairs, pv, scores_out, spans_out, ops_out, ops_stride, ops_count);
 }
 
 int swb200_batch_align(swb200_batch* b, const swb200_params* pp, const swb200_options* opt, void* stream, int* d_scores,
@@ -2558,25 +2470,12 @@ int swb200_batch_align(swb200_batch* b, const swb200_params* pp, const swb200_op
   if (!b || ops_stride < 1 || (b->npairs > 0 && (!d_scores || !d_spans || !d_ops || !d_ops_count)))
     return fail(SWB200_ERR_ARG, "bad batch arguments");
   if (b->keep_order || !b->len1) return fail(SWB200_ERR_ARG, "batch was packed in caller order (banded); re-pack with keep_order=0");
-  const swb200_params p = pp ? *pp : swb200_params{1, -1, 1, 1};
+  const swb200_params p = params_or_default(pp);
   int rc;
   if ((rc = check_params(p)) || (rc = check_align_batch_limits(p, b->max_short))) return rc;
-  swb200_ctx* c = b->ctx;
-  std::lock_guard<std::mutex> lk(c->mu);
-  DeviceGuard guard;
-  SWB_CUDA(cudaSetDevice(c->device));
-  cudaStream_t s = (cudaStream_t)stream;
-  c->info = swb200_run_info{};
-  if (b->npairs == 0) return SWB200_OK;
-  SWB_CUDA(cudaEventRecord(c->ev0, s));
-  if ((rc = align_packed_locked(c, whole_batch(b), b->len1, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info))) return rc;
-  SWB_CUDA(cudaEventRecord(c->ev1, s));
-  SWB_CUDA(cudaStreamSynchronize(s));
-  float ms = 0;
-  SWB_CUDA(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-  c->info.engine_ms = ms;
-  c->info.lanes = 32; c->info.config = 300; c->info.rows = swb::kAlignStrip;
-  return SWB200_OK;
+  return run_device_batch(b, 0, stream, [&](swb200_ctx* c, cudaStream_t s) {
+    return align_packed_locked(c, whole_batch(b), b->len1, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info);
+  });
 }
 
 }  // extern "C"

@@ -91,8 +91,10 @@ SWB200_API int swb200_plan(long long n, long long m, const swb200_params* p, con
  * the HOST-buffer entry points below (and therefore the four legacy names) use devices 0 .. G-1:
  *   - a pair with at least "ring_min_cells" cells (swb200_configure) is spread over an in-process ring of the G
  *     GPUs (one host thread per GPU for the duration of the call, peer access over NVLink, swept from both ends);
- *   - swb200_score_batch / swb200_score_banded_batch cut the batch into G contiguous ranges of pairs, one
- *     copy/compute pipeline per GPU, no communication.
+ *   - the host batch calls (swb200_score_batch, swb200_score_banded_batch, swb200_score_batch_packed,
+ *     swb200_score_banded_batch_packed, swb200_align_batch) cut the batch into G contiguous ranges of pairs, one
+ *     copy/compute pipeline per GPU, no communication; swb200_last_run(NULL, ..) then reports cells and launches summed
+ *     over the GPUs and the longest device time.
  * Results are identical for every G.  count 0 or 1 = one GPU (the default).  Needs peer access between the devices. */
 SWB200_API int swb200_set_devices(int count);
 SWB200_API int swb200_get_devices(void);
@@ -178,7 +180,9 @@ SWB200_API int swb200_last_run(swb200_ctx* ctx, swb200_run_info* info);
  * npairs independent pairs in one kernel, several pairs per warp, nothing leaving the registers.
  * Pair k is seq1_all[off1[k] .. off1[k]+len1[k]) vs seq2_all[off2[k] .. off2[k]+len2[k]).
  * Limits: bytes must be A,C,G,T; min(len1[k], len2[k]) <= 1024 and match*min(len) <= 32766 - match for every
- * pair (SWB200_ERR_RANGE otherwise; such pairs: swb200_score).  Empty sequences score 0. */
+ * pair (SWB200_ERR_RANGE otherwise; such pairs: swb200_score).  Empty sequences score 0.
+ * Every host batch call (HOST buffers, here and below) checks its arguments, lengths, parameters and these limits before
+ * it touches a device, so a bad call fails with SWB200_ERR_ARG / SWB200_ERR_RANGE on any machine. */
 SWB200_API int swb200_score_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
                                   const unsigned char* seq2_all, const long long* off2, const int* len2,
                                   long long npairs, const swb200_params* p, const swb200_options* opt,
