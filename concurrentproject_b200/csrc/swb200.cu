@@ -12,6 +12,7 @@
 #include "swb_batch.cuh"
 #include "swb_banded.cuh"
 #include "swb_align_batch.cuh"
+#include "swb_align_banded.cuh"
 
 #include <cstdio>
 #include <cstdlib>
@@ -2347,6 +2348,35 @@ int check_align_batch_limits(const swb200_params& p, int max_short) {
   return SWB200_OK;
 }
 
+// The trace rounds of both batch alignments, after their first trace launch on stream s: one sync per round reads the
+// error bits and the pending count; an error fails the call, nothing pending ends it; otherwise the pool gets room for
+// pool_need 64-bit words and is emptied, and relaunch(todo, ntodo, pending) runs the pending pairs again.
+int align_rounds_locked(swb200_ctx* c, cudaStream_t s, long long npairs, size_t pool_need, swb200_run_info* info,
+                        const std::function<void(const int* todo, int ntodo, int* pending)>& relaunch) {
+  int rc;
+  for (int cur = 0;;) {
+    unsigned long long h[3] = {0, 0, 0};
+    SWB_CUDA(cudaMemcpyAsync(h, c->ab_misc, sizeof h, cudaMemcpyDeviceToHost, s));
+    SWB_CUDA(cudaStreamSynchronize(s));
+    const int err = (int)(uint32_t)h[0], npend = (int)(h[0] >> 32);
+    if (err & swb::kAlignErrStart) return fail(SWB200_ERR_CUDA, "internal: anchored pass does not reproduce the score");
+    if (err & swb::kAlignErrTrace) return fail(SWB200_ERR_CUDA, "internal: the traceback pass does not reproduce the score");
+    if (err) return fail(SWB200_ERR_CUDA, "internal: the alignment does not re-score to the score");
+    if (npend == 0) {
+      info->cells += (long long)h[2];
+      return SWB200_OK;
+    }
+    // the pool's first taker always fits (pool_need covers the largest rectangle)
+    if ((rc = grow(c->ab_pool, c->ab_pool_cap, pool_need, false, s))) return rc;
+    const int* todo = c->ab_list + (size_t)cur * npairs;
+    cur ^= 1;
+    SWB_CUDA(cudaMemsetAsync(c->ab_misc, 0, 2 * sizeof(unsigned long long), s));
+    relaunch(todo, npend, c->ab_list + (size_t)cur * npairs);
+    SWB_CUDA(cudaGetLastError());
+    info->engine_launches += 1;
+  }
+}
+
 // Passes 1-3 and the walk over a packed range (shorter sequence first, len1 = the caller's seq1 lengths), everything on
 // stream s of c's device.  Synchronises once per trace round (the pending count decides whether another round runs).
 int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, const swb200_params& p, cudaStream_t s,
@@ -2375,40 +2405,73 @@ int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, co
   swb::launch_align_trace(P, (int)blocks, s);
   SWB_CUDA(cudaGetLastError());
   info->engine_launches += 2;
-  for (int cur = 0;;) {
-    unsigned long long h[3] = {0, 0, 0};
-    SWB_CUDA(cudaMemcpyAsync(h, c->ab_misc, sizeof h, cudaMemcpyDeviceToHost, s));
-    SWB_CUDA(cudaStreamSynchronize(s));
-    const int err = (int)(uint32_t)h[0], npend = (int)(h[0] >> 32);
-    if (err & swb::kAlignErrStart) return fail(SWB200_ERR_CUDA, "internal: anchored pass does not reproduce the score");
-    if (err & swb::kAlignErrTrace) return fail(SWB200_ERR_CUDA, "internal: the traceback pass does not reproduce the score");
-    if (err) return fail(SWB200_ERR_CUDA, "internal: the alignment does not re-score to the score");
-    if (npend == 0) {
-      info->cells += (long long)h[2];
-      info->lanes = 32; info->config = 300; info->rows = swb::kAlignStrip;
-      return SWB200_OK;
-    }
-    // rectangles larger than a slot: the pool, emptied for every round; its first taker always fits
-    const size_t need = (size_t)std::max(kAlignPoolWords, swb::align_dir_words(v.max_long, v.max_short));
-    if ((rc = grow(c->ab_pool, c->ab_pool_cap, need, false, s))) return rc;
-    P.pool = c->ab_pool; P.pool_words = (long long)c->ab_pool_cap;
-    P.todo = c->ab_list + (size_t)cur * v.npairs; P.ntodo = npend;
-    cur ^= 1;
-    P.pending = c->ab_list + (size_t)cur * v.npairs;
-    SWB_CUDA(cudaMemsetAsync(c->ab_misc, 0, 2 * sizeof(unsigned long long), s));
-    swb::launch_align_trace(P, (int)std::max(1LL, std::min<long long>(blocks, (npend + 255) / 256)), s);
-    SWB_CUDA(cudaGetLastError());
-    info->engine_launches += 1;
-  }
+  // rectangles larger than a slot: the pool, emptied for every round; its first taker always fits
+  const size_t need = (size_t)std::max(kAlignPoolWords, swb::align_dir_words(v.max_long, v.max_short));
+  if ((rc = align_rounds_locked(c, s, v.npairs, need, info, [&](const int* todo, int ntodo, int* pending) {
+         P.pool = c->ab_pool; P.pool_words = (long long)c->ab_pool_cap;
+         P.todo = todo; P.ntodo = ntodo; P.pending = pending;
+         swb::launch_align_trace(P, (int)std::max(1LL, std::min<long long>(blocks, (ntodo + 255) / 256)), s);
+       }))) return rc;
+  info->lanes = 32; info->config = 300; info->rows = swb::kAlignStrip;
+  return SWB200_OK;
+}
+
+constexpr long long kBandSlotWords = 32LL * 3072;  // direction slot per warp: 384 KB, spans with len1 + len2 < 24 568 (cfg5: ~20 000)
+constexpr int kBandCtasPerSm = 8;                  // 32 resident warps per SM: enough to hide the shuffle chain of a step
+
+// Passes 1-3 and the walk over a packed range in caller order (q = seq1, t = seq2), everything on stream s of c's device:
+// one warp per pair, the trace rounds of align_rounds_locked.  Direction slots: kBandSlotWords per launched warp.
+int align_banded_packed_locked(swb200_ctx* c, const BatchView& v, int band_lo, const swb200_params& p, cudaStream_t s,
+                               int* d_scores, int* d_spans, uint32_t* d_ops, int ops_stride, int* d_ops_count,
+                               swb200_run_info* info) {
+  if (v.npairs == 0) return SWB200_OK;
+  constexpr int W = swb::kBandAlignWarps;
+  int per_sm = 0;
+  SWB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, swb::align_banded_trace_kernel_ptr(), 32 * W, 0));
+  per_sm = std::max(1, std::min(per_sm, kBandCtasPerSm));
+  const long long blocks = std::max(1LL, std::min<long long>((v.npairs + W - 1) / W, (long long)c->sms * per_sm));
+  const long long nw = blocks * W;
+  int rc;
+  if ((rc = grow(c->ab_slot, c->ab_slot_cap, (size_t)(kBandSlotWords * nw + 1) / 2, false, s)) ||
+      (rc = grow(c->ab_list, c->ab_list_cap, 2 * (size_t)v.npairs, false, s)) ||
+      (rc = grow(c->ab_misc, c->ab_misc_cap, 4, false, s))) return rc;
+  SWB_CUDA(cudaMemsetAsync(c->ab_misc, 0, 3 * sizeof(unsigned long long), s));
+  swb::AlignBandedParams P{};
+  P.a_words = v.q_words; P.b_words = v.t_words; P.a_len = v.q_len; P.b_len = v.t_len;
+  P.a_stride = v.q_stride; P.b_stride = v.t_stride; P.npairs = v.npairs; P.band_lo = band_lo;
+  P.match = p.match; P.mismatch = p.mismatch; P.gap_init = p.gap_init; P.gap_ext = p.gap_ext;
+  P.scores = d_scores; P.spans = d_spans; P.nwarps = nw;
+  P.slot = reinterpret_cast<uint32_t*>(c->ab_slot); P.slot_words = kBandSlotWords;
+  P.pool = reinterpret_cast<uint32_t*>(c->ab_pool); P.pool_words = 2 * (long long)c->ab_pool_cap;
+  P.pool_used = c->ab_misc + 1;
+  P.todo = nullptr; P.ntodo = v.npairs;
+  P.pending = c->ab_list; P.npending = reinterpret_cast<int*>(c->ab_misc) + 1;
+  P.ops = d_ops; P.ops_stride = ops_stride; P.ops_count = d_ops_count;
+  P.err = reinterpret_cast<int*>(c->ab_misc); P.cells = c->ab_misc + 2;
+  swb::launch_align_banded_span(P, (int)blocks, s);
+  swb::launch_align_banded_trace(P, (int)blocks, s);
+  SWB_CUDA(cudaGetLastError());
+  info->engine_launches += 2;
+  // spans larger than a slot: the pool (64-bit words here), sized for the largest span the batch can have
+  const size_t need = (size_t)std::max(kAlignPoolWords, (swb::band_dir_words(v.max_short, v.max_long) + 1) / 2);
+  if ((rc = align_rounds_locked(c, s, v.npairs, need, info, [&](const int* todo, int ntodo, int* pending) {
+         P.pool = reinterpret_cast<uint32_t*>(c->ab_pool); P.pool_words = 2 * (long long)c->ab_pool_cap;
+         P.todo = todo; P.ntodo = ntodo; P.pending = pending;
+         swb::launch_align_banded_trace(P, (int)std::max(1LL, std::min<long long>(blocks, (ntodo + W - 1) / W)), s);
+       }))) return rc;
+  info->lanes = 32; info->config = 310; info->rows = 0; info->bands = swb::kBandWidth;
+  info->ctas = (int)blocks; info->warps = (int)nw;
+  return SWB200_OK;
 }
 
 }  // namespace
 
 // One context's share of a host batch alignment (arguments checked by the caller): the copy/pack pipeline of the score
-// calls, then the passes over the whole range, then the outputs back.
+// calls, then the passes over the whole range, then the outputs back.  banded: the pairs stay in caller order and the
+// banded passes run with band band_lo .. band_lo + 63.
 static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part, const PairScan& whole,
-                                const swb200_params& p, int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride,
-                                int* ops_count) {
+                                const swb200_params& p, bool banded, int band_lo, int* scores_out, int* spans_out,
+                                unsigned int* ops_out, int ops_stride, int* ops_count) {
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
   SWB_CUDA(cudaSetDevice(c->device));
@@ -2419,13 +2482,15 @@ static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npa
       (rc = grow(c->hb_ops, c->hb_ops_cap, np * (size_t)ops_stride, false, sc)) || (rc = grow(c->hb_opsn, c->hb_opsn_cap, np, false, sc))) return rc;
   c->info = swb200_run_info{};
   BatchView v;
-  if ((rc = stage_and_pack_locked(c, h, npairs, part, whole, false, &v, nullptr))) return rc;
+  if ((rc = stage_and_pack_locked(c, h, npairs, part, whole, banded, &v, nullptr))) return rc;
   SWB_CUDA(cudaMemcpyAsync(c->h_result, c->d_result, 2 * sizeof(int), cudaMemcpyDeviceToHost, sk));
   SWB_CUDA(cudaStreamSynchronize(sk));
   SWB_CUDA(cudaStreamSynchronize(sc));
   if (c->h_result[1] & swb::STATUS_BAD_SYMBOL) return fail(SWB200_ERR_ALPHABET, "batch input contains bytes other than A,C,G,T");
   SWB_CUDA(cudaMemsetAsync(c->hb_ops, 0, np * (size_t)ops_stride * sizeof(uint32_t), sk));   // overflowed pairs come back as zeros
-  if ((rc = align_packed_locked(c, v, c->hb_len1, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info))) return rc;
+  rc = banded ? align_banded_packed_locked(c, v, band_lo, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info)
+              : align_packed_locked(c, v, c->hb_len1, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info);
+  if (rc) return rc;
   SWB_CUDA(cudaEventRecord(c->ev1, sk));
   SWB_CUDA(cudaMemcpyAsync(scores_out, c->hb_scores, np * sizeof(int), cudaMemcpyDeviceToHost, sk));
   SWB_CUDA(cudaMemcpyAsync(spans_out, c->hb_spans, 4 * np * sizeof(int), cudaMemcpyDeviceToHost, sk));
@@ -2459,7 +2524,7 @@ int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, con
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, scores_out + k0, spans_out + 4 * k0,
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, false, 0, scores_out + k0, spans_out + 4 * k0,
                                     ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
       });
 }
@@ -2475,6 +2540,40 @@ int swb200_batch_align(swb200_batch* b, const swb200_params* pp, const swb200_op
   if ((rc = check_params(p)) || (rc = check_align_batch_limits(p, b->max_short))) return rc;
   return run_device_batch(b, 0, stream, [&](swb200_ctx* c, cudaStream_t s) {
     return align_packed_locked(c, whole_batch(b), b->len1, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info);
+  });
+}
+
+int swb200_align_banded_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                              const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                              int band_lo, int band_hi, const swb200_params* pp, const swb200_options* opt, int* scores_out,
+                              int* spans_out, unsigned int* ops_out, int ops_stride, int* ops_count) {
+  (void)opt;
+  if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
+  if (npairs < 0 || ops_stride < 1 ||
+      (npairs > 0 && (!seq1_all || !seq2_all || !off1 || !off2 || !len1 || !len2 || !scores_out || !spans_out || !ops_out || !ops_count)))
+    return fail(SWB200_ERR_ARG, "bad batch arguments");
+  const swb200_params p = params_or_default(pp);
+  const HostPairs in{seq1_all, off1, len1, seq2_all, off2, len2};
+  auto check = [&](const PairScan& whole) { return check_score_pairs(whole, p, 1, band_lo, band_hi); };
+  if (npairs == 0) return check(PairScan{});
+  return run_host_batch(
+      npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
+      [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, true, band_lo, scores_out + k0, spans_out + 4 * k0,
+                                    ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
+      });
+}
+
+int swb200_batch_align_banded(swb200_batch* b, int band_lo, int band_hi, const swb200_params* pp, const swb200_options* opt,
+                              void* stream, int* d_scores, int* d_spans, unsigned int* d_ops, int ops_stride, int* d_ops_count) {
+  (void)opt;
+  if (!b || ops_stride < 1 || (b->npairs > 0 && (!d_scores || !d_spans || !d_ops || !d_ops_count)))
+    return fail(SWB200_ERR_ARG, "bad batch arguments");
+  const swb200_params p = params_or_default(pp);
+  int rc;
+  if ((rc = check_params(p)) || (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
+  return run_device_batch(b, 0, stream, [&](swb200_ctx* c, cudaStream_t s) {
+    return align_banded_packed_locked(c, whole_batch(b), band_lo, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info);
   });
 }
 

@@ -270,6 +270,34 @@ SWB200_API int swb200_score_banded_batch(const unsigned char* seq1_all, const lo
 SWB200_API int swb200_batch_score_banded(swb200_batch* batch, int band_lo, int band_hi, const swb200_params* p,
                                          const swb200_options* opt, void* stream, int* d_scores);
 
+/* Banded batch alignment: score, span and CIGAR of the best local alignment all of whose cells lie in the band B
+ * (band_lo <= j - i <= band_hi; every aligned pair and every gap position counts as a cell).  For every pair k:
+ *   score      exactly swb200_score_banded_batch's (oracle_gotoh_banded);
+ *   end cell   among in-band cells holding the score, the smallest j, then the smallest i;
+ *   start cell the anchored recurrence over the reversed prefixes seq1[..j_end], seq2[..i_end], cells outside the
+ *              mirrored band (j_end - i_end) - band_hi .. (j_end - i_end) - band_lo unreachable; ties to the largest
+ *              j_start, then the largest i_start;
+ *   operations the anchored recurrence over the span rectangle inside B, 4 direction bits per cell (diagonal before E
+ *              before F; a gap extends only where extending is strictly better than opening), walked back from the end
+ *              cell.  Every cell of the walk lies in B.
+ * Output format, '='/'X' split, ops_stride overflow (ops_count = -n; the host call zero-fills that slot), the "1I1I"
+ * split when gap_ext > gap_init, the device re-score and its SWB200_ERR_CUDA ("internal: ...") are swb200_align_batch's.
+ * When B covers the whole pair (band_lo <= -(len2-1), band_hi >= len1-1) the result is swb200_align_batch's.
+ * Limits and errors are swb200_score_banded_batch's: bytes A,C,G,T (SWB200_ERR_ALPHABET); band_hi == band_lo + 63
+ * (SWB200_ERR_ARG); match*min(len) <= 32766 - match (SWB200_ERR_RANGE), so every accepted pair can be checked against
+ * the score-only call.  All argument checks run before a device is touched.  One warp per pair on the device; the host
+ * call packs in chunks and shards over swb200_set_devices like swb200_align_batch.  opt is reserved (NULL). */
+SWB200_API int swb200_align_banded_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                                         const unsigned char* seq2_all, const long long* off2, const int* len2,
+                                         long long npairs, int band_lo, int band_hi, const swb200_params* p,
+                                         const swb200_options* opt, int* scores_out, int* spans_out,
+                                         unsigned int* ops_out, int ops_stride, int* ops_count);
+/* The same for a device-resident batch packed with keep_order = 1 (SWB200_ERR_ARG for keep_order = 0); every output
+ * pointer is a DEVICE pointer. */
+SWB200_API int swb200_batch_align_banded(swb200_batch* batch, int band_lo, int band_hi, const swb200_params* p,
+                                         const swb200_options* opt, void* stream, int* d_scores, int* d_spans,
+                                         unsigned int* d_ops, int ops_stride, int* d_ops_count);
+
 /* ---- seeded synthetic inputs, generated in HBM (SURVEY.md 8d) -----------------------------------------
  * The portable counter-based generator of concurrentproject_b200/rng.py and oracle/gotoh_oracle.c on the device,
  * bit-identical to both: symbol k of stream s = 2 bits of mix64(seed, s, k / 32) -> "ACGT".  Replaces the reference
