@@ -357,7 +357,10 @@ def get_devices() -> int:
 def align(seq1: Bytes, seq2: Bytes, params: Sequence[int] = DEFAULT_PARAMS):
     """(score, (i_start, j_start, i_end, j_end), cigar): the best local alignment itself (swb200_align).  The extended
     CIGAR reads from the start cell: '=' match, 'X' mismatch, 'I' a base of seq1 against a gap, 'D' a base of seq2 against
-    a gap; re-scored with MATCH / MISMATCH / G_INIT + (k-1) G_EXT per gap of length k it gives the score."""
+    a gap; re-scored with MATCH / MISMATCH / G_INIT + (k-1) G_EXT per gap of length k it gives the score.  A span whose
+    traceback directions (half a byte per cell) do not fit in device memory is traced back in blocks of rows, recomputed
+    from one stored boundary row per block: same result, about one more sweep over the span.  configure("align_block_rows",
+    K) forces blocks of K rows (a multiple of 256)."""
     a, b = _u8(seq1), _u8(seq2)
     out, need = C.c_int(0), C.c_longlong(0)
     span = (C.c_longlong * 4)()

@@ -668,7 +668,7 @@ SWB_HD void engine_warp_s16(const EngineParams& P, const WarpCtx& w, int lw, War
 //  above, which is exactly the recurrence of that column.
 //  DIRS (with ANCH, round 2): also record, for every cell, where its H, E and F came from (4 bits per cell, one 32-bit
 //  word per lane and step for R = 8) -- the traceback matrix of the GLOBAL alignment between the start and the end
-//  cell that swb200_score_span found; walk_traceback_kernel (swb200.cu) follows it back.  Uses the plain row loop
+//  cell that swb200_score_span found; walk_block (swb_traceback.cuh) follows it back.  Uses the plain row loop
 //  (E and F exactly as in main.cpp:57-58, no short-chain rewriting), so the flags mean what they say.
 template <int R, int SLACK, bool GEN = false, bool SHORT = true, bool TRACK = false, bool ANCH = false, bool DIRS = false>
 SWB_HD void engine_warp_s32(const EngineParams& P, const WarpCtx& w, int lw, WarpSmem* sm) {
@@ -710,8 +710,11 @@ SWB_HD void engine_warp_s32(const EngineParams& P, const WarpCtx& w, int lw, War
     const unsigned long long* sink_progress = P.progress + lw + 1;
     // Inner rings are indexed by the CUMULATIVE producer step over all rounds (sbase + step), so a
     // ring is one continuous stream and back-pressure spans band boundaries; the full-length ext
-    // stream restarts at 0 every band (safe: see DESIGN.md, hand-off protocol).
-    const long long sbase = (band / P.ring_total) * (long long)nsteps;
+    // stream restarts at 0 every band (safe: see DESIGN.md, hand-off protocol).  Rounds count from
+    // ring_offset: a blocked traceback launch (swb200_align) runs the band window [ring_offset, NB) on
+    // one GPU, and a producer and its consumer must agree on the round whatever the window's first band.
+    // (Every other launch has ring_offset + lw < ring_total, where this is band / ring_total.)
+    const long long sbase = ((band - P.ring_offset) / P.ring_total) * (long long)nsteps;
     const long long in_base = first_local ? 0 : sbase, out_base = last_local ? 0 : sbase;
 
     uint32_t sel[R];
@@ -884,7 +887,7 @@ SWB_HD void engine_warp_s32(const EngineParams& P, const WarpCtx& w, int lw, War
             if (TRACK) { const int key = (ANCH ? (h > 0 ? h : 0) : h) * 2048 + (cstep - r); bestkey = bestkey > key ? bestkey : key; }
             else if (r & 1) best1 = best1 > h ? best1 : h; else best0 = best0 > h ? best0 : h;
           }
-          if (DIRS) P.dirs[((size_t)band * (size_t)nsteps + (size_t)(i0 + k)) * 32 + lane] = dword;
+          if (DIRS) P.dirs[((size_t)(band - P.ring_offset) * (size_t)nsteps + (size_t)(i0 + k)) * 32 + lane] = dword;   // window-relative band
         }
         if (TRACK) cstep -= 16;
         xsH = Ho[R - 1];

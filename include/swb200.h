@@ -77,7 +77,10 @@ SWB200_API int swb200_device_count(void);
  *   "batch_chunk_bytes" (SWB200_BATCH_CHUNK_BYTES)  chunk size of the host batch calls' copy/compute pipeline (0 = default)
  *   "ring_min_cells" (SWB200_RING_MIN_CELLS)  host-buffer pairs with at least this many cells use all devices chosen
  *                                     with swb200_set_devices (default 2e11)
- *   "chain" (SWB200_CHAIN)            "0": the planner never picks the CTA-chained engine (launch config 7) by itself */
+ *   "chain" (SWB200_CHAIN)            "0": the planner never picks the CTA-chained engine (launch config 7) by itself
+ *   "align_block_rows" (SWB200_ALIGN_BLOCK_ROWS)  swb200_align's traceback in blocks of this many span rows, a positive
+ *                                     multiple of 256 (SWB200_ERR_ARG otherwise), even when the whole rectangle fits;
+ *                                     "0" (default): blocks only when the rectangle's directions do not fit in device memory */
 SWB200_API int swb200_configure(const char* key, const char* value);
 
 /* Diagnostic (needs no GPU): the kernel variant the planner picks for an n x m pair on `sms` SMs in all (148 per B200):
@@ -148,9 +151,14 @@ SWB200_API int swb200_score_span_device(swb200_ctx* ctx, const unsigned char* d_
  * alignments is reported: at every cell diagonal before gap in seq2 (E) before gap in seq1 (F); a gap counts as
  * extended only where extending is strictly better than opening.
  * Three passes: end cell, start cell, then the anchored recurrence over the span rectangle with 4 bits of traceback
- * direction per cell kept in HBM (0.5 byte per cell: the 100 000 x 100 000 pair takes 5 GB; SWB200_ERR_NOMEM when the
- * rectangle does not fit) and a walk back through them.  cigar_out may be NULL to ask for the length only
- * (*cigar_len_out, without the terminating NUL).  Same limits as swb200_score_end. */
+ * direction per cell kept in HBM (0.5 byte per cell: the 100 000 x 100 000 pair takes 5 GB) and a walk back through them.
+ * When the whole rectangle's directions do not fit in free device memory, the third pass runs in blocks of rows: a
+ * forward sweep keeps only the boundary row between blocks (16 bytes per span column each), then the walk goes back
+ * block by block, recomputing each block from the row above it over the columns left of the walk.  Score, span and
+ * CIGAR are byte for byte those of the one-block traceback; the cost is about one more sweep over the span.
+ * SWB200_ERR_NOMEM only when not even a block of 256 rows plus the boundary rows fits.  "align_block_rows"
+ * (swb200_configure) forces the blocked path.  cigar_out may be NULL to ask for the length only (*cigar_len_out,
+ * without the terminating NUL).  Same limits as swb200_score_end. */
 SWB200_API int swb200_align(const unsigned char* seq1, long long n, const unsigned char* seq2, long long m,
                             const swb200_params* p, int* score_out, long long span_out[4], char* cigar_out,
                             long long cigar_cap, long long* cigar_len_out);
