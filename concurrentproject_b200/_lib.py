@@ -83,6 +83,9 @@ EXPORTS = {
     "swb200_batch_pack_device": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                   C.c_longlong, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p, C.POINTER(C.c_void_p)], C.c_int),
     "swb200_batch_score": ([C.c_void_p, C.POINTER(Params), C.POINTER(Options), C.c_void_p, C.c_void_p], C.c_int),
+    "swb200_score_long_batch": ([U8P, C.POINTER(C.c_longlong), C.POINTER(C.c_int), U8P, C.POINTER(C.c_longlong),
+                                 C.POINTER(C.c_int), C.c_longlong, C.POINTER(Params), C.POINTER(Options), C.POINTER(C.c_int)], C.c_int),
+    "swb200_batch_score_long": ([C.c_void_p, C.POINTER(Params), C.POINTER(Options), C.c_void_p, C.c_void_p], C.c_int),
     "swb200_batch_free": ([C.c_void_p], None),
     "swb200_align_batch": ([U8P, C.POINTER(C.c_longlong), C.POINTER(C.c_int), U8P, C.POINTER(C.c_longlong), C.POINTER(C.c_int),
                             C.c_longlong, C.POINTER(Params), C.POINTER(Options), C.POINTER(C.c_int), C.POINTER(C.c_int),

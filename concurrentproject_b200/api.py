@@ -238,6 +238,30 @@ def score_batch_flat(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray, flat
     return out
 
 
+def score_long_batch(seqs1, seqs2, params: Sequence[int] = DEFAULT_PARAMS, *, rows: int = 0, no_linear: bool = False) -> np.ndarray:
+    """Scores of many HOST pairs of any size (swb200_score_long_batch): one warp per pair, the shorter side swept in
+    bands of 64*rows rows, so pairs whose shorter side is over 1024 stay in one batch kernel."""
+    if len(seqs1) != len(seqs2):
+        raise ValueError("seqs1 and seqs2 differ in length")
+    return score_long_batch_flat(*_flatten(seqs1), *_flatten(seqs2), params, rows=rows, no_linear=no_linear)
+
+
+def score_long_batch_flat(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray, flat2: np.ndarray, off2: np.ndarray,
+                          len2: np.ndarray, params: Sequence[int] = DEFAULT_PARAMS, *, rows: int = 0,
+                          no_linear: bool = False) -> np.ndarray:
+    """swb200_score_long_batch on already flattened HOST arrays (uint8 bytes, int64 offsets, int32 lengths)."""
+    n = len(len1)
+    out = np.zeros(n, dtype=np.int32)
+    p, o = _params(params), _options(rows=rows, no_linear=no_linear)
+    LL, I = C.POINTER(C.c_longlong), C.POINTER(C.c_int)
+    rc = _lib.load().swb200_score_long_batch(_ptr(flat1), off1.ctypes.data_as(LL), len1.ctypes.data_as(I), _ptr(flat2),
+                                             off2.ctypes.data_as(LL), len2.ctypes.data_as(I), n, C.byref(p), C.byref(o),
+                                             out.ctypes.data_as(I))
+    if rc != 0:
+        raise SwbError(rc, "swb200_score_long_batch")
+    return out
+
+
 def score_banded_batch(seqs1, seqs2, band_lo: int = -32, band_hi: int = 31, params: Sequence[int] = DEFAULT_PARAMS, *,
                        no_linear: bool = False, config: int = 0) -> np.ndarray:
     """Banded scores of many HOST pairs: cell (i, j) counts iff band_lo <= j - i <= band_hi (64 diagonals)."""
@@ -281,6 +305,14 @@ class PackedBatch:
         rc = _lib.load().swb200_batch_score(self.handle, C.byref(p), C.byref(o), C.c_void_p(stream), C.c_void_p(d_scores))
         if rc != 0:
             raise SwbError(rc, "swb200_batch_score")
+
+    def score_long(self, d_scores: int, params: Sequence[int] = DEFAULT_PARAMS, *, stream: int = 0, rows: int = 0,
+                   no_linear: bool = False) -> None:
+        """Scores with the multi-band kernel (swb200_batch_score_long): any shorter side; keep_order=False batches."""
+        p, o = _params(params), _options(rows=rows, no_linear=no_linear)
+        rc = _lib.load().swb200_batch_score_long(self.handle, C.byref(p), C.byref(o), C.c_void_p(stream), C.c_void_p(d_scores))
+        if rc != 0:
+            raise SwbError(rc, "swb200_batch_score_long")
 
     def score_banded(self, d_scores: int, band_lo: int, band_hi: int, params: Sequence[int] = DEFAULT_PARAMS, *, stream: int = 0,
                      no_linear: bool = False, config: int = 0) -> None:

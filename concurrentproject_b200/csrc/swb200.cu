@@ -287,6 +287,9 @@ struct swb200_ctx {
   int* hb_spans = nullptr; size_t hb_spans_cap = 0;       // host batch alignment: outputs before the copy back
   uint32_t* hb_ops = nullptr; size_t hb_ops_cap = 0;
   int* hb_opsn = nullptr; size_t hb_opsn_cap = 0;
+  // multi-band batch scoring (swb200_score_long_batch / swb200_batch_score_long), grow-only
+  uint32_t* lb_bnd = nullptr; size_t lb_bnd_cap = 0;                  // one boundary row per launched warp
+  unsigned long long* lb_next = nullptr; size_t lb_next_cap = 0;      // the launch's pair counter
 };
 
 namespace swb {
@@ -1048,6 +1051,7 @@ void swb200_ctx_destroy(swb200_ctx* c) {
   cudaFree(c->hb_seq1); cudaFree(c->hb_seq2); cudaFree(c->hb_off1); cudaFree(c->hb_off2); cudaFree(c->hb_len1); cudaFree(c->hb_len2);
   cudaFree(c->hb_scores); cudaFree(c->hb_qw); cudaFree(c->hb_tw); cudaFree(c->hb_ql); cudaFree(c->hb_tl);
   cudaFree(c->ab_col); cudaFree(c->ab_slot); cudaFree(c->ab_pool); cudaFree(c->ab_list); cudaFree(c->ab_misc);
+  cudaFree(c->lb_bnd); cudaFree(c->lb_next);
   cudaFree(c->hb_spans); cudaFree(c->hb_ops); cudaFree(c->hb_opsn);
   if (c->h_result) cudaFreeHost(c->h_result);
   if (c->ev0) cudaEventDestroy(c->ev0);
@@ -1481,6 +1485,67 @@ static int launch_batch_score(swb200_ctx* c, const BatchView& v, const swb200_pa
   return SWB200_OK;
 }
 
+// The multi-band batch kernel (swb_batch.cuh, LONG): one pair per warp, Q cut into bands of 64*R rows, so the shorter
+// side has no cap beyond the 16-bit range.
+static int check_long_score(const swb200_params& p, const swb200_options& o, int keep_order, int max_short) {
+  if (keep_order) return fail(SWB200_ERR_ARG, "batch was packed in caller order (banded); re-pack with keep_order=0");
+  bool known = o.rows == 0;
+  for (int k = 0; k < swb::kNumBatchRowChoices; ++k) known |= o.rows == swb::kBatchRowChoices[k];
+  if (!known) return fail(SWB200_ERR_ARG, "rows must be 0 or one of 2,4,6,8,10,12,16");
+  if ((long long)p.match * max_short > 32767 - p.match - 1)
+    return fail(SWB200_ERR_RANGE, "match * min(len) does not fit the 16-bit lanes of the batch kernel");
+  return SWB200_OK;
+}
+
+// R of the multi-band kernel: options.rows, else the smallest choice whose band of 64*R rows holds the tallest pair, else 16
+static int long_rows(const swb200_options& o, int max_short) {
+  if (o.rows) return o.rows;
+  for (int k = 0; k < swb::kNumBatchRowChoices; ++k)
+    if (64 * swb::kBatchRowChoices[k] >= max_short) return swb::kBatchRowChoices[k];
+  return 16;
+}
+
+// warps of the multi-band kernel resident at once (one pair each): a host chunk is a whole number of them
+static long long long_wave_pairs(swb200_ctx* c, const swb200_params& p, const swb200_options& o, int max_short) {
+  const int mode = (p.gap_init == p.gap_ext && !o.no_linear) ? 1 : 0;
+  int per_sm = 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, swb::long_batch_kernel(long_rows(o, max_short), mode), 256, 0) !=
+          cudaSuccess || per_sm < 1) per_sm = 1;
+  return 8LL * c->sms * per_sm;
+}
+
+static int launch_long_score(swb200_ctx* c, const BatchView& v, const swb200_params& p, const swb200_options& o,
+                             cudaStream_t s, int* d_scores, swb200_run_info* info) {
+  if (v.npairs == 0) return SWB200_OK;
+  const int R = long_rows(o, v.max_short);
+  const int mode = (p.gap_init == p.gap_ext && !o.no_linear) ? 1 : 0;
+  const void* kern = swb::long_batch_kernel(R, mode);
+  if (!kern) return fail(SWB200_ERR_ARG, "no batch kernel for rows=" + std::to_string(R));
+  swb::BatchParams P{};
+  P.q_words = v.q_words; P.t_words = v.t_words; P.q_len = v.q_len; P.t_len = v.t_len;
+  P.q_stride = v.q_stride; P.t_stride = v.t_stride; P.npairs = v.npairs; P.scores = d_scores;
+  P.match = p.match; P.mismatch = p.mismatch; P.gap_init = p.gap_init; P.gap_ext = p.gap_ext;
+  int per_sm = 0;
+  SWB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, 0));
+  per_sm = std::max(per_sm, 1);
+  const long long ctas = std::max<long long>(1, std::min<long long>((v.npairs + 7) / 8, (long long)c->sms * per_sm));
+  // one boundary row of the longest T per launched warp, 128-byte lines
+  long long stride = ((long long)std::max(v.max_long, 1) + 31) / 32 * 32;
+  int rc;
+  if ((rc = grow(c->lb_bnd, c->lb_bnd_cap, (size_t)(ctas * 8) * (size_t)stride, false, s)) ||
+      (rc = grow(c->lb_next, c->lb_next_cap, 1, false, s))) return rc;
+  SWB_CUDA(cudaMemsetAsync(c->lb_next, 0, sizeof(unsigned long long), s));
+  uint32_t* bnd = c->lb_bnd;
+  unsigned long long* next = c->lb_next;
+  void* args[] = {&P, &bnd, &stride, &next};
+  SWB_CUDA(cudaLaunchKernel(kern, dim3((unsigned)ctas), dim3(256), args, 0, s));
+  const int band_rows = 64 * R;
+  info->lanes = 16; info->linear = mode == 1; info->rows = R; info->config = 332; info->ctas = (int)ctas;
+  info->warps = (int)ctas * 8; info->bands = std::max(1, (v.max_short + band_rows - 1) / band_rows);
+  info->engine_launches += 1;
+  return SWB200_OK;
+}
+
 static int check_banded_score(const swb200_params& p, int keep_order, int band_lo, int band_hi, int max1, int max2) {
   if (!keep_order) return fail(SWB200_ERR_ARG, "banded scoring needs a batch packed with keep_order=1");
   if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
@@ -1573,6 +1638,17 @@ int swb200_batch_score(swb200_batch* b, const swb200_params* pp, const swb200_op
   });
 }
 
+int swb200_batch_score_long(swb200_batch* b, const swb200_params* pp, const swb200_options* oo, void* stream, int* d_scores) {
+  if (!b || !d_scores) return fail(SWB200_ERR_ARG, "bad batch arguments");
+  const swb200_params p = params_or_default(pp);
+  const swb200_options o = options_or_default(oo);
+  int rc;
+  if ((rc = check_params(p)) || (rc = check_long_score(p, o, b->keep_order, b->max_short))) return rc;
+  return run_device_batch(b, b->cells, stream, [&](swb200_ctx* c, cudaStream_t s) {
+    return launch_long_score(c, whole_batch(b), p, o, s, d_scores, &c->info);
+  });
+}
+
 int swb200_batch_score_banded(swb200_batch* b, int band_lo, int band_hi, const swb200_params* pp, const swb200_options* oo,
                               void* stream, int* d_scores) {
   if (!b || !d_scores) return fail(SWB200_ERR_ARG, "bad batch arguments");
@@ -1634,11 +1710,19 @@ static PairScan scan_pairs(const HostPairs& h, long long k0, long long k1) {
   return PairScan{neg, mx1, mx2, mxmin, cells, lo1, hi1, lo2, hi2};
 }
 
-static int check_score_pairs(const PairScan& s, const swb200_params& p, int banded, int band_lo, int band_hi) {
+// which kernel a host ASCII score batch runs
+enum class ScoreKind { batch, banded, long_pairs };
+
+static int check_score_pairs(const PairScan& s, const swb200_params& p, const swb200_options& o, ScoreKind kind, int band_lo,
+                             int band_hi) {
   if (s.neg < 0) return fail(SWB200_ERR_ARG, "negative length or offset");
   int rc;
   if ((rc = check_params(p))) return rc;
-  return banded ? check_banded_score(p, 1, band_lo, band_hi, s.max1, s.max2) : check_batch_score(p, 0, s.max_min);
+  switch (kind) {
+    case ScoreKind::banded: return check_banded_score(p, 1, band_lo, band_hi, s.max1, s.max2);
+    case ScoreKind::long_pairs: return check_long_score(p, o, 0, s.max_min);
+    default: return check_batch_score(p, 0, s.max_min);
+  }
 }
 
 // chunk_events of the host pipelines, grow-only: one per chunk of a call
@@ -1656,10 +1740,11 @@ static int chunk_events_at_least(swb200_ctx* c, size_t n) {
 // copies chunk k+1 from the host while aux_stream packs chunk k and runs each_chunk (if any) on it.  The staging pool is
 // sized for the whole range, so chunks need no double buffering: every byte keeps its position relative to the range's
 // lowest offset.  With pinned host buffers the call runs at PCIe speed.  ev0 is recorded at the first pack; *staged is
-// the packed range.
+// the packed range.  wave > 0: every chunk but the last holds a whole multiple of wave pairs.
 static int stage_and_pack_locked(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part,
                                  const PairScan& whole, bool keep_order, BatchView* staged,
-                                 const std::function<int(const BatchView& chunk, long long k0)>& each_chunk) {
+                                 const std::function<int(const BatchView& chunk, long long k0)>& each_chunk,
+                                 long long wave = 0) {
   cudaStream_t sc = c->own_stream, sk = c->aux_stream;
   const size_t np = (size_t)npairs;
   const long long base1 = part.lo1 & ~15LL, base2 = part.lo2 & ~15LL;
@@ -1709,7 +1794,8 @@ static int stage_and_pack_locked(swb200_ctx* c, const HostPairs& h, long long np
     lo1 = std::min(lo1, h.off1[k]); hi1 = std::max(hi1, h.off1[k] + h.len1[k]);
     lo2 = std::min(lo2, h.off2[k]); hi2 = std::max(hi2, h.off2[k] + h.len2[k]);
     acc += (long long)h.len1[k] + h.len2[k];
-    if (!((acc >= target && k + 1 - k0 >= min_pairs) || k + 1 == npairs)) continue;
+    const bool whole_waves = forced > 0 || wave <= 0 || (k + 1 - k0) % wave == 0;
+    if (!((acc >= target && k + 1 - k0 >= min_pairs && whole_waves) || k + 1 == npairs)) continue;
     if ((rc = issue(k + 1))) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sk); return rc; }
     k0 = k + 1; acc = 0; lo1 = LLONG_MAX; hi1 = 0; lo2 = LLONG_MAX; hi2 = 0;
   }
@@ -1719,7 +1805,7 @@ static int stage_and_pack_locked(swb200_ctx* c, const HostPairs& h, long long np
 // One context's share of a host ASCII score batch (arguments checked by the caller): every chunk is scored as soon as it
 // is packed, while the next one is copied.
 static int score_ascii_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part, const PairScan& whole,
-                           const swb200_params& p, const swb200_options& o, int banded, int band_lo, int* scores_out) {
+                           const swb200_params& p, const swb200_options& o, ScoreKind kind, int band_lo, int* scores_out) {
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
   SWB_CUDA(cudaSetDevice(c->device));
@@ -1727,10 +1813,16 @@ static int score_ascii_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, 
   c->info = swb200_run_info{};
   c->info.cells = part.cells;
   BatchView staged;
-  int rc = stage_and_pack_locked(c, h, npairs, part, whole, banded != 0, &staged, [&](const BatchView& v, long long k0) {
-    return banded ? launch_banded_score(c, v, band_lo, p, o, sk, c->hb_scores + k0, &c->info)
-                  : launch_batch_score(c, v, p, o, sk, c->hb_scores + k0, &c->info);
-  });
+  // a multi-band launch runs as long as its longest pairs however few they are: its chunks are whole waves of warps
+  const bool banded = kind == ScoreKind::banded;
+  const long long wave = kind == ScoreKind::long_pairs ? long_wave_pairs(c, p, o, whole.max_min) : 0;
+  int rc = stage_and_pack_locked(c, h, npairs, part, whole, banded, &staged, [&](const BatchView& v, long long k0) {
+    switch (kind) {
+      case ScoreKind::banded: return launch_banded_score(c, v, band_lo, p, o, sk, c->hb_scores + k0, &c->info);
+      case ScoreKind::long_pairs: return launch_long_score(c, v, p, o, sk, c->hb_scores + k0, &c->info);
+      default: return launch_batch_score(c, v, p, o, sk, c->hb_scores + k0, &c->info);
+    }
+  }, wave);
   if (rc) return rc;
   SWB_CUDA(cudaEventRecord(c->ev1, sk));
   SWB_CUDA(cudaMemcpyAsync(scores_out, c->hb_scores, npairs * sizeof(int), cudaMemcpyDeviceToHost, sk));
@@ -1756,8 +1848,8 @@ int swb200_score_banded(const unsigned char* seq1, int n, const unsigned char* s
   const swb200_params pv = params_or_default(p);
   swb200_ctx* c = nullptr;
   int rc;
-  if ((rc = check_score_pairs(s, pv, 1, band_lo, band_hi)) || (rc = default_ctx(&c))) return rc;
-  return score_ascii_ctx(c, in, 1, s, s, pv, swb200_options{}, 1, band_lo, score_out);
+  if ((rc = check_score_pairs(s, pv, swb200_options{}, ScoreKind::banded, band_lo, band_hi)) || (rc = default_ctx(&c))) return rc;
+  return score_ascii_ctx(c, in, 1, s, s, pv, swb200_options{}, ScoreKind::banded, band_lo, score_out);
 }
 
 // ---- one pair over a ring of GPUs (one swb200_ring per GPU / per process) -------------------------
@@ -2116,9 +2208,9 @@ static int score_pair_on_pool(const unsigned char* seq1, long long n, const unsi
   return handled ? SWB200_OK : 1;
 }
 
-// swb200_score_batch / swb200_score_banded_batch
+// swb200_score_batch / swb200_score_banded_batch / swb200_score_long_batch
 static int score_batch_host(const HostPairs& in, long long npairs, const swb200_params* pp, const swb200_options* oo,
-                            int banded, int band_lo, int band_hi, int* scores_out) {
+                            ScoreKind kind, int band_lo, int band_hi, int* scores_out) {
   if (npairs < 0 || (npairs > 0 && (!in.seq1 || !in.seq2 || !in.off1 || !in.off2 || !in.len1 || !in.len2 || !scores_out)))
     return fail(SWB200_ERR_ARG, "bad batch arguments");
   if (npairs == 0) return SWB200_OK;
@@ -2126,9 +2218,9 @@ static int score_batch_host(const HostPairs& in, long long npairs, const swb200_
   const swb200_options o = options_or_default(oo);
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); },
-      [&](const PairScan& whole) { return check_score_pairs(whole, p, banded, band_lo, band_hi); },
+      [&](const PairScan& whole) { return check_score_pairs(whole, p, o, kind, band_lo, band_hi); },
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return score_ascii_ctx(c, in.from(k0), k1 - k0, part, whole, p, o, banded, band_lo, scores_out + k0);
+        return score_ascii_ctx(c, in.from(k0), k1 - k0, part, whole, p, o, kind, band_lo, scores_out + k0);
       });
 }
 
@@ -2242,7 +2334,15 @@ extern "C" {
 int swb200_score_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
                        const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
                        const swb200_params* p, const swb200_options* opt, int* scores_out) {
-  return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, 0, 0, 0, scores_out);
+  return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, ScoreKind::batch, 0, 0,
+                          scores_out);
+}
+
+int swb200_score_long_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                            const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                            const swb200_params* p, const swb200_options* opt, int* scores_out) {
+  return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, ScoreKind::long_pairs, 0, 0,
+                          scores_out);
 }
 
 int swb200_score_banded_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
@@ -2250,7 +2350,8 @@ int swb200_score_banded_batch(const unsigned char* seq1_all, const long long* of
                               int band_lo, int band_hi, const swb200_params* p, const swb200_options* opt,
                               int* scores_out) {
   if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
-  return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, 1, band_lo, band_hi, scores_out);
+  return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, ScoreKind::banded, band_lo,
+                          band_hi, scores_out);
 }
 
 int swb200_batch_strides(int max_short, int max_long, long long* q_stride, long long* t_stride) {
@@ -2632,7 +2733,7 @@ int swb200_align_banded_batch(const unsigned char* seq1_all, const long long* of
     return fail(SWB200_ERR_ARG, "bad batch arguments");
   const swb200_params p = params_or_default(pp);
   const HostPairs in{seq1_all, off1, len1, seq2_all, off2, len2};
-  auto check = [&](const PairScan& whole) { return check_score_pairs(whole, p, 1, band_lo, band_hi); };
+  auto check = [&](const PairScan& whole) { return check_score_pairs(whole, p, swb200_options{}, ScoreKind::banded, band_lo, band_hi); };
   if (npairs == 0) return check(PairScan{});
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,

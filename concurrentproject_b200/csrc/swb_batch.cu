@@ -23,6 +23,22 @@ const void* batch_kernel(int R, int mode, int G) {
   return G == 8 ? batch_lookup<1, 8>(R) : (G == 16 ? batch_lookup<1, 16>(R) : batch_lookup<1, 32>(R));
 }
 
+template <int MODE>
+static const void* long_lookup(int R) {
+  switch (R) {
+    case 2: return (const void*)sw_long_batch_kernel<2, MODE>;
+    case 4: return (const void*)sw_long_batch_kernel<4, MODE>;
+    case 6: return (const void*)sw_long_batch_kernel<6, MODE>;
+    case 8: return (const void*)sw_long_batch_kernel<8, MODE>;
+    case 10: return (const void*)sw_long_batch_kernel<10, MODE>;
+    case 12: return (const void*)sw_long_batch_kernel<12, MODE>;
+    case 16: return (const void*)sw_long_batch_kernel<16, MODE>;
+    default: return nullptr;
+  }
+}
+
+const void* long_batch_kernel(int R, int mode) { return mode == 0 ? long_lookup<0>(R) : long_lookup<1>(R); }
+
 const void* banded_kernel(int mode) {
   return mode == 0 ? (const void*)sw_banded_kernel<0> : (const void*)sw_banded_kernel<1>;
 }

@@ -161,6 +161,14 @@ SWB_HD void atomic_or_i32(int* p, int v) {
 #endif
 }
 
+SWB_HD unsigned long long atomic_fetch_add_u64(unsigned long long* p, unsigned long long v) {
+#if SWB_DEVICE_CODE
+  return atomicAdd(p, v);
+#else
+  return reinterpret_cast<std::atomic<unsigned long long>*>(p)->fetch_add(v);
+#endif
+}
+
 SWB_HD void spin_pause() {
 #if SWB_DEVICE_CODE
   __nanosleep(20);

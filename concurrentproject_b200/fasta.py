@@ -9,9 +9,11 @@ to the GPU kernels:
                          lanes per pair, swb_batch.cuh) and orders each bucket by the longer length, so the
                          pairs a warp scores side by side stream about the same number of columns;
 * ``score_pairs``     -- scores pair k = (seqs1[k], seqs2[k]) for ragged inputs: ACGT pairs whose shorter side
-                         is <= 1024 go bucket by bucket through the batch kernel (swb200_score_batch), everything
-                         else (longer, or other alphabets such as N or amino acids) through the single-pair engine
-                         (swb200_score_ex), which compares bytes exactly like main.cpp:60;
+                         is <= 1024 go bucket by bucket through the batch kernel (swb200_score_batch), longer ACGT
+                         pairs, when the batch beats one call per pair (long_batch_pays), through the multi-band
+                         batch kernel (swb200_batch_score_long), everything else (a few long pairs, or other
+                         alphabets such as N or amino acids) through the single-pair engine (swb200_score_ex), which compares bytes
+                         exactly like main.cpp:60;
 * ``search``          -- one query against every record of a database.
 
 The residues are uploaded to HBM once per call (torch is the plumbing for device memory); a bucket only ships its
@@ -28,6 +30,13 @@ from . import api
 # capacities of the batch kernel: rows-per-sub-lane choices {2,4,6,8,10,12,16} x 16 / 32 / 64 sub-lanes per pair
 BUCKET_EDGES = (32, 64, 96, 128, 160, 192, 256, 320, 384, 512, 640, 768, 1024)
 BATCH_MAX_SHORT = 1024
+# Cost model of the two routes for pairs whose shorter side is over BATCH_MAX_SHORT, fitted to the crossover of
+# bench/long_batch.py (profiles/r06_long_batch.json; one NVIDIA B200, power limit 1000 W).  One single-pair call costs
+# LOOP_CALL_S + LOOP_CELL_S per cell (2, 5, 20 kb: 0.13, 0.21, 0.68 ms).  The multi-band call costs LONG_CALL_S plus
+# the longer of its tallest pair on one warp (padded cells at LONG_WARP_CUPS) and all padded cells at LONG_GPU_CUPS.
+# So a few long pairs stay on the single-pair engine (20 kb: 64 pairs take 0.04 s there, 0.07 s in the batch).
+LOOP_CALL_S, LOOP_CELL_S = 1.8e-4, 1.25e-12
+LONG_CALL_S, LONG_WARP_CUPS, LONG_GPU_CUPS = 3e-4, 5.9e9, 8.3e12
 _IS_ACGT = np.zeros(256, dtype=bool)
 _IS_ACGT[[ord(c) for c in "ACGT"]] = True
 
@@ -98,22 +107,42 @@ def write_fasta(path: str, names: Sequence[str], seqs: Sequence[bytes], width: i
 
 @dataclass
 class Bucket:
-    kind: str            # "batch": one swb200_score_batch call; "single": one swb200_score_ex call per pair
+    kind: str            # "batch": one swb200_score_batch call; "long": one swb200_batch_score_long call;
+                         # "single": one swb200_score_ex call per pair
     cap: int             # capacity class of the shorter side (0 for "single")
     index: np.ndarray    # pair ids, in the order they are handed to the kernel
+
+
+def long_batch_pays(short: np.ndarray, long_: np.ndarray) -> bool:
+    """True when one multi-band batch call over these pairs is expected to beat one single-pair call each."""
+    short = np.asarray(short, dtype=np.int64)
+    long_ = np.asarray(long_, dtype=np.int64)
+    if short.size == 0:
+        return False
+    band = 64 * 16                                                  # the band height the tallest pairs get
+    padded = (-(-short // band) * band * (long_ + 63)).astype(np.float64)
+    loop = short.size * LOOP_CALL_S + float((short * long_).sum()) * LOOP_CELL_S
+    batch = LONG_CALL_S + max(float(padded.max()) / LONG_WARP_CUPS, float(padded.sum()) / LONG_GPU_CUPS)
+    return batch < loop
 
 
 def plan_buckets(len1: np.ndarray, len2: np.ndarray, acgt_only: np.ndarray, min_bucket: int = 512, match: int = 1) -> List[Bucket]:
     """Partition pair ids.  Batch buckets are keyed by the capacity class of min(len1, len2); a class with fewer
     than ``min_bucket`` pairs is merged into the next larger one (a launch costs more than the padding).  Inside a
-    bucket pairs are ordered by max(len1, len2), longest first.  Pairs the 16-bit batch kernel cannot hold
-    (match * min(len) > 32766 - match, swb200.cu: check_batch_score) go to the single-pair engine, which re-runs in
-    re-based or 32-bit lanes by itself."""
+    bucket pairs are ordered by max(len1, len2), longest first.  ACGT pairs with a shorter side over BATCH_MAX_SHORT
+    form one "long" bucket, ordered by padded cells, largest first (the multi-band kernel's warps take pairs in this
+    order, so the longest pairs start first), when that call beats the single-pair engine (long_batch_pays).  Pairs the 16-bit batch
+    kernels cannot hold (match * min(len) > 32766 - match, swb200.cu: check_batch_score) go to the single-pair engine,
+    which re-runs in re-based or 32-bit lanes by itself."""
     len1 = np.asarray(len1, dtype=np.int64)
     len2 = np.asarray(len2, dtype=np.int64)
     short = np.minimum(len1, len2)
     long_ = np.maximum(len1, len2)
-    batchable = np.asarray(acgt_only, dtype=bool) & (short <= BATCH_MAX_SHORT) & (int(match) * short <= 32766 - int(match))
+    in_range = np.asarray(acgt_only, dtype=bool) & (int(match) * short <= 32766 - int(match))
+    batchable = in_range & (short <= BATCH_MAX_SHORT)
+    long_ids = np.flatnonzero(in_range & (short > BATCH_MAX_SHORT))
+    if not long_batch_pays(short[long_ids], long_[long_ids]):
+        long_ids = long_ids[:0]
     out: List[Bucket] = []
     edges = np.array(BUCKET_EDGES)
     cls = np.searchsorted(edges, short, side="left")          # first edge >= short
@@ -131,7 +160,13 @@ def plan_buckets(len1: np.ndarray, len2: np.ndarray, acgt_only: np.ndarray, min_
     if carry.size:
         order = np.argsort(-long_[carry], kind="stable")
         out.append(Bucket("batch", BUCKET_EDGES[-1], carry[order]))
-    rest = np.flatnonzero(~batchable)
+    if long_ids.size:
+        band = 64 * 16                                             # the default band height of the tallest pairs
+        padded = (-(-short[long_ids] // band) * band) * (long_[long_ids] + 63)
+        out.append(Bucket("long", 0, long_ids[np.argsort(-padded, kind="stable")]))
+    routed = batchable.copy()
+    routed[long_ids] = True
+    rest = np.flatnonzero(~routed)
     if rest.size:
         out.append(Bucket("single", 0, rest))
     return out
@@ -197,7 +232,7 @@ def score_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
         stream = torch.cuda.current_stream(dev).cuda_stream
         for bk in buckets:
             ids = bk.index
-            if bk.kind == "batch":
+            if bk.kind in ("batch", "long"):
                 bl1, bl2 = l1[ids], l2[ids]
                 d_o1 = torch.from_numpy(o1[ids]).to(dev); d_o2 = torch.from_numpy(o2[ids]).to(dev)
                 d_l1 = torch.from_numpy(bl1).to(dev); d_l2 = torch.from_numpy(bl2).to(dev)
@@ -207,7 +242,10 @@ def score_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
                 pb = api.PackedBatch(ctx, fa.data_ptr(), d_o1.data_ptr(), d_l1.data_ptr(), fb.data_ptr(), d_o2.data_ptr(),
                                      d_l2.data_ptr(), len(ids), int(short.max()), int(long_.max()), cells, stream=stream)
                 try:
-                    pb.score(d_sc.data_ptr(), params, stream=stream)
+                    if bk.kind == "long":
+                        pb.score_long(d_sc.data_ptr(), params, stream=stream)
+                    else:
+                        pb.score(d_sc.data_ptr(), params, stream=stream)
                 finally:
                     pb.close()
                 scores[ids] = d_sc.cpu().numpy()

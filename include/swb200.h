@@ -238,6 +238,26 @@ SWB200_API int swb200_batch_pack_device(swb200_ctx* ctx, const unsigned char* d_
                                         swb200_batch** batch_out);
 SWB200_API int swb200_batch_score(swb200_batch* batch, const swb200_params* p, const swb200_options* opt,
                                   void* stream, int* d_scores);
+
+/* Batches whose shorter side is over 1024 (gene / contig pairs, long reads without a band, database search with long
+ * queries): the same scores as swb200_score_ex gives each pair, from one multi-band kernel.  One warp per pair; the shorter
+ * sequence is cut into bands of 64*R rows swept one after the other over the whole longer one, the bottom row of a band
+ * carried to the next through a per-warp row in device memory; warps take the next pair from a counter, so a ragged batch
+ * keeps every warp busy.  Argument form and limits are swb200_score_batch's without the 1024 cap: bytes A,C,G,T
+ * (SWB200_ERR_ALPHABET), match*min(len) <= 32766 - match (SWB200_ERR_RANGE); the longer side is limited by int and by
+ * the boundary rows, (max(len) rounded up to 32) * 4 bytes per resident warp (SWB200_ERR_NOMEM).  Both calls run this
+ * kernel for any shorter side, also one of 1024 or less.  opt->rows picks R (2,4,6,8,10,12,16; 0: the smallest R with
+ * 64*R >= the longest shorter side, else 16; other values SWB200_ERR_ARG); opt->no_linear as in swb200_score_batch; other
+ * option fields are ignored.  All checks run before a device is touched.  swb200_last_run reports config 332, rows R and
+ * bands = the band count of the tallest pair.  The host call packs and scores in chunks of whole waves of resident warps
+ * and shards over swb200_set_devices like swb200_score_batch; the device call takes a batch packed with keep_order = 0
+ * (SWB200_ERR_ARG for keep_order = 1). */
+SWB200_API int swb200_score_long_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                                       const unsigned char* seq2_all, const long long* off2, const int* len2,
+                                       long long npairs, const swb200_params* p, const swb200_options* opt,
+                                       int* scores_out);
+SWB200_API int swb200_batch_score_long(swb200_batch* batch, const swb200_params* p, const swb200_options* opt,
+                                       void* stream, int* d_scores);
 SWB200_API void swb200_batch_free(swb200_batch* batch);
 
 /* ---- batch alignment: score, span and CIGAR for every pair of a batch -------------------------------------------------
