@@ -344,6 +344,16 @@ class PackedBatch:
         if rc != 0:
             raise SwbError(rc, "swb200_batch_align_banded")
 
+    def align_long(self, d_scores: int, d_spans: int, d_ops: int, ops_stride: int, d_ops_count: int,
+                   params: Sequence[int] = DEFAULT_PARAMS, *, stream: int = 0) -> None:
+        """Score, span and alignment operations of every pair, any shorter side (swb200_batch_align_long; the batch must
+        be packed with keep_order=False).  Device outputs as align writes them."""
+        p = _params(params)
+        rc = _lib.load().swb200_batch_align_long(self.handle, C.byref(p), None, C.c_void_p(stream), C.c_void_p(d_scores),
+                                                 C.c_void_p(d_spans), C.c_void_p(d_ops), ops_stride, C.c_void_p(d_ops_count))
+        if rc != 0:
+            raise SwbError(rc, "swb200_batch_align_long")
+
     def close(self):
         if self.handle:
             _lib.load().swb200_batch_free(self.handle)
@@ -578,6 +588,53 @@ def align_banded_batch(seqs1, seqs2, band_lo: int = -32, band_hi: int = 31, para
         stride = int((l1[redo].astype(np.int64) + l2[redo]).max())
         _, _, ops2, cnt2 = align_banded_batch_ops(f1, o1[redo].copy(), l1[redo].copy(), f2, o2[redo].copy(), l2[redo].copy(),
                                                   band_lo, band_hi, params, stride)
+        for r, k in enumerate(redo.tolist()):
+            cigars[k] = cigar_string(ops2[r, :cnt2[r]])
+    return scores, spans, cigars
+
+
+# ---- long-pair batch alignment (swb200_align_long_batch) --------------------------------------------------------------
+LONG_OPS_STRIDE = 4096    # operations per pair in the first attempt.  On 20 000 seeded 5 kb pairs (half planted with 10 %
+                          # substitutions, half random; default scoring) the alignments need 1 963 operations at the median,
+                          # 3 735 at the 99th percentile and 3 816 at most (bench/align_long_batch.py, NVIDIA B200); 20 kb
+                          # planted pairs need 2 875 at the median.  The ops buffer costs 16 KB per pair.
+
+
+def align_long_batch_ops(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray, flat2: np.ndarray, off2: np.ndarray,
+                         len2: np.ndarray, params: Sequence[int] = DEFAULT_PARAMS, ops_stride: int = LONG_OPS_STRIDE):
+    """swb200_align_long_batch on flattened HOST arrays: (scores int32[n], spans int32[n, 4], ops uint32[n, ops_stride],
+    ops_count int32[n]) as align_batch_ops returns them; ops_count[k] < 0 where pair k needed more than ops_stride."""
+    n = len(len1)
+    scores = np.zeros(n, dtype=np.int32)
+    spans = np.zeros((n, 4), dtype=np.int32)
+    ops = np.zeros((n, ops_stride), dtype=np.uint32)
+    cnt = np.zeros(n, dtype=np.int32)
+    p = _params(params)
+    LL, I = C.POINTER(C.c_longlong), C.POINTER(C.c_int)
+    rc = _lib.load().swb200_align_long_batch(_ptr(flat1), off1.ctypes.data_as(LL), len1.ctypes.data_as(I), _ptr(flat2),
+                                             off2.ctypes.data_as(LL), len2.ctypes.data_as(I), n, C.byref(p), None,
+                                             scores.ctypes.data_as(I), spans.ctypes.data_as(I),
+                                             ops.ctypes.data_as(C.POINTER(C.c_uint)), ops_stride, cnt.ctypes.data_as(I))
+    if rc != 0:
+        raise SwbError(rc, "swb200_align_long_batch")
+    return scores, spans, ops, cnt
+
+
+def align_long_batch(seqs1, seqs2, params: Sequence[int] = DEFAULT_PARAMS, *, ops_stride: int = LONG_OPS_STRIDE):
+    """(scores int32[n], spans int32[n, 4], cigars list[str]): align(seqs1[k], seqs2[k]) for every pair of any size, in
+    one batch call (swb200_align_long_batch; the limits of score_long_batch).  Pairs whose alignment needs more than
+    ops_stride operations are aligned again with room for len1 + len2 operations, which always suffices."""
+    if len(seqs1) != len(seqs2):
+        raise ValueError("seqs1 and seqs2 differ in length")
+    f1, o1, l1 = _flatten(seqs1)
+    f2, o2, l2 = _flatten(seqs2)
+    scores, spans, ops, cnt = align_long_batch_ops(f1, o1, l1, f2, o2, l2, params, ops_stride)
+    cigars = [cigar_string(ops[k, :c]) if c >= 0 else None for k, c in enumerate(cnt.tolist())]
+    redo = np.flatnonzero(cnt < 0)
+    if len(redo):
+        stride = int((l1[redo].astype(np.int64) + l2[redo]).max())
+        _, _, ops2, cnt2 = align_long_batch_ops(f1, o1[redo].copy(), l1[redo].copy(), f2, o2[redo].copy(), l2[redo].copy(),
+                                                params, stride)
         for r, k in enumerate(redo.tolist()):
             cigars[k] = cigar_string(ops2[r, :cnt2[r]])
     return scores, spans, cigars

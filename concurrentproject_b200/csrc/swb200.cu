@@ -14,6 +14,7 @@
 #include "swb_banded.cuh"
 #include "swb_align_batch.cuh"
 #include "swb_align_banded.cuh"
+#include "swb_align_long.cuh"
 
 #include <cstdio>
 #include <cstdlib>
@@ -2643,13 +2644,93 @@ int align_banded_packed_locked(swb200_ctx* c, const BatchView& v, int band_lo, c
   return SWB200_OK;
 }
 
+constexpr int kLongTraceCtasPerSm = 4;    // 16 warps per SM trace (each owns a direction slot); the span kernel runs full
+
+// Direction storage of the long-pair alignment, in 64-bit words: *slot per warp of the trace launch and *pool shared.
+// A slot holds the largest span the batch can have (max_long x max_short), capped so that the slots of all nw warps take
+// at most a fifth of the device memory free to this context (free memory plus the slots it already holds): with the
+// quarter of headroom grow() adds, under a quarter.  The pool, used only when a span exceeds a slot, gets the same
+// share, and at least the largest span (its first taker always fits).  On a 180 GB B200 with 2 368 trace warps: 5 kb
+// pairs need 12.9 MB a span, 30.5 GB of slots in all, one trace round; 20 kb pairs need 202 MB a span, get 15 MB slots
+// and share a ~35 GB pool, about 170 spans a round.
+static int long_dir_budget(swb200_ctx* c, const BatchView& v, long long nw, long long* slot, size_t* pool) {
+  size_t fr = 0, tot = 0;
+  SWB_CUDA(cudaMemGetInfo(&fr, &tot));
+  const long long share = (long long)((fr + c->ab_slot_cap * sizeof(uint64_t)) / 5 / sizeof(uint64_t));
+  const long long largest = (swb::long_dir_words(v.max_long, v.max_short) + 1) / 2;
+  *slot = std::max(1LL, std::min(largest, share / nw));
+  *pool = (size_t)std::max(largest, std::max(kAlignPoolWords, share));
+  return SWB200_OK;
+}
+
+// Passes 1-3 and the walk over a packed range (shorter sequence first, len1 = the caller's seq1 lengths) whose shorter
+// side may exceed 1024, everything on stream s of c's device: one warp per pair, warps drawing pairs from a counter,
+// the trace rounds of align_rounds_locked.
+int align_long_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, const swb200_params& p, cudaStream_t s,
+                             int* d_scores, int* d_spans, uint32_t* d_ops, int ops_stride, int* d_ops_count,
+                             swb200_run_info* info) {
+  if (v.npairs == 0) return SWB200_OK;
+  constexpr int W = swb::kLongAlignWarps;
+  int span_sm = 0, trace_sm = 0;
+  SWB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&span_sm, swb::align_long_span_kernel_ptr(), 32 * W, 0));
+  SWB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&trace_sm, swb::align_long_trace_kernel_ptr(), 32 * W, 0));
+  const long long want = (v.npairs + W - 1) / W;
+  const long long span_blocks = std::max(1LL, std::min<long long>(want, (long long)c->sms * std::max(1, span_sm)));
+  const long long blocks = std::max(1LL, std::min<long long>(want, (long long)c->sms * std::max(1, std::min(trace_sm, kLongTraceCtasPerSm))));
+  const long long nw = blocks * W;
+  const long long row_stride = ((long long)std::max(v.max_long, 1) + 31) / 32 * 32;   // int2 entries, 128-byte lines
+  long long slot_words = 0;
+  size_t pool_need = 0;
+  int rc;
+  if ((rc = long_dir_budget(c, v, nw, &slot_words, &pool_need)) ||
+      (rc = grow(c->lb_bnd, c->lb_bnd_cap, (size_t)(2 * row_stride * std::max(span_blocks, blocks) * W), false, s)) ||
+      (rc = grow(c->ab_slot, c->ab_slot_cap, (size_t)(slot_words * nw), false, s)) ||
+      (rc = grow(c->ab_list, c->ab_list_cap, 2 * (size_t)v.npairs, false, s)) ||
+      (rc = grow(c->ab_misc, c->ab_misc_cap, 5, false, s))) return rc;
+  // [0] err | npending << 32, [1] pool words used, [2] cells, [3] the span kernel's pair counter, [4] the trace kernel's
+  SWB_CUDA(cudaMemsetAsync(c->ab_misc, 0, 5 * sizeof(unsigned long long), s));
+  swb::AlignBatchParams P{};
+  P.q_words = v.q_words; P.t_words = v.t_words; P.q_len = v.q_len; P.t_len = v.t_len; P.len1 = d_len1;
+  P.q_stride = v.q_stride; P.t_stride = v.t_stride; P.npairs = v.npairs;
+  P.match = p.match; P.mismatch = p.mismatch; P.gap_init = p.gap_init; P.gap_ext = p.gap_ext;
+  P.scores = d_scores; P.spans = d_spans;
+  P.col = reinterpret_cast<int2*>(c->lb_bnd); P.row_stride = row_stride; P.nthreads = nw * 32;
+  P.slot = c->ab_slot; P.slot_words = slot_words; P.pool = c->ab_pool; P.pool_words = (long long)c->ab_pool_cap;
+  P.pool_used = c->ab_misc + 1;
+  P.todo = nullptr; P.ntodo = v.npairs;
+  P.pending = c->ab_list; P.npending = reinterpret_cast<int*>(c->ab_misc) + 1;
+  P.ops = d_ops; P.ops_stride = ops_stride; P.ops_count = d_ops_count;
+  P.err = reinterpret_cast<int*>(c->ab_misc); P.cells = c->ab_misc + 2;
+  P.next = c->ab_misc + 3;
+  swb::launch_align_long_span(P, (int)span_blocks, s);
+  P.next = c->ab_misc + 4;
+  swb::launch_align_long_trace(P, (int)blocks, s);
+  SWB_CUDA(cudaGetLastError());
+  info->engine_launches += 2;
+  // spans larger than a slot: the pool, emptied for every round (the relaunch restarts the trace kernel's counter; a
+  // failed memset shows in align_rounds_locked's cudaGetLastError)
+  if ((rc = align_rounds_locked(c, s, v.npairs, pool_need, info, [&](const int* todo, int ntodo, int* pending) {
+         cudaMemsetAsync(c->ab_misc + 4, 0, sizeof(unsigned long long), s);
+         P.pool = c->ab_pool; P.pool_words = (long long)c->ab_pool_cap;
+         P.todo = todo; P.ntodo = ntodo; P.pending = pending;
+         swb::launch_align_long_trace(P, (int)std::max(1LL, std::min<long long>(blocks, (ntodo + W - 1) / W)), s);
+       }))) return rc;
+  info->lanes = 32; info->config = 320; info->rows = swb::kLongLaneRows;
+  info->bands = std::max(1, (v.max_short + swb::kLongBandRows - 1) / swb::kLongBandRows);
+  info->ctas = (int)blocks; info->warps = (int)nw;
+  return SWB200_OK;
+}
+
 }  // namespace
+
+// which kernels a host batch alignment runs
+enum class AlignKind { batch, banded, long_pairs };
 
 // One context's share of a host batch alignment (arguments checked by the caller): the copy/pack pipeline of the score
 // calls, then the passes over the whole range, then the outputs back.  banded: the pairs stay in caller order and the
 // banded passes run with band band_lo .. band_lo + 63.
 static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part, const PairScan& whole,
-                                const swb200_params& p, bool banded, int band_lo, int* scores_out, int* spans_out,
+                                const swb200_params& p, AlignKind kind, int band_lo, int* scores_out, int* spans_out,
                                 unsigned int* ops_out, int ops_stride, int* ops_count) {
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
@@ -2661,14 +2742,22 @@ static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npa
       (rc = grow(c->hb_ops, c->hb_ops_cap, np * (size_t)ops_stride, false, sc)) || (rc = grow(c->hb_opsn, c->hb_opsn_cap, np, false, sc))) return rc;
   c->info = swb200_run_info{};
   BatchView v;
-  if ((rc = stage_and_pack_locked(c, h, npairs, part, whole, banded, &v, nullptr))) return rc;
+  if ((rc = stage_and_pack_locked(c, h, npairs, part, whole, kind == AlignKind::banded, &v, nullptr))) return rc;
   SWB_CUDA(cudaMemcpyAsync(c->h_result, c->d_result, 2 * sizeof(int), cudaMemcpyDeviceToHost, sk));
   SWB_CUDA(cudaStreamSynchronize(sk));
   SWB_CUDA(cudaStreamSynchronize(sc));
   if (c->h_result[1] & swb::STATUS_BAD_SYMBOL) return fail(SWB200_ERR_ALPHABET, "batch input contains bytes other than A,C,G,T");
   SWB_CUDA(cudaMemsetAsync(c->hb_ops, 0, np * (size_t)ops_stride * sizeof(uint32_t), sk));   // overflowed pairs come back as zeros
-  rc = banded ? align_banded_packed_locked(c, v, band_lo, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info)
-              : align_packed_locked(c, v, c->hb_len1, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info);
+  switch (kind) {
+    case AlignKind::banded:
+      rc = align_banded_packed_locked(c, v, band_lo, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info);
+      break;
+    case AlignKind::long_pairs:
+      rc = align_long_packed_locked(c, v, c->hb_len1, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info);
+      break;
+    default:
+      rc = align_packed_locked(c, v, c->hb_len1, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info);
+  }
   if (rc) return rc;
   SWB_CUDA(cudaEventRecord(c->ev1, sk));
   SWB_CUDA(cudaMemcpyAsync(scores_out, c->hb_scores, np * sizeof(int), cudaMemcpyDeviceToHost, sk));
@@ -2703,7 +2792,7 @@ int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, con
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, false, 0, scores_out + k0, spans_out + 4 * k0,
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::batch, 0, scores_out + k0, spans_out + 4 * k0,
                                     ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
       });
 }
@@ -2738,7 +2827,7 @@ int swb200_align_banded_batch(const unsigned char* seq1_all, const long long* of
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, true, band_lo, scores_out + k0, spans_out + 4 * k0,
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::banded, band_lo, scores_out + k0, spans_out + 4 * k0,
                                     ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
       });
 }
@@ -2753,6 +2842,40 @@ int swb200_batch_align_banded(swb200_batch* b, int band_lo, int band_hi, const s
   if ((rc = check_params(p)) || (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
   return run_device_batch(b, 0, stream, [&](swb200_ctx* c, cudaStream_t s) {
     return align_banded_packed_locked(c, whole_batch(b), band_lo, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info);
+  });
+}
+
+int swb200_align_long_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                            const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                            const swb200_params* pp, const swb200_options* opt, int* scores_out, int* spans_out,
+                            unsigned int* ops_out, int ops_stride, int* ops_count) {
+  (void)opt;
+  if (npairs < 0 || ops_stride < 1 ||
+      (npairs > 0 && (!seq1_all || !seq2_all || !off1 || !off2 || !len1 || !len2 || !scores_out || !spans_out || !ops_out || !ops_count)))
+    return fail(SWB200_ERR_ARG, "bad batch arguments");
+  const swb200_params p = params_or_default(pp);
+  const HostPairs in{seq1_all, off1, len1, seq2_all, off2, len2};
+  auto check = [&](const PairScan& whole) { return check_score_pairs(whole, p, swb200_options{}, ScoreKind::long_pairs, 0, 0); };
+  if (npairs == 0) return check(PairScan{});
+  return run_host_batch(
+      npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
+      [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::long_pairs, 0, scores_out + k0,
+                                    spans_out + 4 * k0, ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
+      });
+}
+
+int swb200_batch_align_long(swb200_batch* b, const swb200_params* pp, const swb200_options* opt, void* stream, int* d_scores,
+                            int* d_spans, unsigned int* d_ops, int ops_stride, int* d_ops_count) {
+  (void)opt;
+  if (!b || ops_stride < 1 || (b->npairs > 0 && (!d_scores || !d_spans || !d_ops || !d_ops_count)))
+    return fail(SWB200_ERR_ARG, "bad batch arguments");
+  if (b->keep_order || !b->len1) return fail(SWB200_ERR_ARG, "batch was packed in caller order (banded); re-pack with keep_order=0");
+  const swb200_params p = params_or_default(pp);
+  int rc;
+  if ((rc = check_params(p)) || (rc = check_long_score(p, swb200_options{}, 0, b->max_short))) return rc;
+  return run_device_batch(b, 0, stream, [&](swb200_ctx* c, cudaStream_t s) {
+    return align_long_packed_locked(c, whole_batch(b), b->len1, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info);
   });
 }
 

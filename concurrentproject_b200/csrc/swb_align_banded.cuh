@@ -171,32 +171,44 @@ SWB_HD long long band_span_pair(const AlignBandedParams& P, const WarpCtx& w, lo
   return nc;
 }
 
+// The run-length encoder of the warp walks (band_walk, long_walk).  Operations arrive last-first; WRITE = false counts
+// them and re-scores, WRITE = true stores them first-first (ops[n - 1 - t]).  tot sums main.cpp's costs of the runs.
+// emit(..., opened = true) for a gap that was opened ends its run when gap_ext > gap_init (two gaps, not one extended).
+template <bool WRITE>
+struct OpEncoder {
+  int match, mismatch, gap_init, gap_ext;
+  uint32_t* ops;
+  int n;
+  int nops = 0, run = 0;
+  uint32_t cur = 0;
+  bool brk = false;
+  long long tot = 0;
+  SWB_HD void flush() {
+    if (run <= 0) return;
+    if (cur == kOpEq) tot += (long long)run * match;
+    else if (cur == kOpX) tot += (long long)run * mismatch;
+    else tot -= gap_init + (long long)(run - 1) * gap_ext;
+    if (WRITE) ops[n - 1 - nops] = ((uint32_t)run << 4) | cur;
+    ++nops;
+  }
+  SWB_HD void emit(uint32_t op, int cnt, bool opened = false) {
+    if (op == cur && !brk) run += cnt;
+    else { flush(); cur = op; run = cnt; }
+    brk = opened && gap_ext > gap_init;
+  }
+};
+
 // The walk over the direction lines of a span (band lo, X / Y as pass 3 saw them) from its last cell back to (0, 0).
 // Lane 0 walks; before it runs out of staged lines the warp copies the next kBandStageLines lines below into stage.
-// Operations come out last-first; WRITE = false counts them and re-scores, WRITE = true stores them first-first
-// (ops[n - 1 - t]).  Returns the count and *total in every lane; a step out of the band poisons *total.
+// Operations come out last-first (OpEncoder).  Returns the count and *total in every lane; a step out of the band
+// poisons *total.
 template <bool WRITE>
 SWB_HD int band_walk(const AlignBandedParams& P, const WarpCtx& w, const uint32_t* dirs, const AlignSeq& X, const AlignSeq& Y,
                      int lo, uint32_t* stage, int n, uint32_t* ops, int* total) {
   const int lane = w.lane;
-  const bool split = P.gap_ext > P.gap_init;
-  int x = X.len, y = Y.len, state = 0, nops = 0, run = 0;
-  uint32_t cur = 0;
-  bool brk = false, outside = false;
-  long long tot = 0;
-  auto flush = [&]() {
-    if (run <= 0) return;
-    if (cur == kOpEq) tot += (long long)run * P.match;
-    else if (cur == kOpX) tot += (long long)run * P.mismatch;
-    else tot -= P.gap_init + (long long)(run - 1) * P.gap_ext;
-    if (WRITE) ops[n - 1 - nops] = ((uint32_t)run << 4) | cur;
-    ++nops;
-  };
-  auto emit = [&](uint32_t op, int cnt) {
-    if (op == cur && !brk) { run += cnt; return; }
-    flush();
-    cur = op; run = cnt; brk = false;
-  };
+  int x = X.len, y = Y.len, state = 0;
+  bool outside = false;
+  OpEncoder<WRITE> enc{P.match, P.mismatch, P.gap_init, P.gap_ext, ops, n};
   for (;;) {
     const int top = (int)w.shfl((uint32_t)((x + y) >> 3), 0);
     const int base = top - kBandStageLines + 1 > 0 ? top - kBandStageLines + 1 : 0;
@@ -213,20 +225,18 @@ SWB_HD int band_walk(const AlignBandedParams& P, const WarpCtx& w, const uint32_
         const uint32_t d = (stage[((t >> 3) - base) * 32 + (int)(kl >> 1)] >> (4 * (t & 7))) & 0xFu;
         if (state == 0) {
           const uint32_t src = d & 3u;
-          if (src == 0) { emit(align_code(X, x - 1) == align_code(Y, y - 1) ? kOpEq : kOpX, 1); --x; --y; }
+          if (src == 0) { enc.emit(align_code(X, x - 1) == align_code(Y, y - 1) ? kOpEq : kOpX, 1); --x; --y; }
           else state = (int)src;
         } else if (state == 1) {                   // E: a base of seq1 against a gap
-          emit(kOpIns, 1);
           const bool opened = !(d & 4u);
+          enc.emit(kOpIns, 1, opened);
           state = opened ? 0 : 1;
           --x;
-          brk = opened && split;
         } else {                                   // F: a base of seq2 against a gap
-          emit(kOpDel, 1);
           const bool opened = !(d & 8u);
+          enc.emit(kOpDel, 1, opened);
           state = opened ? 0 : 2;
           --y;
-          brk = opened && split;
         }
       }
       done = outside || !(x > 0 && y > 0);
@@ -236,13 +246,13 @@ SWB_HD int band_walk(const AlignBandedParams& P, const WarpCtx& w, const uint32_
   int tl = 0;
   if (lane == 0) {
     // the rest runs along row 0 or column 0 of the span: leading gaps, in the band because (0, 0) and (x, y) are
-    if (x > 0) emit(kOpIns, x);
-    if (y > 0) emit(kOpDel, y);
-    flush();
-    tl = outside ? kAlignNeg : (int)tot;
+    if (x > 0) enc.emit(kOpIns, x);
+    if (y > 0) enc.emit(kOpDel, y);
+    enc.flush();
+    tl = outside ? kAlignNeg : (int)enc.tot;
   }
   *total = (int)w.shfl((uint32_t)tl, 0);
-  return (int)w.shfl((uint32_t)nops, 0);
+  return (int)w.shfl((uint32_t)enc.nops, 0);
 }
 
 // Pass 3 and the walk for pair k (score and span from band_span_pair).  Returns this lane's in-band cells, or -1 if the

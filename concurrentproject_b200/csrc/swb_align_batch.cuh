@@ -72,6 +72,10 @@ struct AlignBatchParams {
   int* ops_count;            // per pair: number of operations, -(number) if more than ops_stride
   int* err;                  // kAlignErr* bits
   unsigned long long* cells; // cells the passes computed (one atomic add per thread and launch)
+  // the long-pair kernels (swb_align_long.cuh) only: col is one boundary row of row_stride entries per launched warp,
+  // warp w's at col + w * row_stride, slot_words counts per warp, and warps draw pairs from the counter *next
+  long long row_stride;
+  unsigned long long* next;
 };
 
 // A view of 2-bit symbols: positions [0, len) of words at off (forward) or of off + len - 1 downwards (reversed).

@@ -14,7 +14,11 @@ to the GPU kernels:
                          batch kernel (swb200_batch_score_long), everything else (a few long pairs, or other
                          alphabets such as N or amino acids) through the single-pair engine (swb200_score_ex), which compares bytes
                          exactly like main.cpp:60;
-* ``search``          -- one query against every record of a database.
+* ``search``          -- one query against every record of a database;
+* ``align_pairs``     -- score, span and CIGAR of (seqs1[k], seqs2[k]), each as api.align returns it: ACGT pairs whose
+                         shorter side is <= 1024 through the batch alignment (swb200_batch_align), longer ACGT pairs,
+                         when the batch beats one call per pair (align_long_batch_pays), through the long-pair batch
+                         alignment (swb200_batch_align_long), everything else pair by pair (swb200_align_device).
 
 The residues are uploaded to HBM once per call (torch is the plumbing for device memory); a bucket only ships its
 offsets and lengths and is packed and scored where the bytes already are.  There is no CPU scoring path here."""
@@ -37,6 +41,14 @@ BATCH_MAX_SHORT = 1024
 # So a few long pairs stay on the single-pair engine (20 kb: 64 pairs take 0.04 s there, 0.07 s in the batch).
 LOOP_CALL_S, LOOP_CELL_S = 1.8e-4, 1.25e-12
 LONG_CALL_S, LONG_WARP_CUPS, LONG_GPU_CUPS = 3e-4, 5.9e9, 8.3e12
+# The same form for alignment (align_long_batch_pays), fitted to the crossover of bench/align_long_batch.py
+# (profiles/r07_align_long_batch.json; one NVIDIA B200, power limit 1000 W).  One single-pair alignment costs
+# ALIGN_LOOP_CALL_S + ALIGN_LOOP_CELL_S per cell (12, 38 ms for a 5, 20 kb pair; measured on 16 pairs: 12.8, 8.7 and
+# 36.8 ms for 2, 5 and 20 kb, and the per-pair loop varies between runs, so these are fitted to the decisions, not to
+# the times).  The long-pair alignment call costs ALIGN_LONG_CALL_S plus the longer of its tallest pair on one warp and
+# all padded cells (256-row bands, three passes) on the whole GPU.
+ALIGN_LOOP_CALL_S, ALIGN_LOOP_CELL_S = 1.03e-2, 6.9e-11
+ALIGN_LONG_CALL_S, ALIGN_LONG_WARP_CUPS, ALIGN_LONG_GPU_CUPS = 2e-3, 4.6e8, 1.0e11
 _IS_ACGT = np.zeros(256, dtype=bool)
 _IS_ACGT[[ord(c) for c in "ACGT"]] = True
 
@@ -126,14 +138,29 @@ def long_batch_pays(short: np.ndarray, long_: np.ndarray) -> bool:
     return batch < loop
 
 
-def plan_buckets(len1: np.ndarray, len2: np.ndarray, acgt_only: np.ndarray, min_bucket: int = 512, match: int = 1) -> List[Bucket]:
+def align_long_batch_pays(short: np.ndarray, long_: np.ndarray) -> bool:
+    """True when one long-pair alignment call (swb200_batch_align_long) over these pairs is expected to beat one
+    swb200_align_device call each."""
+    short = np.asarray(short, dtype=np.int64)
+    long_ = np.asarray(long_, dtype=np.int64)
+    if short.size == 0:
+        return False
+    padded = (3 * -(-short // 256) * 256 * (long_ + 31)).astype(np.float64)
+    loop = short.size * ALIGN_LOOP_CALL_S + float((short * long_).sum()) * ALIGN_LOOP_CELL_S
+    batch = ALIGN_LONG_CALL_S + max(float(padded.max()) / ALIGN_LONG_WARP_CUPS, float(padded.sum()) / ALIGN_LONG_GPU_CUPS)
+    return batch < loop
+
+
+def plan_buckets(len1: np.ndarray, len2: np.ndarray, acgt_only: np.ndarray, min_bucket: int = 512, match: int = 1, *,
+                 pays=long_batch_pays) -> List[Bucket]:
     """Partition pair ids.  Batch buckets are keyed by the capacity class of min(len1, len2); a class with fewer
     than ``min_bucket`` pairs is merged into the next larger one (a launch costs more than the padding).  Inside a
     bucket pairs are ordered by max(len1, len2), longest first.  ACGT pairs with a shorter side over BATCH_MAX_SHORT
     form one "long" bucket, ordered by padded cells, largest first (the multi-band kernel's warps take pairs in this
     order, so the longest pairs start first), when that call beats the single-pair engine (long_batch_pays).  Pairs the 16-bit batch
     kernels cannot hold (match * min(len) > 32766 - match, swb200.cu: check_batch_score) go to the single-pair engine,
-    which re-runs in re-based or 32-bit lanes by itself."""
+    which re-runs in re-based or 32-bit lanes by itself.  ``pays`` judges the "long" bucket: long_batch_pays for
+    scoring, align_long_batch_pays for alignment."""
     len1 = np.asarray(len1, dtype=np.int64)
     len2 = np.asarray(len2, dtype=np.int64)
     short = np.minimum(len1, len2)
@@ -141,7 +168,7 @@ def plan_buckets(len1: np.ndarray, len2: np.ndarray, acgt_only: np.ndarray, min_
     in_range = np.asarray(acgt_only, dtype=bool) & (int(match) * short <= 32766 - int(match))
     batchable = in_range & (short <= BATCH_MAX_SHORT)
     long_ids = np.flatnonzero(in_range & (short > BATCH_MAX_SHORT))
-    if not long_batch_pays(short[long_ids], long_[long_ids]):
+    if not pays(short[long_ids], long_[long_ids]):
         long_ids = long_ids[:0]
     out: List[Bucket] = []
     edges = np.array(BUCKET_EDGES)
@@ -263,9 +290,11 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
                   params: Sequence[int] = api.DEFAULT_PARAMS, *, min_bucket: int = 512, device: int = 0,
                   ops_stride: int = api.OPS_STRIDE):
     """Align pair k = (a[ia[k]], b[ib[k]]): (scores int32[n], spans int32[n, 4], cigars list[str]) in pair order, each
-    as api.align returns it.  The buckets of score_records: batch buckets are packed in place and aligned by
-    swb200_batch_align (pairs that need more than ops_stride operations once more with room for len1 + len2); the
-    rest (bytes other than A,C,G,T, a shorter side over 1024) pair by pair through swb200_align_device."""
+    as api.align returns it.  The buckets of score_records, with the long bucket judged by align_long_batch_pays: batch
+    buckets are packed in place and aligned by swb200_batch_align, the long bucket by swb200_batch_align_long (pairs
+    that need more than ops_stride, or api.LONG_OPS_STRIDE, operations once more with room for len1 + len2); the rest
+    (bytes other than A,C,G,T, long pairs where the batch does not pay, pairs whose span could not get direction
+    storage) pair by pair through swb200_align_device."""
     import torch
     ia = np.asarray(ia, dtype=np.int64)
     ib = np.asarray(ib, dtype=np.int64)
@@ -286,10 +315,15 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
         fb, ok_b = (fa, ok_a) if b is a else _device_records(b, torch, dev)
         l1, l2 = a.lengths[ia].astype(np.int32), b.lengths[ib].astype(np.int32)
         o1, o2 = a.offsets[ia].astype(np.int64), b.offsets[ib].astype(np.int64)
-        buckets = plan_buckets(l1, l2, ok_a[ia] & ok_b[ib], min_bucket, match=int(params[0]))
+        # a long pair goes to the batch only if direction storage for its largest possible span (4 bits a cell in
+        # 256-row bands) takes at most a quarter of the free device memory
+        short = np.minimum(l1, l2).astype(np.int64)
+        dir_bytes = -(-short // 256) * (np.maximum(l1, l2).astype(np.int64) + 31) * 128
+        fits = (short <= BATCH_MAX_SHORT) | (dir_bytes <= torch.cuda.mem_get_info(dev)[0] // 4)
+        buckets = plan_buckets(l1, l2, ok_a[ia] & ok_b[ib] & fits, min_bucket, match=int(params[0]), pays=align_long_batch_pays)
         stream = torch.cuda.current_stream(dev).cuda_stream
 
-        def run(ids, stride):
+        def run(ids, stride, long_pairs=False):
             bl1, bl2 = l1[ids], l2[ids]
             d_o1 = torch.from_numpy(o1[ids]).to(dev); d_o2 = torch.from_numpy(o2[ids]).to(dev)
             d_l1 = torch.from_numpy(bl1).to(dev); d_l2 = torch.from_numpy(bl2).to(dev)
@@ -302,15 +336,17 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
             pb = api.PackedBatch(ctx, fa.data_ptr(), d_o1.data_ptr(), d_l1.data_ptr(), fb.data_ptr(), d_o2.data_ptr(),
                                  d_l2.data_ptr(), len(ids), int(short.max()), int(long_.max()), cells, stream=stream)
             try:
-                pb.align(d_sc.data_ptr(), d_sp.data_ptr(), d_ops.data_ptr(), stride, d_cnt.data_ptr(), params, stream=stream)
+                align = pb.align_long if long_pairs else pb.align
+                align(d_sc.data_ptr(), d_sp.data_ptr(), d_ops.data_ptr(), stride, d_cnt.data_ptr(), params, stream=stream)
             finally:
                 pb.close()
             return d_sc.cpu().numpy(), d_sp.cpu().numpy(), d_ops.cpu().numpy().view(np.uint32), d_cnt.cpu().numpy()
 
         for bk in buckets:
             ids = bk.index
-            if bk.kind == "batch":
-                sc, sp, ops, cnt = run(ids, ops_stride)
+            if bk.kind in ("batch", "long"):
+                lp = bk.kind == "long"
+                sc, sp, ops, cnt = run(ids, api.LONG_OPS_STRIDE if lp else ops_stride, lp)
                 scores[ids] = sc
                 spans[ids] = sp
                 for r, pid in enumerate(ids.tolist()):
@@ -318,7 +354,7 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
                         cigars[pid] = api.cigar_string(ops[r, :cnt[r]])
                 redo = ids[cnt < 0]
                 if len(redo):
-                    _, _, ops2, cnt2 = run(redo, int((l1[redo].astype(np.int64) + l2[redo]).max()))
+                    _, _, ops2, cnt2 = run(redo, int((l1[redo].astype(np.int64) + l2[redo]).max()), lp)
                     for r, pid in enumerate(redo.tolist()):
                         cigars[pid] = api.cigar_string(ops2[r, :cnt2[r]])
             else:

@@ -284,6 +284,27 @@ SWB200_API int swb200_align_batch(const unsigned char* seq1_all, const long long
 SWB200_API int swb200_batch_align(swb200_batch* batch, const swb200_params* p, const swb200_options* opt, void* stream,
                                   int* d_scores, int* d_spans, unsigned int* d_ops, int ops_stride, int* d_ops_count);
 
+/* Batch alignment without the 1024 cap: for every pair k the score, span and operations that swb200_align returns for
+ * that pair alone, with swb200_align_batch's tie rules, output format, ops_stride overflow rule (ops_count = -n; the host
+ * call zero-fills that slot), "1I1I" split when gap_ext > gap_init (the one documented difference from swb200_align) and
+ * device re-score (SWB200_ERR_CUDA "internal: ..." on a mismatch).  One warp per pair, the shorter sequence cut into bands
+ * of 256 rows (DESIGN.md section 4e); short pairs are accepted too.  Limits and errors are swb200_score_long_batch's, so
+ * every score can be checked against it: bytes A,C,G,T (SWB200_ERR_ALPHABET); match*min(len) <= 32766 - match
+ * (SWB200_ERR_RANGE).  SWB200_ERR_NOMEM when the boundary rows, or direction storage for the largest span the batch can
+ * have (4 bits per cell of max(len) x max(min(len)), in 256-row bands), cannot be allocated: swb200_align, whose blocked
+ * traceback needs no such storage, is the route for those pairs.  All argument checks run before a device is touched.
+ * The host call packs in chunks and shards over swb200_set_devices like swb200_align_batch (results identical for every
+ * G).  swb200_last_run: config 320, lanes 32, rows 8, bands = the band count of the tallest pair, cells summed over the
+ * three passes.  opt is reserved (NULL). */
+SWB200_API int swb200_align_long_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                                       const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                                       const swb200_params* p, const swb200_options* opt, int* scores_out, int* spans_out,
+                                       unsigned int* ops_out, int ops_stride, int* ops_count);
+/* The same for a device-resident batch packed with keep_order = 0 (SWB200_ERR_ARG for keep_order = 1); every output
+ * pointer is a DEVICE pointer. */
+SWB200_API int swb200_batch_align_long(swb200_batch* batch, const swb200_params* p, const swb200_options* opt, void* stream,
+                                       int* d_scores, int* d_spans, unsigned int* d_ops, int ops_stride, int* d_ops_count);
+
 /* ---- banded batches (long reads): cell (i,j), i = row in seq2, j = column in seq1, is scored iff
  * band_lo <= j - i <= band_hi; everything outside the band is H=E=F=0 and excluded from the max.  The reference
  * has no banded mode; semantics = main.cpp:57-63 restricted to the band (oracle: oracle_gotoh_banded).
