@@ -264,7 +264,9 @@ def score_long_batch_flat(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray,
 
 def score_banded_batch(seqs1, seqs2, band_lo: int = -32, band_hi: int = 31, params: Sequence[int] = DEFAULT_PARAMS, *,
                        no_linear: bool = False, config: int = 0) -> np.ndarray:
-    """Banded scores of many HOST pairs: cell (i, j) counts iff band_lo <= j - i <= band_hi (64 diagonals)."""
+    """Banded scores of many HOST pairs: cell (i, j) counts iff band_lo <= j - i <= band_hi.  The band holds
+    band_hi - band_lo + 1 = 64, 128, 256 or 512 diagonals (any other width raises SwbError -2); `config` picks among the
+    64-diagonal layouts and is ignored for wider bands."""
     if len(seqs1) != len(seqs2):
         raise ValueError("seqs1 and seqs2 differ in length")
     return score_banded_batch_flat(*_flatten(seqs1), *_flatten(seqs2), band_lo, band_hi, params, no_linear=no_linear,
@@ -335,8 +337,8 @@ class PackedBatch:
 
     def align_banded(self, d_scores: int, d_spans: int, d_ops: int, ops_stride: int, d_ops_count: int, band_lo: int = -32,
                      band_hi: int = 31, params: Sequence[int] = DEFAULT_PARAMS, *, stream: int = 0) -> None:
-        """Score, span and alignment operations of every pair inside the band band_lo <= j - i <= band_hi
-        (swb200_batch_align_banded; the batch must be packed with keep_order=True).  Device outputs as align writes them."""
+        """Score, span and alignment operations of every pair inside the band band_lo <= j - i <= band_hi of 64, 128,
+        256 or 512 diagonals (swb200_batch_align_banded; the batch must be packed with keep_order=True).  Device outputs as align writes them."""
         p = _params(params)
         rc = _lib.load().swb200_batch_align_banded(self.handle, band_lo, band_hi, C.byref(p), None, C.c_void_p(stream),
                                                    C.c_void_p(d_scores), C.c_void_p(d_spans), C.c_void_p(d_ops), ops_stride,
@@ -574,8 +576,8 @@ def align_banded_batch_ops(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray
 def align_banded_batch(seqs1, seqs2, band_lo: int = -32, band_hi: int = 31, params: Sequence[int] = DEFAULT_PARAMS, *,
                        ops_stride: int = BANDED_OPS_STRIDE):
     """(scores int32[n], spans int32[n, 4], cigars list[str]): the best local alignment of every pair inside the band
-    band_lo <= j - i <= band_hi (64 diagonals), in one batch call (swb200_align_banded_batch; the limits of
-    score_banded_batch).  Pairs whose alignment needs more than ops_stride operations are aligned again with room for
+    band_lo <= j - i <= band_hi (64, 128, 256 or 512 diagonals), in one batch call (swb200_align_banded_batch; the
+    limits of score_banded_batch).  Pairs whose alignment needs more than ops_stride operations are aligned again with room for
     len1 + len2 operations, which always suffices."""
     if len(seqs1) != len(seqs2):
         raise ValueError("seqs1 and seqs2 differ in length")

@@ -1547,42 +1547,55 @@ static int launch_long_score(swb200_ctx* c, const BatchView& v, const swb200_par
   return SWB200_OK;
 }
 
+// The band widths the banded kernels have: W = band_hi - band_lo + 1 in {64, 128, 256, 512}.  Every banded call checks
+// here first.
+static int check_band_width(int band_lo, int band_hi) {
+  const long long w = (long long)band_hi - band_lo + 1;
+  if (w != 64 && w != 128 && w != 256 && w != 512)
+    return fail(SWB200_ERR_ARG, "the banded kernels handle bands of 64, 128, 256 or 512 diagonals");
+  return SWB200_OK;
+}
+
 static int check_banded_score(const swb200_params& p, int keep_order, int band_lo, int band_hi, int max1, int max2) {
   if (!keep_order) return fail(SWB200_ERR_ARG, "banded scoring needs a batch packed with keep_order=1");
-  if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
+  if (int rc = check_band_width(band_lo, band_hi)) return rc;
   if ((long long)p.match * std::min(max1, max2) > 32767 - p.match - 1)
     return fail(SWB200_ERR_RANGE, "match * min(len) does not fit the 16-bit lanes of the banded kernel");
   return SWB200_OK;
 }
 
-// kernel, threads per CTA and pairs per CTA of the banded layout the options ask for
-static const void* banded_layout(const swb200_params& p, const swb200_options& o, int* threads, int* mode_out) {
+// Kernel, threads per CTA, pairs per CTA and run-info config code of the banded layout for a band of band_w diagonals
+// and the options.  64 diagonals: four layouts, 4 threads per pair with eight register sets each (the default), 8 threads
+// with four (options.config = 8), 16 threads with two (16) and 2 threads with sixteen (2), the last three kept for
+// comparison; 16 pairs per CTA in each.  128, 256, 512 diagonals: band_w / 16 threads per pair with eight register sets,
+// two warps and 1024 / band_w pairs per CTA, config 2128 / 2256 / 2512 whatever options.config says.
+struct BandedLayout {
+  const void* kern;
+  int threads, pairs_per_cta, config, mode;
+};
+static BandedLayout banded_layout(const swb200_params& p, const swb200_options& o, int band_w) {
   const int mode = (p.gap_init == p.gap_ext && !o.no_linear) ? 1 : 0;
+  if (band_w != swb::kBandWidth) return BandedLayout{swb::banded_wide_kernel(mode, band_w), 64, 1024 / band_w, 2000 + band_w, mode};
   const bool wide = o.config == 16, mid = o.config == 8, two = o.config == 2;
-  *threads = wide ? 256 : (mid ? 128 : (two ? 32 : 64));
-  if (mode_out) *mode_out = mode;
-  return wide ? swb::banded_kernel(mode) : (mid ? swb::banded8_kernel(mode) : (two ? swb::banded2_kernel(mode) : swb::banded4_kernel(mode)));
+  const void* kern = wide ? swb::banded_kernel(mode) : (mid ? swb::banded8_kernel(mode) : (two ? swb::banded2_kernel(mode) : swb::banded4_kernel(mode)));
+  return BandedLayout{kern, wide ? 256 : (mid ? 128 : (two ? 32 : 64)), 16, wide ? 216 : (mid ? 208 : (two ? 202 : 204)), mode};
 }
 
-// pairs one full wave of resident CTAs scores (16 pairs per CTA in every layout)
-static long long banded_wave_pairs(swb200_ctx* c, const swb200_params& p, const swb200_options& o) {
-  int threads = 0;
-  const void* kern = banded_layout(p, o, &threads, nullptr);
-  cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+// pairs one full wave of resident CTAs scores
+static long long banded_wave_pairs(swb200_ctx* c, const swb200_params& p, const swb200_options& o, int band_w) {
+  const BandedLayout L = banded_layout(p, o, band_w);
+  cudaFuncSetAttribute(L.kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   int per_sm = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-  return 16LL * c->sms * per_sm;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, L.kern, L.threads, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
+  return (long long)L.pairs_per_cta * c->sms * per_sm;
 }
 
-static int launch_banded_score(swb200_ctx* c, const BatchView& v, int band_lo, const swb200_params& p,
+static int launch_banded_score(swb200_ctx* c, const BatchView& v, int band_lo, int band_w, const swb200_params& p,
                                const swb200_options& o, cudaStream_t s, int* d_scores, swb200_run_info* info) {
   if (v.npairs == 0) return SWB200_OK;
-  // four layouts: 4 threads per pair with eight register sets each (the default), 8 threads with four (options.config =
-  // 8), 16 threads with two (16) and 2 threads with sixteen (2), the last three kept for comparison
-  const bool wide = o.config == 16, mid = o.config == 8, two = o.config == 2;
-  int threads = 0, mode = 0;
-  const void* kern = banded_layout(p, o, &threads, &mode);
-  const int pairs_per_cta = 16;
+  const BandedLayout L = banded_layout(p, o, band_w);
+  const void* kern = L.kern;
+  const int threads = L.threads, mode = L.mode, pairs_per_cta = L.pairs_per_cta;
   // several CTAs of 34-35 KB static shared memory per SM: ask for the large shared-memory carve-out
   cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   swb::BandedParams P{};
@@ -1595,8 +1608,8 @@ static int launch_banded_score(swb200_ctx* c, const BatchView& v, int band_lo, c
   const long long ctas = std::max<long long>(1, std::min<long long>((v.npairs + pairs_per_cta - 1) / pairs_per_cta, (long long)c->sms * per_sm));
   void* args[] = {&P};
   SWB_CUDA(cudaLaunchKernel(kern, dim3((unsigned)ctas), dim3((unsigned)threads), args, 0, s));
-  info->lanes = 16; info->linear = mode == 1; info->rows = 0; info->config = wide ? 216 : (mid ? 208 : (two ? 202 : 204)); info->ctas = (int)ctas;
-  info->warps = (int)ctas * (threads / 32); info->bands = swb::kBandWidth; info->engine_launches += 1;
+  info->lanes = 16; info->linear = mode == 1; info->rows = 0; info->config = L.config; info->ctas = (int)ctas;
+  info->warps = (int)ctas * (threads / 32); info->bands = band_w; info->engine_launches += 1;
   return SWB200_OK;
 }
 
@@ -1658,7 +1671,7 @@ int swb200_batch_score_banded(swb200_batch* b, int band_lo, int band_hi, const s
   int rc;
   if ((rc = check_params(p)) || (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
   return run_device_batch(b, b->cells, stream, [&](swb200_ctx* c, cudaStream_t s) {
-    return launch_banded_score(c, whole_batch(b), band_lo, p, o, s, d_scores, &c->info);
+    return launch_banded_score(c, whole_batch(b), band_lo, band_hi - band_lo + 1, p, o, s, d_scores, &c->info);
   });
 }
 
@@ -1806,7 +1819,8 @@ static int stage_and_pack_locked(swb200_ctx* c, const HostPairs& h, long long np
 // One context's share of a host ASCII score batch (arguments checked by the caller): every chunk is scored as soon as it
 // is packed, while the next one is copied.
 static int score_ascii_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part, const PairScan& whole,
-                           const swb200_params& p, const swb200_options& o, ScoreKind kind, int band_lo, int* scores_out) {
+                           const swb200_params& p, const swb200_options& o, ScoreKind kind, int band_lo, int band_w,
+                           int* scores_out) {
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
   SWB_CUDA(cudaSetDevice(c->device));
@@ -1819,7 +1833,7 @@ static int score_ascii_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, 
   const long long wave = kind == ScoreKind::long_pairs ? long_wave_pairs(c, p, o, whole.max_min) : 0;
   int rc = stage_and_pack_locked(c, h, npairs, part, whole, banded, &staged, [&](const BatchView& v, long long k0) {
     switch (kind) {
-      case ScoreKind::banded: return launch_banded_score(c, v, band_lo, p, o, sk, c->hb_scores + k0, &c->info);
+      case ScoreKind::banded: return launch_banded_score(c, v, band_lo, band_w, p, o, sk, c->hb_scores + k0, &c->info);
       case ScoreKind::long_pairs: return launch_long_score(c, v, p, o, sk, c->hb_scores + k0, &c->info);
       default: return launch_batch_score(c, v, p, o, sk, c->hb_scores + k0, &c->info);
     }
@@ -1840,7 +1854,7 @@ static int score_ascii_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, 
 int swb200_score_banded(const unsigned char* seq1, int n, const unsigned char* seq2, int m, int band_lo, int band_hi,
                         const swb200_params* p, int* score_out) {
   if (n < 0 || m < 0 || !score_out || (n > 0 && !seq1) || (m > 0 && !seq2)) return fail(SWB200_ERR_ARG, "bad sequence arguments");
-  if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
+  if (int rc = check_band_width(band_lo, band_hi)) return rc;
   *score_out = 0;
   if (n == 0 || m == 0) { if (p) { int rc = check_params(*p); if (rc) return rc; } return SWB200_OK; }
   const long long off = 0;
@@ -1850,7 +1864,7 @@ int swb200_score_banded(const unsigned char* seq1, int n, const unsigned char* s
   swb200_ctx* c = nullptr;
   int rc;
   if ((rc = check_score_pairs(s, pv, swb200_options{}, ScoreKind::banded, band_lo, band_hi)) || (rc = default_ctx(&c))) return rc;
-  return score_ascii_ctx(c, in, 1, s, s, pv, swb200_options{}, ScoreKind::banded, band_lo, score_out);
+  return score_ascii_ctx(c, in, 1, s, s, pv, swb200_options{}, ScoreKind::banded, band_lo, band_hi - band_lo + 1, score_out);
 }
 
 // ---- one pair over a ring of GPUs (one swb200_ring per GPU / per process) -------------------------
@@ -2221,7 +2235,7 @@ static int score_batch_host(const HostPairs& in, long long npairs, const swb200_
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); },
       [&](const PairScan& whole) { return check_score_pairs(whole, p, o, kind, band_lo, band_hi); },
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return score_ascii_ctx(c, in.from(k0), k1 - k0, part, whole, p, o, kind, band_lo, scores_out + k0);
+        return score_ascii_ctx(c, in.from(k0), k1 - k0, part, whole, p, o, kind, band_lo, band_hi - band_lo + 1, scores_out + k0);
       });
 }
 
@@ -2253,7 +2267,7 @@ static LenScan scan_lens(const int* q_len, const int* t_len, long long k0, long 
 static int score_batch_packed_ctx(swb200_ctx* c, const unsigned long long* q_words, long long q_stride,
                                   const unsigned long long* t_words, long long t_stride, const int* q_len, const int* t_len,
                                   long long npairs, int max_short, int max_long, long long cells, const swb200_params& pv,
-                                  const swb200_options& ov, int banded, int band_lo, int* scores_out) {
+                                  const swb200_options& ov, int banded, int band_lo, int band_w, int* scores_out) {
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
   SWB_CUDA(cudaSetDevice(c->device));
@@ -2270,7 +2284,7 @@ static int score_batch_packed_ctx(swb200_ctx* c, const unsigned long long* q_wor
   if (banded && forced <= 0) {
     // a banded kernel runs as long as its pairs are long however few they are: chunks are whole waves of resident CTAs
     // (10 kb reads: 14 208 pairs = 72 MB; 48 MB chunks left a third of every launch idle: 42.5 -> 30 ms for 250 000 pairs)
-    const long long wave = banded_wave_pairs(c, pv, ov);
+    const long long wave = banded_wave_pairs(c, pv, ov, band_w);
     chunk_pairs = wave * std::max<long long>(1, (target + wave * per_pair / 2) / (wave * per_pair));
   }
   const size_t nchunks = (size_t)((npairs + chunk_pairs - 1) / chunk_pairs);
@@ -2288,7 +2302,7 @@ static int score_batch_packed_ctx(swb200_ctx* c, const unsigned long long* q_wor
     SWB_CUDA(cudaStreamWaitEvent(sk, c->chunk_events[ci], 0));
     if (first) { SWB_CUDA(cudaEventRecord(c->ev0, sk)); first = false; }
     const BatchView v{c->hb_qw + k0 * q_stride, c->hb_tw + k0 * t_stride, c->hb_ql + k0, c->hb_tl + k0, q_stride, t_stride, nk, max_short, max_long};
-    rc = banded ? launch_banded_score(c, v, band_lo, pv, ov, sk, c->hb_scores + k0, &c->info)
+    rc = banded ? launch_banded_score(c, v, band_lo, band_w, pv, ov, sk, c->hb_scores + k0, &c->info)
                 : launch_batch_score(c, v, pv, ov, sk, c->hb_scores + k0, &c->info);
     if (rc) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sk); return rc; }
   }
@@ -2326,7 +2340,7 @@ static int score_packed_host(const unsigned long long* q_words, long long q_stri
       [&](swb200_ctx* c, long long k0, long long k1, const LenScan& part, const LenScan& whole) {
         return score_batch_packed_ctx(c, q_words + k0 * q_stride, q_stride, t_words + k0 * t_stride, t_stride, q_len + k0,
                                       t_len + k0, k1 - k0, whole.max_q, whole.max_t, part.cells, p, o, banded, band_lo,
-                                      scores_out + k0);
+                                      band_hi - band_lo + 1, scores_out + k0);
       });
 }
 
@@ -2350,7 +2364,7 @@ int swb200_score_banded_batch(const unsigned char* seq1_all, const long long* of
                               const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
                               int band_lo, int band_hi, const swb200_params* p, const swb200_options* opt,
                               int* scores_out) {
-  if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
+  if (int rc = check_band_width(band_lo, band_hi)) return rc;
   return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, ScoreKind::banded, band_lo,
                           band_hi, scores_out);
 }
@@ -2596,23 +2610,37 @@ int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, co
   return SWB200_OK;
 }
 
-constexpr long long kBandSlotWords = 32LL * 3072;  // direction slot per warp: 384 KB, spans with len1 + len2 < 24 568 (cfg5: ~20 000)
+constexpr long long kBandSlotWords = 32LL * 3072;  // direction slot per warp and K: 384 KB, spans with len1 + len2 < 24 568 (cfg5: ~20 000)
 constexpr int kBandCtasPerSm = 8;                  // 32 resident warps per SM: enough to hide the shuffle chain of a step
 
 // Passes 1-3 and the walk over a packed range in caller order (q = seq1, t = seq2), everything on stream s of c's device:
-// one warp per pair, the trace rounds of align_rounds_locked.  Direction slots: kBandSlotWords per launched warp.
-int align_banded_packed_locked(swb200_ctx* c, const BatchView& v, int band_lo, const swb200_params& p, cudaStream_t s,
+// one warp per pair, the trace rounds of align_rounds_locked.  A band of band_w = 64 K diagonals stores K nibbles per
+// lane and anti-diagonal, so the direction slot of a launched warp is K x kBandSlotWords: the same spans fit one slot at
+// every width.  The slots of all warps take at most a fifth of the device memory free to this context (free memory plus
+// the slots it already holds): if K x kBandSlotWords per warp would take more, fewer warps are launched (at least one
+// CTA per SM).  On a 180 GB B200 occupancy allows 8 / 5 / 4 / 3 CTAs per SM at K = 1 / 2 / 4 / 8: 1.8 / 2.3 / 3.7 / 5.6 GB
+// of slots, well inside the share.
+int align_banded_packed_locked(swb200_ctx* c, const BatchView& v, int band_lo, int band_w, const swb200_params& p, cudaStream_t s,
                                int* d_scores, int* d_spans, uint32_t* d_ops, int ops_stride, int* d_ops_count,
                                swb200_run_info* info) {
   if (v.npairs == 0) return SWB200_OK;
   constexpr int W = swb::kBandAlignWarps;
+  const int K = band_w / 64;
+  const long long slot_words = kBandSlotWords * K;
   int per_sm = 0;
-  SWB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, swb::align_banded_trace_kernel_ptr(), 32 * W, 0));
+  SWB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, swb::align_banded_trace_kernel_ptr(K), 32 * W, 0));
   per_sm = std::max(1, std::min(per_sm, kBandCtasPerSm));
+  if (K > 1) {
+    size_t fr = 0, tot = 0;
+    SWB_CUDA(cudaMemGetInfo(&fr, &tot));
+    const double share = (double)(fr + c->ab_slot_cap * sizeof(uint64_t)) / 5;
+    const long long fit = (long long)(share / ((double)slot_words * sizeof(uint32_t) * W * c->sms));   // CTAs per SM
+    per_sm = std::max(1, std::min<int>(per_sm, (int)std::min<long long>(fit, kBandCtasPerSm)));
+  }
   const long long blocks = std::max(1LL, std::min<long long>((v.npairs + W - 1) / W, (long long)c->sms * per_sm));
   const long long nw = blocks * W;
   int rc;
-  if ((rc = grow(c->ab_slot, c->ab_slot_cap, (size_t)(kBandSlotWords * nw + 1) / 2, false, s)) ||
+  if ((rc = grow(c->ab_slot, c->ab_slot_cap, (size_t)(slot_words * nw + 1) / 2, false, s)) ||
       (rc = grow(c->ab_list, c->ab_list_cap, 2 * (size_t)v.npairs, false, s)) ||
       (rc = grow(c->ab_misc, c->ab_misc_cap, 4, false, s))) return rc;
   SWB_CUDA(cudaMemsetAsync(c->ab_misc, 0, 3 * sizeof(unsigned long long), s));
@@ -2621,25 +2649,25 @@ int align_banded_packed_locked(swb200_ctx* c, const BatchView& v, int band_lo, c
   P.a_stride = v.q_stride; P.b_stride = v.t_stride; P.npairs = v.npairs; P.band_lo = band_lo;
   P.match = p.match; P.mismatch = p.mismatch; P.gap_init = p.gap_init; P.gap_ext = p.gap_ext;
   P.scores = d_scores; P.spans = d_spans; P.nwarps = nw;
-  P.slot = reinterpret_cast<uint32_t*>(c->ab_slot); P.slot_words = kBandSlotWords;
+  P.slot = reinterpret_cast<uint32_t*>(c->ab_slot); P.slot_words = slot_words;
   P.pool = reinterpret_cast<uint32_t*>(c->ab_pool); P.pool_words = 2 * (long long)c->ab_pool_cap;
   P.pool_used = c->ab_misc + 1;
   P.todo = nullptr; P.ntodo = v.npairs;
   P.pending = c->ab_list; P.npending = reinterpret_cast<int*>(c->ab_misc) + 1;
   P.ops = d_ops; P.ops_stride = ops_stride; P.ops_count = d_ops_count;
   P.err = reinterpret_cast<int*>(c->ab_misc); P.cells = c->ab_misc + 2;
-  swb::launch_align_banded_span(P, (int)blocks, s);
-  swb::launch_align_banded_trace(P, (int)blocks, s);
+  swb::launch_align_banded_span(P, K, (int)blocks, s);
+  swb::launch_align_banded_trace(P, K, (int)blocks, s);
   SWB_CUDA(cudaGetLastError());
   info->engine_launches += 2;
   // spans larger than a slot: the pool (64-bit words here), sized for the largest span the batch can have
-  const size_t need = (size_t)std::max(kAlignPoolWords, (swb::band_dir_words(v.max_short, v.max_long) + 1) / 2);
+  const size_t need = (size_t)std::max(kAlignPoolWords, (K * swb::band_dir_words(v.max_short, v.max_long) + 1) / 2);
   if ((rc = align_rounds_locked(c, s, v.npairs, need, info, [&](const int* todo, int ntodo, int* pending) {
          P.pool = reinterpret_cast<uint32_t*>(c->ab_pool); P.pool_words = 2 * (long long)c->ab_pool_cap;
          P.todo = todo; P.ntodo = ntodo; P.pending = pending;
-         swb::launch_align_banded_trace(P, (int)std::max(1LL, std::min<long long>(blocks, (ntodo + W - 1) / W)), s);
+         swb::launch_align_banded_trace(P, K, (int)std::max(1LL, std::min<long long>(blocks, (ntodo + W - 1) / W)), s);
        }))) return rc;
-  info->lanes = 32; info->config = 310; info->rows = 0; info->bands = swb::kBandWidth;
+  info->lanes = 32; info->config = K == 1 ? 310 : (K == 2 ? 311 : (K == 4 ? 312 : 313)); info->rows = 0; info->bands = band_w;
   info->ctas = (int)blocks; info->warps = (int)nw;
   return SWB200_OK;
 }
@@ -2728,9 +2756,9 @@ enum class AlignKind { batch, banded, long_pairs };
 
 // One context's share of a host batch alignment (arguments checked by the caller): the copy/pack pipeline of the score
 // calls, then the passes over the whole range, then the outputs back.  banded: the pairs stay in caller order and the
-// banded passes run with band band_lo .. band_lo + 63.
+// banded passes run with band band_lo .. band_lo + band_w - 1.
 static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part, const PairScan& whole,
-                                const swb200_params& p, AlignKind kind, int band_lo, int* scores_out, int* spans_out,
+                                const swb200_params& p, AlignKind kind, int band_lo, int band_w, int* scores_out, int* spans_out,
                                 unsigned int* ops_out, int ops_stride, int* ops_count) {
   std::lock_guard<std::mutex> lk(c->mu);
   DeviceGuard guard;
@@ -2750,7 +2778,8 @@ static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npa
   SWB_CUDA(cudaMemsetAsync(c->hb_ops, 0, np * (size_t)ops_stride * sizeof(uint32_t), sk));   // overflowed pairs come back as zeros
   switch (kind) {
     case AlignKind::banded:
-      rc = align_banded_packed_locked(c, v, band_lo, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info);
+      rc = align_banded_packed_locked(c, v, band_lo, band_w, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn,
+                                      &c->info);
       break;
     case AlignKind::long_pairs:
       rc = align_long_packed_locked(c, v, c->hb_len1, p, sk, c->hb_scores, c->hb_spans, c->hb_ops, ops_stride, c->hb_opsn, &c->info);
@@ -2792,7 +2821,7 @@ int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, con
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::batch, 0, scores_out + k0, spans_out + 4 * k0,
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::batch, 0, 0, scores_out + k0, spans_out + 4 * k0,
                                     ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
       });
 }
@@ -2816,7 +2845,7 @@ int swb200_align_banded_batch(const unsigned char* seq1_all, const long long* of
                               int band_lo, int band_hi, const swb200_params* pp, const swb200_options* opt, int* scores_out,
                               int* spans_out, unsigned int* ops_out, int ops_stride, int* ops_count) {
   (void)opt;
-  if (band_hi - band_lo != swb::kBandWidth - 1) return fail(SWB200_ERR_ARG, "the banded kernel handles exactly 64 diagonals");
+  if (int rc = check_band_width(band_lo, band_hi)) return rc;
   if (npairs < 0 || ops_stride < 1 ||
       (npairs > 0 && (!seq1_all || !seq2_all || !off1 || !off2 || !len1 || !len2 || !scores_out || !spans_out || !ops_out || !ops_count)))
     return fail(SWB200_ERR_ARG, "bad batch arguments");
@@ -2827,7 +2856,8 @@ int swb200_align_banded_batch(const unsigned char* seq1_all, const long long* of
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::banded, band_lo, scores_out + k0, spans_out + 4 * k0,
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::banded, band_lo, band_hi - band_lo + 1,
+                                    scores_out + k0, spans_out + 4 * k0,
                                     ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
       });
 }
@@ -2841,7 +2871,8 @@ int swb200_batch_align_banded(swb200_batch* b, int band_lo, int band_hi, const s
   int rc;
   if ((rc = check_params(p)) || (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
   return run_device_batch(b, 0, stream, [&](swb200_ctx* c, cudaStream_t s) {
-    return align_banded_packed_locked(c, whole_batch(b), band_lo, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info);
+    return align_banded_packed_locked(c, whole_batch(b), band_lo, band_hi - band_lo + 1, p, s, d_scores, d_spans, d_ops, ops_stride,
+                                      d_ops_count, &c->info);
   });
 }
 
@@ -2860,7 +2891,7 @@ int swb200_align_long_batch(const unsigned char* seq1_all, const long long* off1
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::long_pairs, 0, scores_out + k0,
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::long_pairs, 0, 0, scores_out + k0,
                                     spans_out + 4 * k0, ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
       });
 }

@@ -1,6 +1,6 @@
 // swb_align_banded.cuh -- score, span and CIGAR for every pair of a banded batch (swb200_align_banded_batch,
 // swb200_batch_align_banded): the best local alignment all of whose cells lie in the band B, band_lo <= j - i <= band_hi
-// (64 diagonals; i is the row in seq2, j the column in seq1).
+// (W = 64 K diagonals, K = 1, 2, 4 or 8; i is the row in seq2, j the column in seq1).
 //
 // One warp per pair.  A 10 kb pair's direction nibbles take ~16 B x (len1 + len2) = 320 KB, so a thread per pair (as in
 // swb_align_batch.cuh) would need gigabytes in flight; a warp needs 32x less, and its storage grows with the resident
@@ -11,6 +11,10 @@
 // register and the left one lane l-1's second register (one shfl for H, one for E); on an odd step the left one is the
 // lane's own first register and the upper one lane l+1's first register (H and F).  The diagonal neighbour is the
 // cell's own register of two steps ago.  This is the geometry of swb_banded.cuh, in 32-bit lanes.
+//
+// Wider bands (K > 1, DESIGN.md 4f): lane l owns the 2K consecutive diagonals lo + 2Kl .. lo + 2Kl + 2K - 1, of which K
+// have a cell on each anti-diagonal.  Neighbours inside the lane stay in registers; only the lane's outer diagonals use
+// the two shfls above.  A lane writes K nibbles per anti-diagonal, so one direction word holds 8 / K anti-diagonals.
 //
 //   pass 1  local recurrence over the pair, band lo = band_lo: the end cell (max H, then the smallest j, then the
 //           smallest i; out-of-band cells are H = E = F = 0, as in oracle_gotoh_banded);
@@ -44,7 +48,7 @@ struct AlignBandedParams {
   const int* b_len;
   long long a_stride, b_stride;
   long long npairs;
-  int band_lo;               // the band is band_lo <= j - i <= band_lo + 63
+  int band_lo;               // the band is band_lo <= j - i <= band_lo + 64 K - 1 (K: the kernels' template argument)
   int match, mismatch, gap_init, gap_ext;
   int* scores;               // per pair
   int* spans;                // per pair {i_start, j_start, i_end, j_end}, 1-based
@@ -66,78 +70,103 @@ struct AlignBandedParams {
   unsigned long long* cells; // in-band cells the passes computed (one atomic add per lane and launch)
 };
 
-// 32-bit direction words a lx x ly span takes: one line of 32 words per 8 anti-diagonals t = 0 .. lx + ly
-SWB_HD long long band_dir_words(int lx, int ly) { return 32LL * (((long long)lx + ly) / 8 + 1); }
+// 32-bit direction words a lx x ly span takes: one line of 32 words per 8 / K anti-diagonals t = 0 .. lx + ly
+template <int K = 1>
+SWB_HD long long band_dir_words(int lx, int ly) { return 32LL * (((long long)lx + ly) / (8 / K) + 1); }
 
 // the end / start cell's tie rule: the larger H; among equal H > 0 the smaller x (j), then the smaller y (i)
 SWB_HD bool band_better(int h, int x, int y, int bh, int bx, int by) {
   return h > bh || (h == bh && h > 0 && (x < bx || (x == bx && y < by)));
 }
 
-// One recurrence over X (columns x = 1..X.len) x Y (rows y = 1..Y.len), restricted to the 64 diagonals
-// lo <= x - y <= lo + 63; the same result in every lane.
+// One recurrence over X (columns x = 1..X.len) x Y (rows y = 1..Y.len), restricted to the 64 K diagonals
+// lo <= x - y <= lo + 64 K - 1; the same result in every lane.
 //   MODE 0: local, returns the maximum and its cell;  MODE 1: anchored from (0, 0) (which must lie in the band), the same;
-//   MODE 2: anchored with direction nibbles into dirs (band_dir_words(X.len, Y.len) words), returns H at (X.len, Y.len).
+//   MODE 2: anchored with direction nibbles into dirs (band_dir_words<K>(X.len, Y.len) words), returns H at (X.len, Y.len).
 // *cells += the in-band cells of the rectangle this lane computed.
-template <int MODE>
+template <int MODE, int K = 1>
 SWB_HD int band_dp(const AlignBandedParams& P, const WarpCtx& w, const AlignSeq& X, const AlignSeq& Y, int lo, uint32_t* dirs,
                    int* bx, int* by, long long* cells) {
   constexpr bool ANCH = MODE >= 1, DIRS = MODE == 2;
   const int nx = X.len, ny = Y.len, lane = w.lane;
   const int gi = P.gap_init, ge = P.gap_ext, gmin = gi < ge ? gi : ge;
   const int ma = P.match, mi = P.mismatch;
+  constexpr int W = 64 * K, TW = 8 / K, TWS = K == 1 ? 3 : (K == 2 ? 2 : (K == 4 ? 1 : 0));   // TW = 2^TWS anti-diagonals a word, 2K = 2^(4-TWS)
   const int OUT = ANCH ? kAlignNeg : 0;          // H, E, F outside the band or the rectangle (anchored: borders aside)
   *bx = 0; *by = 0;
   // the diagonals that have cells, and the anti-diagonals t0 .. t1 they span
-  const int klo = lo > 1 - ny ? lo : 1 - ny, khi = lo + 63 < nx - 1 ? lo + 63 : nx - 1;
+  const int klo = lo > 1 - ny ? lo : 1 - ny, khi = lo + (W - 1) < nx - 1 ? lo + (W - 1) : nx - 1;
   if (nx <= 0 || ny <= 0 || klo > khi) return 0;
   const int t0 = 2 + (klo > 0 ? klo : (khi < 0 ? -khi : 0));
   const int kc = nx - ny < klo ? klo : (nx - ny > khi ? khi : nx - ny);
   const int t1 = nx + ny - (nx - ny - kc > 0 ? nx - ny - kc : kc - (nx - ny));
-  const int kA = lo + 2 * lane;                  // this lane's first diagonal; kA + 1 its second
+  const int kA = lo + 2 * K * lane;              // this lane's first diagonal; kA + 2K - 1 its last
   const int up_src = (lane + 1) & 31, left_src = (lane + 31) & 31;
-  int hA = OUT, eA = OUT, fA = OUT, hB = OUT, eB = OUT, fB = OUT;
+  // diagonal kA + q in hv[q], ev[q], fv[q]
+  int hv[2 * K], ev[2 * K], fv[2 * K];
+#pragma unroll
+  for (int q = 0; q < 2 * K; ++q) { hv[q] = OUT; ev[q] = OUT; fv[q] = OUT; }
   int best = 0, bxx = 0, byy = 0;
   long long nc = 0;
   uint32_t dword = 0;
   // two steps before t0 every cell is a border cell or outside: the registers hold correct neighbours from then on
   for (int t = t0 - 2; t <= t1; ++t) {
     const bool odd = ((t - lo) & 1) != 0;
-    const int nh = (int)w.shfl((uint32_t)(odd ? hA : hB), odd ? up_src : left_src);
-    const int ng = (int)w.shfl((uint32_t)(odd ? fA : eB), odd ? up_src : left_src);
-    const bool edge = odd ? lane == 31 : lane == 0;          // diagonal lo + 64 / lo - 1: outside the band
+    const int nh = (int)w.shfl((uint32_t)(odd ? hv[0] : hv[2 * K - 1]), odd ? up_src : left_src);
+    const int ng = (int)w.shfl((uint32_t)(odd ? fv[0] : ev[2 * K - 1]), odd ? up_src : left_src);
+    const bool edge = odd ? lane == 31 : lane == 0;          // diagonal lo + W / lo - 1: outside the band
     const int xh = edge ? OUT : nh, xg = edge ? OUT : ng;
-    const int lh = odd ? hA : xh, lg = odd ? eA : xg;        // left (y, x-1)
-    const int uh = odd ? xh : hB, ug = odd ? xg : fB;        // up (y-1, x)
-    const int dh = odd ? hB : hA;                            // diagonal (y-1, x-1)
-    const int k = kA + (odd ? 1 : 0);
-    const int x = (t + k) >> 1, y = (t - k) >> 1;            // t + k is even
-    const bool in = x >= 1 && x <= nx && y >= 1 && y <= ny;
-    const int s = align_code(X, in ? x - 1 : 0) == align_code(Y, in ? y - 1 : 0) ? ma : mi;
-    const int e_ext = lg - ge, e_open = lh - gi, f_ext = ug - ge, f_open = uh - gi;
-    int e = imax2(e_ext, e_open), f = imax2(f_ext, f_open);
-    const int d = dh + s;
-    int h = imax2(d, imax2(e, f));
-    if (!ANCH) h = imax2(h, 0);
-    if (!in) {
-      e = OUT; f = OUT; h = OUT;
-      if (ANCH && x >= 0 && y >= 0 && (x == 0 || y == 0)) h = x + y == 0 ? 0 : -(gi + (x + y - 1) * gmin);
+    int hn[K], en[K], fn[K];
+    uint32_t nib = 0;
+#pragma unroll
+    for (int c = 0; c < K; ++c) {
+      // the cell on diagonal kA + q, q = 2c + odd: left = q - 1, up = q + 1 (both of the previous step), diagonal = q itself
+      const int qa = 2 * c, qb = 2 * c + 1;
+      const int lh = odd ? hv[qa] : (c == 0 ? xh : hv[c == 0 ? 0 : qa - 1]);          // left (y, x-1)
+      const int lg = odd ? ev[qa] : (c == 0 ? xg : ev[c == 0 ? 0 : qa - 1]);
+      const int uh = odd ? (c == K - 1 ? xh : hv[c == K - 1 ? 0 : qb + 1]) : hv[qb];  // up (y-1, x)
+      const int ug = odd ? (c == K - 1 ? xg : fv[c == K - 1 ? 0 : qb + 1]) : fv[qb];
+      const int dh = odd ? hv[qb] : hv[qa];                                           // diagonal (y-1, x-1)
+      const int k = kA + (odd ? qb : qa);
+      const int x = (t + k) >> 1, y = (t - k) >> 1;            // t + k is even
+      const bool in = x >= 1 && x <= nx && y >= 1 && y <= ny;
+      const int s = align_code(X, in ? x - 1 : 0) == align_code(Y, in ? y - 1 : 0) ? ma : mi;
+      const int e_ext = lg - ge, e_open = lh - gi, f_ext = ug - ge, f_open = uh - gi;
+      int e = imax2(e_ext, e_open), f = imax2(f_ext, f_open);
+      const int d = dh + s;
+      int h = imax2(d, imax2(e, f));
+      if (!ANCH) h = imax2(h, 0);
+      if (!in) {
+        e = OUT; f = OUT; h = OUT;
+        if (ANCH && x >= 0 && y >= 0 && (x == 0 || y == 0)) h = x + y == 0 ? 0 : -(gi + (x + y - 1) * gmin);
+      }
+      nc += in ? 1 : 0;
+      if (DIRS) {
+        const uint32_t src = h == d ? 0u : (h == e ? 1u : 2u);
+        nib |= (src | (e_ext > e_open ? 4u : 0u) | (f_ext > f_open ? 8u : 0u)) << (4 * c);
+      } else if (in && band_better(h, x, y, best, bxx, byy)) {
+        best = h; bxx = x; byy = y;
+      }
+      hn[c] = h; en[c] = e; fn[c] = f;
     }
-    nc += in ? 1 : 0;
     if (DIRS) {
-      const uint32_t src = h == d ? 0u : (h == e ? 1u : 2u);
-      dword |= (src | (e_ext > e_open ? 4u : 0u) | (f_ext > f_open ? 8u : 0u)) << (4 * (t & 7));
-      if ((t & 7) == 7 || t == t1) { dirs[(long long)(t >> 3) * 32 + lane] = dword; dword = 0; }
-    } else if (in && band_better(h, x, y, best, bxx, byy)) {
-      best = h; bxx = x; byy = y;
+      dword |= nib << (4 * K * (t & (TW - 1)));
+      if ((t & (TW - 1)) == TW - 1 || t == t1) { dirs[(long long)(t >> TWS) * 32 + lane] = dword; dword = 0; }
     }
-    if (odd) { hB = h; eB = e; fB = f; } else { hA = h; eA = e; fA = f; }
+#pragma unroll
+    for (int c = 0; c < K; ++c) {
+      if (odd) { hv[2 * c + 1] = hn[c]; ev[2 * c + 1] = en[c]; fv[2 * c + 1] = fn[c]; }
+      else { hv[2 * c] = hn[c]; ev[2 * c] = en[c]; fv[2 * c] = fn[c]; }
+    }
   }
   *cells += nc;
   if constexpr (DIRS) {
     // H(nx, ny) is the last cell of diagonal nx - ny, computed at t1 = nx + ny
-    const int kl = nx - ny - lo;
-    return (int)w.shfl((uint32_t)((kl & 1) ? hB : hA), kl >> 1);
+    const int kl = nx - ny - lo, q = kl & (2 * K - 1);
+    int hq = hv[0];
+#pragma unroll
+    for (int r = 1; r < 2 * K; ++r) hq = q == r ? hv[r] : hq;
+    return (int)w.shfl((uint32_t)hq, kl >> (4 - TWS));
   } else {
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -151,16 +180,18 @@ SWB_HD int band_dp(const AlignBandedParams& P, const WarpCtx& w, const AlignSeq&
 }
 
 // Passes 1 and 2 for pair k: score and span.  Returns this lane's in-band cells.
+template <int K = 1>
 SWB_HD long long band_span_pair(const AlignBandedParams& P, const WarpCtx& w, long long k) {
   const int n = P.a_len[k], m = P.b_len[k];
   const uint64_t* aw = P.a_words + k * P.a_stride;
   const uint64_t* bw = P.b_words + k * P.b_stride;
   long long nc = 0;
   int je = 0, ie = 0, rj = 0, ri = 0;
-  const int s = band_dp<0>(P, w, AlignSeq{aw, 0, n, false}, AlignSeq{bw, 0, m, false}, P.band_lo, nullptr, &je, &ie, &nc);
+  const int s = band_dp<0, K>(P, w, AlignSeq{aw, 0, n, false}, AlignSeq{bw, 0, m, false}, P.band_lo, nullptr, &je, &ie, &nc);
   int s2 = s;
   if (s > 0)
-    s2 = band_dp<1>(P, w, AlignSeq{aw, 0, je, true}, AlignSeq{bw, 0, ie, true}, (je - ie) - (P.band_lo + 63), nullptr, &rj, &ri, &nc);
+    s2 = band_dp<1, K>(P, w, AlignSeq{aw, 0, je, true}, AlignSeq{bw, 0, ie, true}, (je - ie) - (P.band_lo + (64 * K - 1)), nullptr,
+                       &rj, &ri, &nc);
   if (w.lane == 0) {
     int* span = P.spans + 4 * k;
     P.scores[k] = s;
@@ -202,15 +233,16 @@ struct OpEncoder {
 // Lane 0 walks; before it runs out of staged lines the warp copies the next kBandStageLines lines below into stage.
 // Operations come out last-first (OpEncoder).  Returns the count and *total in every lane; a step out of the band
 // poisons *total.
-template <bool WRITE>
+template <bool WRITE, int K = 1>
 SWB_HD int band_walk(const AlignBandedParams& P, const WarpCtx& w, const uint32_t* dirs, const AlignSeq& X, const AlignSeq& Y,
                      int lo, uint32_t* stage, int n, uint32_t* ops, int* total) {
+  constexpr int TWS = K == 1 ? 3 : (K == 2 ? 2 : (K == 4 ? 1 : 0));   // a direction line holds 2^TWS = 8 / K anti-diagonals
   const int lane = w.lane;
   int x = X.len, y = Y.len, state = 0;
   bool outside = false;
   OpEncoder<WRITE> enc{P.match, P.mismatch, P.gap_init, P.gap_ext, ops, n};
   for (;;) {
-    const int top = (int)w.shfl((uint32_t)((x + y) >> 3), 0);
+    const int top = (int)w.shfl((uint32_t)((x + y) >> TWS), 0);
     const int base = top - kBandStageLines + 1 > 0 ? top - kBandStageLines + 1 : 0;
     w.sync();
     for (int q = 0; q < kBandStageLines && base + q <= top; ++q) stage[q * 32 + lane] = dirs[(long long)(base + q) * 32 + lane];
@@ -219,10 +251,12 @@ SWB_HD int band_walk(const AlignBandedParams& P, const WarpCtx& w, const uint32_
     if (lane == 0) {
       while (x > 0 && y > 0) {
         const int t = x + y;
-        if ((t >> 3) < base) break;
+        if ((t >> TWS) < base) break;
         const unsigned kl = (unsigned)(x - y - lo);
-        if (kl > 63u) { outside = true; break; }
-        const uint32_t d = (stage[((t >> 3) - base) * 32 + (int)(kl >> 1)] >> (4 * (t & 7))) & 0xFu;
+        if (kl > 64u * K - 1) { outside = true; break; }
+        // lane kl / 2K, nibble K (t mod 8/K) + (kl mod 2K) / 2
+        const uint32_t nib = K * (t & ((1 << TWS) - 1)) + ((kl & (2 * K - 1)) >> 1);
+        const uint32_t d = (stage[((t >> TWS) - base) * 32 + (int)(kl >> (4 - TWS))] >> (4 * nib)) & 0xFu;
         if (state == 0) {
           const uint32_t src = d & 3u;
           if (src == 0) { enc.emit(align_code(X, x - 1) == align_code(Y, y - 1) ? kOpEq : kOpX, 1); --x; --y; }
@@ -257,13 +291,14 @@ SWB_HD int band_walk(const AlignBandedParams& P, const WarpCtx& w, const uint32_
 
 // Pass 3 and the walk for pair k (score and span from band_span_pair).  Returns this lane's in-band cells, or -1 if the
 // pair must wait for the next round (pool exhausted).
+template <int K = 1>
 SWB_HD long long band_trace_pair(const AlignBandedParams& P, const WarpCtx& w, long long k, long long warp, uint32_t* stage) {
   const int s = P.scores[k];
   if (s <= 0) { if (w.lane == 0) P.ops_count[k] = 0; return 0; }
   const int* span = P.spans + 4 * k;
   const int is = span[0], js = span[1], ie = span[2], je = span[3];
   const int lx = je - js + 1, ly = ie - is + 1, lo = P.band_lo - (js - is);
-  const long long words = band_dir_words(lx, ly);
+  const long long words = band_dir_words<K>(lx, ly);
   uint32_t* dirs;
   if (words <= P.slot_words) {
     dirs = P.slot + warp * P.slot_words;
@@ -280,47 +315,50 @@ SWB_HD long long band_trace_pair(const AlignBandedParams& P, const WarpCtx& w, l
   const AlignSeq X{P.a_words + k * P.a_stride, js - 1, lx, false}, Y{P.b_words + k * P.b_stride, is - 1, ly, false};
   long long nc = 0;
   int unused0 = 0, unused1 = 0;
-  const int h = band_dp<2>(P, w, X, Y, lo, dirs, &unused0, &unused1, &nc);
+  const int h = band_dp<2, K>(P, w, X, Y, lo, dirs, &unused0, &unused1, &nc);
   if (h != s) {
     if (w.lane == 0) { atomic_or_i32(P.err, kAlignErrTrace); P.ops_count[k] = 0; }
     return nc;
   }
   int total = 0;
-  const int n = band_walk<false>(P, w, dirs, X, Y, lo, stage, 0, nullptr, &total);
+  const int n = band_walk<false, K>(P, w, dirs, X, Y, lo, stage, 0, nullptr, &total);
   if (total != s) {
     if (w.lane == 0) { atomic_or_i32(P.err, kAlignErrRescore); P.ops_count[k] = 0; }
     return nc;
   }
   if (n > P.ops_stride) { if (w.lane == 0) P.ops_count[k] = -n; return nc; }
-  band_walk<true>(P, w, dirs, X, Y, lo, stage, n, P.ops + k * (long long)P.ops_stride, &total);
+  band_walk<true, K>(P, w, dirs, X, Y, lo, stage, n, P.ops + k * (long long)P.ops_stride, &total);
   if (w.lane == 0) P.ops_count[k] = n;
   return nc;
 }
 
 #if defined(__CUDACC__) && defined(SWB_ALIGN_BANDED_KERNELS)   // defined in swb_align_banded.cu only: one definition
+template <int K>
 __global__ void __launch_bounds__(32 * kBandAlignWarps) align_banded_span_kernel(const __grid_constant__ AlignBandedParams P) {
   const WarpCtx w{(int)(threadIdx.x & 31)};
   const long long warp = (long long)blockIdx.x * kBandAlignWarps + threadIdx.x / 32;
   long long cells = 0;
-  for (long long k = warp; k < P.npairs; k += P.nwarps) cells += band_span_pair(P, w, k);
+  for (long long k = warp; k < P.npairs; k += P.nwarps) cells += band_span_pair<K>(P, w, k);
   if (cells) atomicAdd(P.cells, (unsigned long long)cells);
 }
-__global__ void __launch_bounds__(32 * kBandAlignWarps) align_banded_trace_kernel(const __grid_constant__ AlignBandedParams P) {
+// __maxnreg__: without a register limit ptxas gives K = 2 64 registers and 20 bytes of spills
+template <int K>
+__global__ void __launch_bounds__(32 * kBandAlignWarps) __maxnreg__(K == 2 ? 128 : 255) align_banded_trace_kernel(const __grid_constant__ AlignBandedParams P) {
   __shared__ uint32_t stage[kBandAlignWarps][kBandStageLines * 32];
   const WarpCtx w{(int)(threadIdx.x & 31)};
   const long long warp = (long long)blockIdx.x * kBandAlignWarps + threadIdx.x / 32;
   long long cells = 0;
   for (long long t = warp; t < P.ntodo; t += P.nwarps) {
-    const long long c = band_trace_pair(P, w, P.todo ? P.todo[t] : t, warp, stage[threadIdx.x / 32]);
+    const long long c = band_trace_pair<K>(P, w, P.todo ? P.todo[t] : t, warp, stage[threadIdx.x / 32]);
     cells += c > 0 ? c : 0;
   }
   if (cells) atomicAdd(P.cells, (unsigned long long)cells);
 }
 #endif
 
-// host launchers (swb_align_banded.cu); blocks x kBandAlignWarps warps must not exceed P.nwarps
-void launch_align_banded_span(const AlignBandedParams& P, int blocks, cudaStream_t s);
-void launch_align_banded_trace(const AlignBandedParams& P, int blocks, cudaStream_t s);
-const void* align_banded_trace_kernel_ptr();
+// host launchers (swb_align_banded.cu) for K = 1, 2, 4, 8; blocks x kBandAlignWarps warps must not exceed P.nwarps
+void launch_align_banded_span(const AlignBandedParams& P, int K, int blocks, cudaStream_t s);
+void launch_align_banded_trace(const AlignBandedParams& P, int K, int blocks, cudaStream_t s);
+const void* align_banded_trace_kernel_ptr(int K);
 
 }  // namespace swb

@@ -37,7 +37,7 @@ struct BandedParams {
   const int* b_len;
   long long a_stride, b_stride;
   long long npairs;
-  int band_lo;               // band is band_lo <= j-i <= band_lo+63
+  int band_lo;               // band is band_lo <= j-i <= band_lo+W-1 (W: the kernel's width)
   int* scores;
   int match, mismatch, gap_init, gap_ext;
 };
@@ -359,19 +359,38 @@ const void* banded8_kernel(int mode);
 //  per cell vector (linear), 9.4 instead of 10.75 (affine).
 //  Positions (0-based) at double step h, with y = I0 - (S/2) u - 1 + h and x = J0 + (S/2) u - 1 + h:
 //  set 2e: row y - e, column x + e; set 2e+1: row y - e, column x + e + 1; hi halves 16 rows up, 16 columns right.
+//
+//  Wider bands (W = 128, 256, 512 diagonals; DESIGN.md 4f) use the same layout with S = 8 and TP = W / 16 threads per
+//  pair (32 / TP pairs per warp): thread u holds diagonals S*u + s and S*u + s + W/2, so a register's hi half is W/4 rows
+//  up and W/4 columns right of its lo half and a selector pairs rows y and y - W/4.  The seam between diagonals W/2 - 1
+//  and W/2 rides on the rotation between the last thread and thread 0 with the same two selectors.  A chunk reads rows
+//  [Yc - W/4 + 1, Yc + 32) and columns [Xc, Xc + W/2 + 32) while the previous chunk's reads may still be in flight, so
+//  the rings hold W/4 + 64 rows and W/2 + 64 columns (kBandRingFor).  The selectors of wide bands are refilled by the
+//  guarded per-symbol path; the column tables keep the rolling window.
 // =================================================================================================
-template <int S>
+// ring entries of a W-diagonal band: a power of two >= W/2 + 64 (128 for W = 64 and 128, 256 for 256, 512 for 512)
+template <int W>
+constexpr int kBandRingFor = W <= 128 ? kBandRing : (W <= 256 ? 256 : 512);
+
+template <int S, int W = kBandWidth>
 struct BandedWarpSmemS {
-  // S pairs per warp read the same ring offsets in the same instruction: pair g's rings start (g mod S/2) + 16 (g / (S/2))
-  // words into their row, so that the 32 threads (offsets (S/2) u inside a pair) hit 32 different banks
-  uint32_t tab[S][2 * kBandRing + 32];
-  uint32_t sel[S][2 * kBandRing + 32];
+  // The pairs of a warp read the same ring offsets in the same instruction: pair g's rings start (g mod S/2) + 16 (g / (S/2))
+  // words into their row, so that the 32 threads (offsets (S/2) u inside a pair) hit 32 different banks.  (From W = 256 on,
+  // threads u and u + 8 of one pair read 32 words apart: 2-way, at W = 512 4-way conflicts that no offset removes.)
+  static constexpr int kPairs = 32 * 2 * S / W, kRing = kBandRingFor<W>;
+  uint32_t tab[kPairs][2 * kRing + 32];
+  uint32_t sel[kPairs][2 * kRing + 32];
 };
 
-template <int MODE, int S>
-SWB_HD void banded_warpS(const BandedParams& P, const WarpCtx& w, long long warp_id, long long num_warps, BandedWarpSmemS<S>* sm) {
+template <int MODE, int S, int W = kBandWidth>
+SWB_HD void banded_warpS(const BandedParams& P, const WarpCtx& w, long long warp_id, long long num_warps, BandedWarpSmemS<S, W>* sm) {
   static_assert(S >= 4 && S <= 16 && (S & (S - 1)) == 0, "register sets per thread: 4, 8 or 16");
-  constexpr int TP = 32 / S, H2 = S / 2;
+  static_assert(W == kBandWidth || (S == 8 && (W == 128 || W == 256 || W == 512)), "band width: 64, or 128 / 256 / 512 with S = 8");
+  constexpr int TP = W / (2 * S), H2 = S / 2, G = 32 / TP;      // threads per pair, pairs per warp
+  constexpr int Q = W / 4;                                      // rows up / columns right of a register's hi half
+  constexpr int RING = kBandRingFor<W>;
+  constexpr int PRE = Q > kChunk ? Q : kChunk;                  // rows below the first chunk the rings start with
+  constexpr bool ROW_WINDOW = Q == 16;                          // rows y and y - 16 come from one 64-bit funnel
   const int lane = w.lane;
   const int u = lane & (TP - 1), grp = lane / TP;
   const int src_prev = grp * TP + ((u + TP - 1) & (TP - 1));   // even step: set 0's left neighbours come from thread u-1 (rotating)
@@ -386,12 +405,12 @@ SWB_HD void banded_warpS(const BandedParams& P, const WarpCtx& w, long long warp
   const uint32_t sel_up = u == 0 ? 0x7632u : 0x3210u;          // thread 0 -> last thread: (its set 0 hi = diagonal 32, border)
   uint32_t* tab = sm->tab[grp] + (grp % H2) + 16 * (grp / H2);
   uint32_t* sel = sm->sel[grp] + (grp % H2) + 16 * (grp / H2);
-  const long long ngroups = (P.npairs + S - 1) / S;
+  const long long ngroups = (P.npairs + G - 1) / G;
   const int tA0 = 2 - ((2 - P.band_lo) & 1);                             // first even-set anti-diagonal (see banded_warp)
   const int I0 = (tA0 - P.band_lo) / 2, J0 = (tA0 + P.band_lo) / 2;
 
   for (long long pg = warp_id; pg < ngroups; pg += num_warps) {
-    const long long pair = pg * S + grp;
+    const long long pair = pg * G + grp;
     const bool valid = pair < P.npairs;
     const int n = valid ? P.a_len[pair] : 0, m = valid ? P.b_len[pair] : 0;
     const uint64_t* aw = P.a_words + (valid ? pair : 0) * P.a_stride;
@@ -405,28 +424,30 @@ SWB_HD void banded_warpS(const BandedParams& P, const WarpCtx& w, long long warp
     for (int k = 0; k < S; ++k) { Ho[k] = nopen; E[k] = nopen; F[k] = nopen; }
     uint32_t best = 0;
 
-    // ---- rings (slot of row y: (y - Yc0) & 127, of column x: (x - Xc0) & 127 -- a chunk's 32 new entries never wrap):
-    // everything pad, then selectors for rows [Yc0-32, Yc0) and tables for columns [Xc0, Xc0+32)
+    // ---- rings (slot of row y: (y - Yc0) & (RING-1), of column x: (x - Xc0) & (RING-1) -- a chunk's 32 new entries
+    // never wrap): everything pad, then selectors for rows [Yc0-PRE, Yc0) and tables for columns [Xc0, Xc0+W/2)
     const int Yc0 = I0 - 1, Xc0 = J0 - 1;                                  // thread 0's positions at h = 0
     w.sync();
-    for (int k = u; k < 2 * kBandRing; k += TP) { tab[k] = padw; sel[k] = padsel; }
+    for (int k = u; k < 2 * RING; k += TP) { tab[k] = padw; sel[k] = padsel; }
     w.sync();
-    for (int k = u; k < kChunk; k += TP) {
-      const int y = Yc0 - kChunk + k;
-      const uint32_t sv = mk_sel16(packed_code(bw, y, m), packed_code(bw, y - 16, m));
-      sel[(kBandRing - kChunk) + k] = sv; sel[(kBandRing - kChunk) + k + kBandRing] = sv;
+    for (int k = u; k < W / 2; k += TP) {
+      if (k < PRE) {
+        const int y = Yc0 - PRE + k;
+        const uint32_t sv = mk_sel16(packed_code(bw, y, m), packed_code(bw, y - Q, m));
+        sel[(RING - PRE) + k] = sv; sel[(RING - PRE) + k + RING] = sv;
+      }
       const int x = Xc0 + k;
       const uint32_t tv = table_word(packed_code(aw, x, n), padw, flip);
-      tab[k] = tv; tab[k + kBandRing] = tv;
+      tab[k] = tv; tab[k + RING] = tv;
     }
     // Rolling 32-symbol windows of the packed sequences (64 bits each), so that a chunk whose new rows and columns lie
     // inside the sequences costs ONE 64-bit load per sequence, issued a chunk ahead, instead of 24 guarded ones per thread
     // (the refill was 39 % of this kernel's stall samples, most of them waiting for those loads):
-    //   RA = rows [Yc-16, Yc+16) of the coming chunk, RN = the same for the chunk after it, TC = columns [Xc+32, Xc+64).
+    //   RA = rows [Yc-16, Yc+16) of the coming chunk, RN = the same for the chunk after it, TC = columns [Xc+W/2, Xc+W/2+32).
     // Word indices are clamped to the pair's words: a window that overlaps the outside holds garbage there and is not
     // used (such chunks take the guarded per-symbol path below).
     const int wr_i = (Yc0 - 16) >> 5, wr_sh = 2 * ((Yc0 - 16) & 31);
-    const int wc_i = (Xc0 + kChunk) >> 5, wc_sh = 2 * ((Xc0 + kChunk) & 31);
+    const int wc_i = (Xc0 + W / 2) >> 5, wc_sh = 2 * ((Xc0 + W / 2) & 31);
     uint64_t RA, RN, r_last, TC, c_last;
     {
       const uint64_t r0 = packed_word(bw, P.b_stride, wr_i), r1 = packed_word(bw, P.b_stride, wr_i + 1);
@@ -436,16 +457,16 @@ SWB_HD void banded_warpS(const BandedParams& P, const WarpCtx& w, long long warp
       c_last = packed_word(aw, P.a_stride, wc_i + 1);
       TC = funnel64(c0, c_last, wc_sh);
     }
-    const int su = 2 * H2 * u;                                             // this thread's entries: k = H2 u + j + 16 i (the offsets
-                                                                           // the step loop reads with: no bank conflicts)
+    const int su = 2 * H2 * u;                                             // W = 64: this thread's entries are k = H2 u + j + 16 i
+                                                                           // (the offsets the step loop reads with: no bank conflicts)
     for (int c = 0; c < nchunks; ++c) {
-      // ---- this chunk reads rows [Yc-16, Yc+32) and columns [Xc, Xc+64): add rows [Yc, Yc+32), columns [Xc+32, Xc+64)
+      // ---- this chunk reads rows [Yc-Q, Yc+32) and columns [Xc, Xc+W/2+32): add rows [Yc, Yc+32), columns [Xc+W/2, Xc+W/2+32)
       const int Yc = Yc0 + c * kChunk, Xc = Xc0 + c * kChunk;
       const uint64_t r_new = packed_word(bw, P.b_stride, wr_i + c + 3);    // consumed at the end of the chunk
       const uint64_t c_new = packed_word(aw, P.a_stride, wc_i + c + 2);
-      uint32_t* const selw = sel + ((c * kChunk) & (kBandRing - 1));
-      uint32_t* const tabw = tab + (((c + 1) * kChunk) & (kBandRing - 1));
-      if (Yc >= 16 && Yc + kChunk <= m) {
+      uint32_t* const selw = sel + ((c * kChunk) & (RING - 1));
+      uint32_t* const tabw = tab + ((c * kChunk + W / 2) & (RING - 1));
+      if (ROW_WINDOW && Yc >= 16 && Yc + kChunk <= m) {
         const uint32_t a_lo = (uint32_t)RA, b_lo = (uint32_t)(RA >> 32), b_hi = (uint32_t)RN;   // rows y - 16: RA; rows y: RA.hi, RN.lo
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
@@ -453,48 +474,57 @@ SWB_HD void banded_warpS(const BandedParams& P, const WarpCtx& w, long long warp
 #pragma unroll
           for (int j = 0; j < H2; ++j) {
             const uint32_t sv = 0xC480u + ((wb >> (2 * j)) & 3u) * 0x11u + ((wa >> (2 * j)) & 3u) * 0x1100u;   // = mk_sel16 of two real codes
-            selw[H2 * u + j + 16 * i] = sv; selw[H2 * u + j + 16 * i + kBandRing] = sv;
+            selw[H2 * u + j + 16 * i] = sv; selw[H2 * u + j + 16 * i + RING] = sv;
           }
         }
       } else {
         for (int k = u; k < kChunk; k += TP) {
           const int y = Yc + k;
-          const uint32_t sv = mk_sel16(packed_code(bw, y, m), packed_code(bw, y - 16, m));
-          selw[k] = sv; selw[k + kBandRing] = sv;
+          const uint32_t sv = mk_sel16(packed_code(bw, y, m), packed_code(bw, y - Q, m));
+          selw[k] = sv; selw[k + RING] = sv;
         }
       }
-      if (Xc + kChunk >= 0 && Xc + 2 * kChunk <= n) {
+      if (Xc + W / 2 >= 0 && Xc + W / 2 + kChunk <= n) {
+        if constexpr (ROW_WINDOW) {
 #pragma unroll
-        for (int i = 0; i < 2; ++i) {
-          const uint32_t wt = (i ? (uint32_t)(TC >> 32) : (uint32_t)TC) >> su;
+          for (int i = 0; i < 2; ++i) {
+            const uint32_t wt = (i ? (uint32_t)(TC >> 32) : (uint32_t)TC) >> su;
 #pragma unroll
-          for (int j = 0; j < H2; ++j) {
-            const uint32_t tv = padw ^ (flip << (8u * ((wt >> (2 * j)) & 3u)));
-            tabw[H2 * u + j + 16 * i] = tv; tabw[H2 * u + j + 16 * i + kBandRing] = tv;
+            for (int j = 0; j < H2; ++j) {
+              const uint32_t tv = padw ^ (flip << (8u * ((wt >> (2 * j)) & 3u)));
+              tabw[H2 * u + j + 16 * i] = tv; tabw[H2 * u + j + 16 * i + RING] = tv;
+            }
+          }
+        } else {                                                           // W > 64: 32 / TP consecutive entries a thread
+#pragma unroll
+          for (int j = 0; j < kChunk / TP; ++j) {
+            const int k = (kChunk / TP) * u + j;
+            const uint32_t tv = padw ^ (flip << (8u * ((uint32_t)(TC >> (2 * k)) & 3u)));
+            tabw[k] = tv; tabw[k + RING] = tv;
           }
         }
       } else {
         for (int k = u; k < kChunk; k += TP) {
-          const int x = Xc + kChunk + k;
+          const int x = Xc + W / 2 + k;
           const uint32_t tv = table_word(packed_code(aw, x, n), padw, flip);
-          tabw[k] = tv; tabw[k + kBandRing] = tv;
+          tabw[k] = tv; tabw[k + RING] = tv;
         }
       }
       RA = RN; RN = funnel64(r_last, r_new, wr_sh); r_last = r_new;
       TC = funnel64(c_last, c_new, wc_sh); c_last = c_new;
       w.sync();
       // ring windows of this thread: selp[h] = selector of row y (read back to -(S/2 - 1)); tabp[h] = table of column x
-      const uint32_t* selp = sel + ((c * kChunk - H2 * u - (H2 - 1)) & (kBandRing - 1)) + (H2 - 1);
-      const uint32_t* tabp = tab + ((c * kChunk + H2 * u) & (kBandRing - 1));
-      uint32_t a[H2 + 1], b[H2 + 1], sv[H2];        // columns x .. x + S/2 (and 16 further right), rows y .. y - S/2 + 1
+      const uint32_t* selp = sel + ((c * kChunk - H2 * u - (H2 - 1)) & (RING - 1)) + (H2 - 1);
+      const uint32_t* tabp = tab + ((c * kChunk + H2 * u) & (RING - 1));
+      uint32_t a[H2 + 1], b[H2 + 1], sv[H2];        // columns x .. x + S/2 (and Q further right), rows y .. y - S/2 + 1
 #pragma unroll
-      for (int e = 0; e < H2; ++e) { a[e] = tabp[e]; b[e] = tabp[e + 16]; }
+      for (int e = 0; e < H2; ++e) { a[e] = tabp[e]; b[e] = tabp[e + Q]; }
 #pragma unroll
       for (int e = 1; e < H2; ++e) sv[e] = selp[-e];
 #pragma unroll (2)
       for (int h = 0; h < kChunk; ++h) {
         sv[0] = selp[h];
-        a[H2] = tabp[h + H2]; b[H2] = tabp[h + H2 + 16];
+        a[H2] = tabp[h + H2]; b[H2] = tabp[h + H2 + Q];
         uint32_t sub[S];
 #pragma unroll
         for (int e = 0; e < H2; ++e) {
@@ -590,5 +620,18 @@ __global__ void __launch_bounds__(32, 6) sw_banded2_kernel(const __grid_constant
 #endif
 
 const void* banded2_kernel(int mode);
+
+#ifdef __CUDACC__
+// Bands of W = 128, 256 or 512 diagonals: W / 16 threads per pair with eight register sets each, 1024 / W pairs per CTA.
+template <int MODE, int W>
+__global__ void __launch_bounds__(64, 6) sw_banded_wide_kernel(const __grid_constant__ BandedParams P) {
+  __shared__ BandedWarpSmemS<8, W> sm[2];
+  WarpCtx w{(int)(threadIdx.x & 31)};
+  const int wi = (int)(threadIdx.x >> 5);
+  banded_warpS<MODE, 8, W>(P, w, (long long)blockIdx.x * 2 + wi, (long long)gridDim.x * 2, &sm[wi]);
+}
+#endif
+
+const void* banded_wide_kernel(int mode, int width);   // null for a width without a kernel
 
 }  // namespace swb

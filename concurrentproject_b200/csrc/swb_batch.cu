@@ -51,6 +51,14 @@ const void* banded2_kernel(int mode) {
 const void* banded8_kernel(int mode) {
   return mode == 0 ? (const void*)sw_banded8_kernel<0> : (const void*)sw_banded8_kernel<1>;
 }
+const void* banded_wide_kernel(int mode, int width) {
+  switch (width) {
+    case 128: return mode == 0 ? (const void*)sw_banded_wide_kernel<0, 128> : (const void*)sw_banded_wide_kernel<1, 128>;
+    case 256: return mode == 0 ? (const void*)sw_banded_wide_kernel<0, 256> : (const void*)sw_banded_wide_kernel<1, 256>;
+    case 512: return mode == 0 ? (const void*)sw_banded_wide_kernel<0, 512> : (const void*)sw_banded_wide_kernel<1, 512>;
+    default: return nullptr;
+  }
+}
 
 // Packs a batch: for every pair the shorter sequence becomes Q, the longer one T; both as 2-bit codes,
 // 32 per 64-bit word, fixed word strides per pair.  One thread per output word.

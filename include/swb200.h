@@ -46,7 +46,8 @@ typedef struct {
                       7 = the CTA-chained engine (csrc/swb_chain.cuh: one band per warp, four consecutive bands per CTA handed
                       over through shared memory; plain 16-bit lanes, one GPU, rows 1,2,3,4,6,8) -- what "auto" picks for
                       fill-dominated pairs such as 100 000 x 100 000.
-                      banded calls: 0 = 4 threads per pair (default), 8 = 8 threads per pair, 16 = 16 threads per pair, 2 = 2 threads per pair */
+                      banded calls with a 64-diagonal band: 0 = 4 threads per pair (default), 8 = 8 threads per pair, 16 = 16
+                      threads per pair, 2 = 2 threads per pair; ignored for wider bands */
   int ctas;        /* thread blocks (<= co-resident limit); 0 auto */
   int no_linear;   /* 1 = keep the affine kernel even when gap_init == gap_ext */
   int orient;      /* 0 auto (stripe the longer sequence across lanes), 1 = stripe seq1, 2 = stripe seq2 */
@@ -308,7 +309,10 @@ SWB200_API int swb200_batch_align_long(swb200_batch* batch, const swb200_params*
 /* ---- banded batches (long reads): cell (i,j), i = row in seq2, j = column in seq1, is scored iff
  * band_lo <= j - i <= band_hi; everything outside the band is H=E=F=0 and excluded from the max.  The reference
  * has no banded mode; semantics = main.cpp:57-63 restricted to the band (oracle: oracle_gotoh_banded).
- * This kernel handles exactly 64 diagonals: band_hi == band_lo + 63. */
+ * The band holds W = band_hi - band_lo + 1 diagonals, W = 64, 128, 256 or 512; any other width is SWB200_ERR_ARG.  The
+ * 16-bit range rule match*min(len) <= 32766 - match (SWB200_ERR_RANGE) does not depend on W.  swb200_last_run reports
+ * bands = W and config 204 / 208 / 216 / 202 (W = 64: the layout options.config picks) or 2128 / 2256 / 2512 (W = 128 /
+ * 256 / 512: W / 16 threads per pair, options.config ignored). */
 /* One banded pair (the batch call with npairs = 1). */
 SWB200_API int swb200_score_banded(const unsigned char* seq1, int n, const unsigned char* seq2, int m, int band_lo,
                                    int band_hi, const swb200_params* p, int* score_out);
@@ -332,10 +336,11 @@ SWB200_API int swb200_batch_score_banded(swb200_batch* batch, int band_lo, int b
  * Output format, '='/'X' split, ops_stride overflow (ops_count = -n; the host call zero-fills that slot), the "1I1I"
  * split when gap_ext > gap_init, the device re-score and its SWB200_ERR_CUDA ("internal: ...") are swb200_align_batch's.
  * When B covers the whole pair (band_lo <= -(len2-1), band_hi >= len1-1) the result is swb200_align_batch's.
- * Limits and errors are swb200_score_banded_batch's: bytes A,C,G,T (SWB200_ERR_ALPHABET); band_hi == band_lo + 63
- * (SWB200_ERR_ARG); match*min(len) <= 32766 - match (SWB200_ERR_RANGE), so every accepted pair can be checked against
+ * Limits and errors are swb200_score_banded_batch's: bytes A,C,G,T (SWB200_ERR_ALPHABET); W = band_hi - band_lo + 1
+ * in {64, 128, 256, 512} (SWB200_ERR_ARG); match*min(len) <= 32766 - match (SWB200_ERR_RANGE), so every accepted pair can be checked against
  * the score-only call.  All argument checks run before a device is touched.  One warp per pair on the device; the host
- * call packs in chunks and shards over swb200_set_devices like swb200_align_batch.  opt is reserved (NULL). */
+ * call packs in chunks and shards over swb200_set_devices like swb200_align_batch.  opt is reserved (NULL).
+ * swb200_last_run: lanes 32, bands = W, config 310 / 311 / 312 / 313 for W = 64 / 128 / 256 / 512. */
 SWB200_API int swb200_align_banded_batch(const unsigned char* seq1_all, const long long* off1, const int* len1,
                                          const unsigned char* seq2_all, const long long* off2, const int* len2,
                                          long long npairs, int band_lo, int band_hi, const swb200_params* p,
