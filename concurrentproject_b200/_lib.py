@@ -92,6 +92,13 @@ EXPORTS = {
                             C.POINTER(C.c_uint), C.c_int, C.POINTER(C.c_int)], C.c_int),
     "swb200_batch_align": ([C.c_void_p, C.POINTER(Params), C.POINTER(Options), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                             C.c_int, C.c_void_p], C.c_int),
+    "swb200_score_batch_bytes": ([U8P, C.POINTER(C.c_longlong), C.POINTER(C.c_int), U8P, C.POINTER(C.c_longlong), C.POINTER(C.c_int),
+                                  C.c_longlong, C.POINTER(Params), C.POINTER(Options), C.POINTER(C.c_int)], C.c_int),
+    "swb200_align_batch_bytes": ([U8P, C.POINTER(C.c_longlong), C.POINTER(C.c_int), U8P, C.POINTER(C.c_longlong), C.POINTER(C.c_int),
+                                  C.c_longlong, C.POINTER(Params), C.POINTER(Options), C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                  C.POINTER(C.c_uint), C.c_int, C.POINTER(C.c_int)], C.c_int),
+    "swb200_batch_pack_device_bytes": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_longlong, C.c_int, C.c_int, C.c_longlong, C.c_void_p, C.POINTER(C.c_void_p)], C.c_int),
     "swb200_align_banded_batch": ([U8P, C.POINTER(C.c_longlong), C.POINTER(C.c_int), U8P, C.POINTER(C.c_longlong),
                                    C.POINTER(C.c_int), C.c_longlong, C.c_int, C.c_int, C.POINTER(Params), C.POINTER(Options),
                                    C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_uint), C.c_int, C.POINTER(C.c_int)], C.c_int),

@@ -289,12 +289,25 @@ def score_banded_batch_flat(flat1, off1, len1, flat2, off2, len2, band_lo: int =
 
 
 class PackedBatch:
-    """A batch packed into the HBM-resident 2-bit format (swb200_batch_*).  All arguments are device addresses."""
+    """A batch packed into the HBM-resident 2-bit format (swb200_batch_*).  All arguments are device addresses.
+    byte_symbols=True keeps every byte as it is (swb200_batch_pack_device_bytes: any alphabet, shorter side <= 1024);
+    such a batch is scored by score and aligned by align with the byte kernels, and refused by the other calls."""
 
     def __init__(self, ctx: Context, d_seq1: int, d_off1: int, d_len1: int, d_seq2: int, d_off2: int, d_len2: int, npairs: int,
-                 max_short: int, max_long: int, total_cells: int, stream: int = 0, keep_order: bool = False):
+                 max_short: int, max_long: int, total_cells: int, stream: int = 0, keep_order: bool = False,
+                 byte_symbols: bool = False):
         self.ctx, self.npairs = ctx, npairs
         self.handle = C.c_void_p()
+        if byte_symbols:
+            if keep_order:
+                raise ValueError("a byte batch puts the shorter sequence first: keep_order must be False")
+            rc = _lib.load().swb200_batch_pack_device_bytes(ctx.handle, C.c_void_p(d_seq1), C.c_void_p(d_off1), C.c_void_p(d_len1),
+                                                            C.c_void_p(d_seq2), C.c_void_p(d_off2), C.c_void_p(d_len2), npairs,
+                                                            max_short, max_long, total_cells, C.c_void_p(stream),
+                                                            C.byref(self.handle))
+            if rc != 0:
+                raise SwbError(rc, "swb200_batch_pack_device_bytes")
+            return
         rc = _lib.load().swb200_batch_pack_device(ctx.handle, C.c_void_p(d_seq1), C.c_void_p(d_off1), C.c_void_p(d_len1),
                                                   C.c_void_p(d_seq2), C.c_void_p(d_off2), C.c_void_p(d_len2), npairs, max_short,
                                                   max_long, total_cells, int(keep_order), C.c_void_p(stream), C.byref(self.handle))
@@ -539,6 +552,69 @@ def align_batch(seqs1, seqs2, params: Sequence[int] = DEFAULT_PARAMS, *, ops_str
     if len(redo):
         stride = int((l1[redo].astype(np.int64) + l2[redo]).max())
         _, _, ops2, cnt2 = align_batch_ops(f1, o1[redo].copy(), l1[redo].copy(), f2, o2[redo].copy(), l2[redo].copy(), params, stride)
+        for r, k in enumerate(redo.tolist()):
+            cigars[k] = cigar_string(ops2[r, :cnt2[r]])
+    return scores, spans, cigars
+
+
+# ---- byte batches: any bytes, shorter side <= 1024 (swb200_score_batch_bytes, swb200_align_batch_bytes) -------------
+def score_batch_bytes(seqs1, seqs2, params: Sequence[int] = DEFAULT_PARAMS) -> np.ndarray:
+    """score_batch for pairs in any bytes (N, IUPAC codes, lower case, amino acids): bytes compare as they are, exactly
+    as score compares them, in one batch call (swb200_score_batch_bytes; the limits of score_batch without its alphabet)."""
+    if len(seqs1) != len(seqs2):
+        raise ValueError("seqs1 and seqs2 differ in length")
+    return score_batch_bytes_flat(*_flatten(seqs1), *_flatten(seqs2), params)
+
+
+def score_batch_bytes_flat(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray, flat2: np.ndarray, off2: np.ndarray,
+                           len2: np.ndarray, params: Sequence[int] = DEFAULT_PARAMS) -> np.ndarray:
+    """swb200_score_batch_bytes on already flattened HOST arrays (uint8 bytes, int64 offsets, int32 lengths)."""
+    n = len(len1)
+    out = np.zeros(n, dtype=np.int32)
+    p = _params(params)
+    LL, I = C.POINTER(C.c_longlong), C.POINTER(C.c_int)
+    rc = _lib.load().swb200_score_batch_bytes(_ptr(flat1), off1.ctypes.data_as(LL), len1.ctypes.data_as(I), _ptr(flat2),
+                                              off2.ctypes.data_as(LL), len2.ctypes.data_as(I), n, C.byref(p), None,
+                                              out.ctypes.data_as(I))
+    if rc != 0:
+        raise SwbError(rc, "swb200_score_batch_bytes")
+    return out
+
+
+def align_batch_bytes_ops(flat1: np.ndarray, off1: np.ndarray, len1: np.ndarray, flat2: np.ndarray, off2: np.ndarray,
+                          len2: np.ndarray, params: Sequence[int] = DEFAULT_PARAMS, ops_stride: int = OPS_STRIDE):
+    """swb200_align_batch_bytes on flattened HOST arrays: (scores, spans, ops, ops_count) as align_batch_ops returns them."""
+    n = len(len1)
+    scores = np.zeros(n, dtype=np.int32)
+    spans = np.zeros((n, 4), dtype=np.int32)
+    ops = np.zeros((n, ops_stride), dtype=np.uint32)
+    cnt = np.zeros(n, dtype=np.int32)
+    p = _params(params)
+    LL, I = C.POINTER(C.c_longlong), C.POINTER(C.c_int)
+    rc = _lib.load().swb200_align_batch_bytes(_ptr(flat1), off1.ctypes.data_as(LL), len1.ctypes.data_as(I), _ptr(flat2),
+                                              off2.ctypes.data_as(LL), len2.ctypes.data_as(I), n, C.byref(p), None,
+                                              scores.ctypes.data_as(I), spans.ctypes.data_as(I),
+                                              ops.ctypes.data_as(C.POINTER(C.c_uint)), ops_stride, cnt.ctypes.data_as(I))
+    if rc != 0:
+        raise SwbError(rc, "swb200_align_batch_bytes")
+    return scores, spans, ops, cnt
+
+
+def align_batch_bytes(seqs1, seqs2, params: Sequence[int] = DEFAULT_PARAMS, *, ops_stride: int = OPS_STRIDE):
+    """(scores int32[n], spans int32[n, 4], cigars list[str]): align(seqs1[k], seqs2[k]) for every pair in any bytes, in
+    one batch call (swb200_align_batch_bytes; the limits of align_batch without its alphabet).  Pairs whose alignment
+    needs more than ops_stride operations are aligned again with room for len1 + len2 operations."""
+    if len(seqs1) != len(seqs2):
+        raise ValueError("seqs1 and seqs2 differ in length")
+    f1, o1, l1 = _flatten(seqs1)
+    f2, o2, l2 = _flatten(seqs2)
+    scores, spans, ops, cnt = align_batch_bytes_ops(f1, o1, l1, f2, o2, l2, params, ops_stride)
+    cigars = [cigar_string(ops[k, :c]) if c >= 0 else None for k, c in enumerate(cnt.tolist())]
+    redo = np.flatnonzero(cnt < 0)
+    if len(redo):
+        stride = int((l1[redo].astype(np.int64) + l2[redo]).max())
+        _, _, ops2, cnt2 = align_batch_bytes_ops(f1, o1[redo].copy(), l1[redo].copy(), f2, o2[redo].copy(), l2[redo].copy(),
+                                                 params, stride)
         for r, k in enumerate(redo.tolist()):
             cigars[k] = cigar_string(ops2[r, :cnt2[r]])
     return scores, spans, cigars

@@ -298,14 +298,18 @@ void launch_pack_batch(const uint8_t* seq1, const long long* off1, const int* le
                        const long long* off2, const int* len2, long long npairs, long long q_stride, long long t_stride,
                        uint64_t* q_words, uint64_t* t_words, int* q_len, int* t_len, int keep_order, int* status,
                        int blocks, cudaStream_t s);
+void launch_pack_bytes(const uint8_t* seq1, const long long* off1, const int* len1, const uint8_t* seq2,
+                       const long long* off2, const int* len2, long long npairs, long long q_stride, long long t_stride,
+                       uint64_t* q_words, uint64_t* t_words, int* q_len, int* t_len, int blocks, cudaStream_t s);
 }
 
-// A packed batch resident in HBM (2-bit codes, fixed word strides, shorter sequence of each pair first).
+// A packed batch resident in HBM (2-bit codes, or bytes, fixed word strides, shorter sequence of each pair first).
 struct swb200_batch {
   swb200_ctx* ctx = nullptr;
   long long npairs = 0, q_stride = 0, t_stride = 0;
   int max_short = 0, max_long = 0;
   int keep_order = 0;          // 1: q = seq1, t = seq2 exactly as given (banded scoring needs j-i)
+  int bytes = 0;               // 1: raw bytes, 8 per word (swb200_batch_pack_device_bytes; the byte kernels only)
   uint64_t* q_words = nullptr;
   uint64_t* t_words = nullptr;
   int* q_len = nullptr;
@@ -1400,10 +1404,25 @@ static bool fits_strides(int q, int t, const Strides& s, bool keep_order) {
   const Strides need = batch_strides_for(q, t, keep_order);
   return q >= 0 && t >= 0 && need.q <= s.q && need.t <= s.t;
 }
+// Word strides of the byte layout (8 bytes per 64-bit word, shorter sequence first): at least one word; the byte kernels
+// read no word past a sequence's end.
+static Strides byte_strides_for(int max_q, int max_t) {
+  return Strides{std::max(1, (max_q + 7) / 8), std::max(1, (max_t + 7) / 8)};
+}
+// The packer of either layout: bytes = raw bytes (byte_strides_for, never keep_order), else 2-bit codes.
+static void launch_pack(bool bytes, const uint8_t* seq1, const long long* off1, const int* len1, const uint8_t* seq2,
+                        const long long* off2, const int* len2, long long npairs, const Strides& st, uint64_t* q_words,
+                        uint64_t* t_words, int* q_len, int* t_len, int keep_order, int* status, int blocks, cudaStream_t s) {
+  if (bytes)
+    swb::launch_pack_bytes(seq1, off1, len1, seq2, off2, len2, npairs, st.q, st.t, q_words, t_words, q_len, t_len, blocks, s);
+  else
+    swb::launch_pack_batch(seq1, off1, len1, seq2, off2, len2, npairs, st.q, st.t, q_words, t_words, q_len, t_len, keep_order,
+                           status, blocks, s);
+}
 
-int swb200_batch_pack_device(swb200_ctx* c, const unsigned char* d_seq1, const long long* d_off1, const int* d_len1,
+static int batch_pack_device(swb200_ctx* c, const unsigned char* d_seq1, const long long* d_off1, const int* d_len1,
                              const unsigned char* d_seq2, const long long* d_off2, const int* d_len2, long long npairs,
-                             int max_short, int max_long, long long total_cells, int keep_order, void* stream,
+                             int max_short, int max_long, long long total_cells, int keep_order, bool bytes, void* stream,
                              swb200_batch** out) {
   if (!c || !out || npairs < 0 || max_short < 0 || max_long < 0 || (!keep_order && max_long < max_short))
     return fail(SWB200_ERR_ARG, "bad batch arguments");
@@ -1414,7 +1433,8 @@ int swb200_batch_pack_device(swb200_ctx* c, const unsigned char* d_seq1, const l
   std::unique_ptr<swb200_batch, BatchDeleter> b(new swb200_batch());   // freed on every early return
   b->ctx = c; b->npairs = npairs; b->max_short = max_short; b->max_long = max_long; b->cells = total_cells;
   b->keep_order = keep_order ? 1 : 0;
-  const Strides st = batch_strides_for(max_short, max_long, keep_order);
+  b->bytes = bytes ? 1 : 0;
+  const Strides st = bytes ? byte_strides_for(max_short, max_long) : batch_strides_for(max_short, max_long, keep_order);
   b->q_stride = st.q; b->t_stride = st.t;
   const size_t np = (size_t)std::max<long long>(npairs, 1);
   SWB_CUDA(cudaMalloc(&b->q_words, np * b->q_stride * sizeof(uint64_t)));
@@ -1426,8 +1446,8 @@ int swb200_batch_pack_device(swb200_ctx* c, const unsigned char* d_seq1, const l
   if (npairs > 0) {
     const long long total = npairs * (b->q_stride + b->t_stride);
     const int blocks = (int)std::min<long long>((total + 255) / 256, 64LL * c->sms);
-    swb::launch_pack_batch(d_seq1, d_off1, d_len1, d_seq2, d_off2, d_len2, npairs, b->q_stride, b->t_stride, b->q_words,
-                           b->t_words, b->q_len, b->t_len, b->keep_order, c->d_result, blocks, s);
+    launch_pack(bytes, d_seq1, d_off1, d_len1, d_seq2, d_off2, d_len2, npairs, st, b->q_words, b->t_words, b->q_len, b->t_len,
+                b->keep_order, c->d_result, blocks, s);
     SWB_CUDA(cudaGetLastError());
     if (b->len1) SWB_CUDA(cudaMemcpyAsync(b->len1, d_len1, (size_t)npairs * sizeof(int), cudaMemcpyDeviceToDevice, s));
   }
@@ -1439,12 +1459,34 @@ int swb200_batch_pack_device(swb200_ctx* c, const unsigned char* d_seq1, const l
   return SWB200_OK;
 }
 
+int swb200_batch_pack_device(swb200_ctx* c, const unsigned char* d_seq1, const long long* d_off1, const int* d_len1,
+                             const unsigned char* d_seq2, const long long* d_off2, const int* d_len2, long long npairs,
+                             int max_short, int max_long, long long total_cells, int keep_order, void* stream,
+                             swb200_batch** out) {
+  return batch_pack_device(c, d_seq1, d_off1, d_len1, d_seq2, d_off2, d_len2, npairs, max_short, max_long, total_cells,
+                           keep_order, false, stream, out);
+}
+
+int swb200_batch_pack_device_bytes(swb200_ctx* c, const unsigned char* d_seq1, const long long* d_off1, const int* d_len1,
+                                   const unsigned char* d_seq2, const long long* d_off2, const int* d_len2, long long npairs,
+                                   int max_short, int max_long, long long total_cells, void* stream, swb200_batch** out) {
+  return batch_pack_device(c, d_seq1, d_off1, d_len1, d_seq2, d_off2, d_len2, npairs, max_short, max_long, total_cells, 0,
+                           true, stream, out);
+}
+
 // A contiguous range of pairs of a packed batch (all pointers already offset to its first pair).
 struct BatchView {
   const uint64_t* q_words; const uint64_t* t_words; const int* q_len; const int* t_len;
   long long q_stride, t_stride, npairs;
   int max_short, max_long;      // of the WHOLE batch: every range of one batch runs the same kernel
+  bool bytes = false;           // the byte layout (byte_strides_for): only the byte kernels read it
 };
+
+// The calls that have no byte kernel refuse a byte batch.
+static int refuse_bytes(const swb200_batch* b) {
+  return b->bytes ? fail(SWB200_ERR_ARG, "batch was packed as bytes; only swb200_batch_score and swb200_batch_align take it")
+                  : SWB200_OK;
+}
 
 static int check_batch_score(const swb200_params& p, int keep_order, int max_short) {
   if (keep_order) return fail(SWB200_ERR_ARG, "batch was packed in caller order (banded); re-pack with keep_order=0");
@@ -1483,6 +1525,34 @@ static int launch_batch_score(swb200_ctx* c, const BatchView& v, const swb200_pa
   SWB_CUDA(cudaLaunchKernel(kern, dim3((unsigned)ctas), dim3(256), args, 0, s));
   info->lanes = 16; info->linear = mode == 1; info->rows = R; info->config = 100 + G; info->ctas = (int)ctas;
   info->warps = (int)ctas * 8; info->bands = 0; info->engine_launches += 1;
+  return SWB200_OK;
+}
+
+// The byte score kernel (swb_bytes_batch.cu): one thread per pair, as many threads as are resident at once.
+static long long bytes_score_threads(swb200_ctx* c) {
+  int per_sm = 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, swb::bytes_score_kernel_ptr(), 256, 0) != cudaSuccess || per_sm < 1)
+    per_sm = 1;
+  return 256LL * c->sms * per_sm;
+}
+
+// Launches the byte score kernel for one range of a byte batch; no synchronisation, no events.  The column buffer is
+// ab_col, shared by the ranges of one call (they run one after another on stream s).
+static int launch_bytes_score(swb200_ctx* c, const BatchView& v, const swb200_params& p, cudaStream_t s, int* d_scores,
+                              swb200_run_info* info) {
+  if (v.npairs == 0) return SWB200_OK;
+  const long long blocks = std::max(1LL, std::min<long long>((v.npairs + 255) / 256, bytes_score_threads(c) / 256));
+  const long long nt = blocks * 256;
+  if (int rc = grow(c->ab_col, c->ab_col_cap, (size_t)(v.max_short + 1) * nt, false, s)) return rc;
+  swb::AlignBatchParams P{};
+  P.q_words = v.q_words; P.t_words = v.t_words; P.q_len = v.q_len; P.t_len = v.t_len;
+  P.q_stride = v.q_stride; P.t_stride = v.t_stride; P.npairs = v.npairs;
+  P.match = p.match; P.mismatch = p.mismatch; P.gap_init = p.gap_init; P.gap_ext = p.gap_ext;
+  P.scores = d_scores; P.col = c->ab_col; P.nthreads = nt;
+  swb::launch_bytes_score(P, (int)blocks, s);
+  SWB_CUDA(cudaGetLastError());
+  info->lanes = 32; info->linear = 0; info->rows = swb::kAlignStrip; info->config = 101; info->ctas = (int)blocks;
+  info->warps = (int)blocks * 8; info->bands = 0; info->engine_launches += 1;
   return SWB200_OK;
 }
 
@@ -1614,7 +1684,8 @@ static int launch_banded_score(swb200_ctx* c, const BatchView& v, int band_lo, i
 }
 
 static BatchView whole_batch(const swb200_batch* b) {
-  return BatchView{b->q_words, b->t_words, b->q_len, b->t_len, b->q_stride, b->t_stride, b->npairs, b->max_short, b->max_long};
+  return BatchView{b->q_words, b->t_words, b->q_len, b->t_len, b->q_stride, b->t_stride, b->npairs, b->max_short, b->max_long,
+                   b->bytes != 0};
 }
 
 // The device-batch calls after their argument checks: b's context locked and its device current, the run info reset to
@@ -1648,7 +1719,8 @@ int swb200_batch_score(swb200_batch* b, const swb200_params* pp, const swb200_op
   int rc;
   if ((rc = check_params(p)) || (rc = check_batch_score(p, b->keep_order, b->max_short))) return rc;
   return run_device_batch(b, b->cells, stream, [&](swb200_ctx* c, cudaStream_t s) {
-    return launch_batch_score(c, whole_batch(b), p, o, s, d_scores, &c->info);
+    return b->bytes ? launch_bytes_score(c, whole_batch(b), p, s, d_scores, &c->info)
+                    : launch_batch_score(c, whole_batch(b), p, o, s, d_scores, &c->info);
   });
 }
 
@@ -1657,7 +1729,7 @@ int swb200_batch_score_long(swb200_batch* b, const swb200_params* pp, const swb2
   const swb200_params p = params_or_default(pp);
   const swb200_options o = options_or_default(oo);
   int rc;
-  if ((rc = check_params(p)) || (rc = check_long_score(p, o, b->keep_order, b->max_short))) return rc;
+  if ((rc = refuse_bytes(b)) || (rc = check_params(p)) || (rc = check_long_score(p, o, b->keep_order, b->max_short))) return rc;
   return run_device_batch(b, b->cells, stream, [&](swb200_ctx* c, cudaStream_t s) {
     return launch_long_score(c, whole_batch(b), p, o, s, d_scores, &c->info);
   });
@@ -1669,7 +1741,8 @@ int swb200_batch_score_banded(swb200_batch* b, int band_lo, int band_hi, const s
   const swb200_params p = params_or_default(pp);
   const swb200_options o = options_or_default(oo);
   int rc;
-  if ((rc = check_params(p)) || (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
+  if ((rc = refuse_bytes(b)) || (rc = check_params(p)) ||
+      (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
   return run_device_batch(b, b->cells, stream, [&](swb200_ctx* c, cudaStream_t s) {
     return launch_banded_score(c, whole_batch(b), band_lo, band_hi - band_lo + 1, p, o, s, d_scores, &c->info);
   });
@@ -1724,8 +1797,8 @@ static PairScan scan_pairs(const HostPairs& h, long long k0, long long k1) {
   return PairScan{neg, mx1, mx2, mxmin, cells, lo1, hi1, lo2, hi2};
 }
 
-// which kernel a host ASCII score batch runs
-enum class ScoreKind { batch, banded, long_pairs };
+// which kernel a host ASCII score batch runs (bytes: the byte layout and its score kernel, the limits of batch)
+enum class ScoreKind { batch, banded, long_pairs, bytes };
 
 static int check_score_pairs(const PairScan& s, const swb200_params& p, const swb200_options& o, ScoreKind kind, int band_lo,
                              int band_hi) {
@@ -1754,16 +1827,16 @@ static int chunk_events_at_least(swb200_ctx* c, size_t n) {
 // copies chunk k+1 from the host while aux_stream packs chunk k and runs each_chunk (if any) on it.  The staging pool is
 // sized for the whole range, so chunks need no double buffering: every byte keeps its position relative to the range's
 // lowest offset.  With pinned host buffers the call runs at PCIe speed.  ev0 is recorded at the first pack; *staged is
-// the packed range.  wave > 0: every chunk but the last holds a whole multiple of wave pairs.
+// the packed range.  wave > 0: every chunk but the last holds a whole multiple of wave pairs.  bytes: the byte layout.
 static int stage_and_pack_locked(swb200_ctx* c, const HostPairs& h, long long npairs, const PairScan& part,
-                                 const PairScan& whole, bool keep_order, BatchView* staged,
+                                 const PairScan& whole, bool keep_order, bool bytes, BatchView* staged,
                                  const std::function<int(const BatchView& chunk, long long k0)>& each_chunk,
                                  long long wave = 0) {
   cudaStream_t sc = c->own_stream, sk = c->aux_stream;
   const size_t np = (size_t)npairs;
   const long long base1 = part.lo1 & ~15LL, base2 = part.lo2 & ~15LL;
   const int max_short = whole.max_short(keep_order), max_long = whole.max_long(keep_order);
-  const Strides st = batch_strides_for(max_short, max_long, keep_order);
+  const Strides st = bytes ? byte_strides_for(max_short, max_long) : batch_strides_for(max_short, max_long, keep_order);
   int rc;
   if ((rc = grow(c->hb_seq1, c->hb_seq1_cap, (size_t)(part.hi1 - base1) + 16, false, sc)) ||
       (rc = grow(c->hb_seq2, c->hb_seq2_cap, (size_t)(part.hi2 - base2) + 16, false, sc)) ||
@@ -1772,7 +1845,7 @@ static int stage_and_pack_locked(swb200_ctx* c, const HostPairs& h, long long np
       (rc = grow(c->hb_scores, c->hb_scores_cap, np, false, sc)) ||
       (rc = grow(c->hb_qw, c->hb_qw_cap, np * st.q, false, sc)) || (rc = grow(c->hb_tw, c->hb_tw_cap, np * st.t, false, sc)) ||
       (rc = grow(c->hb_ql, c->hb_ql_cap, np, false, sc)) || (rc = grow(c->hb_tl, c->hb_tl_cap, np, false, sc))) return rc;
-  *staged = BatchView{c->hb_qw, c->hb_tw, c->hb_ql, c->hb_tl, st.q, st.t, npairs, max_short, max_long};
+  *staged = BatchView{c->hb_qw, c->hb_tw, c->hb_ql, c->hb_tl, st.q, st.t, npairs, max_short, max_long, bytes};
   SWB_CUDA(cudaMemsetAsync(c->d_result, 0, 10 * sizeof(int), sc));
   SWB_CUDA(cudaMemcpyAsync(c->hb_off1, h.off1, np * sizeof(long long), cudaMemcpyHostToDevice, sc));
   SWB_CUDA(cudaMemcpyAsync(c->hb_off2, h.off2, np * sizeof(long long), cudaMemcpyHostToDevice, sc));
@@ -1791,14 +1864,14 @@ static int stage_and_pack_locked(swb200_ctx* c, const HostPairs& h, long long np
     const long long nk = k1 - k0;
     const int blocks = (int)std::min<long long>((nk * (st.q + st.t) + 255) / 256, 64LL * c->sms);
     // the pack kernel adds the absolute offsets: hand it the staging pointers shifted back by the range's base
-    swb::launch_pack_batch(c->hb_seq1 - base1, c->hb_off1 + k0, c->hb_len1 + k0, c->hb_seq2 - base2, c->hb_off2 + k0,
-                           c->hb_len2 + k0, nk, st.q, st.t, c->hb_qw + k0 * st.q, c->hb_tw + k0 * st.t, c->hb_ql + k0,
-                           c->hb_tl + k0, keep_order ? 1 : 0, c->d_result, blocks, sk);
+    launch_pack(bytes, c->hb_seq1 - base1, c->hb_off1 + k0, c->hb_len1 + k0, c->hb_seq2 - base2, c->hb_off2 + k0,
+                c->hb_len2 + k0, nk, st, c->hb_qw + k0 * st.q, c->hb_tw + k0 * st.t, c->hb_ql + k0, c->hb_tl + k0,
+                keep_order ? 1 : 0, c->d_result, blocks, sk);
     SWB_CUDA(cudaGetLastError());
     c->info.aux_launches += 1;
     if (!each_chunk) return SWB200_OK;
     return each_chunk(BatchView{c->hb_qw + k0 * st.q, c->hb_tw + k0 * st.t, c->hb_ql + k0, c->hb_tl + k0, st.q, st.t, nk,
-                                max_short, max_long}, k0);
+                                max_short, max_long, bytes}, k0);
   };
   // a chunk is issued the moment the scan over the pairs has found its end, so the GPU works while the host is still
   // cutting the later chunks
@@ -1828,13 +1901,15 @@ static int score_ascii_ctx(swb200_ctx* c, const HostPairs& h, long long npairs, 
   c->info = swb200_run_info{};
   c->info.cells = part.cells;
   BatchView staged;
-  // a multi-band launch runs as long as its longest pairs however few they are: its chunks are whole waves of warps
-  const bool banded = kind == ScoreKind::banded;
-  const long long wave = kind == ScoreKind::long_pairs ? long_wave_pairs(c, p, o, whole.max_min) : 0;
-  int rc = stage_and_pack_locked(c, h, npairs, part, whole, banded, &staged, [&](const BatchView& v, long long k0) {
+  // a multi-band launch runs as long as its longest pairs however few they are: its chunks are whole waves of warps; a
+  // byte launch runs one pair per thread: its chunks are whole waves of resident threads
+  const bool banded = kind == ScoreKind::banded, bytes = kind == ScoreKind::bytes;
+  const long long wave = kind == ScoreKind::long_pairs ? long_wave_pairs(c, p, o, whole.max_min) : (bytes ? bytes_score_threads(c) : 0);
+  int rc = stage_and_pack_locked(c, h, npairs, part, whole, banded, bytes, &staged, [&](const BatchView& v, long long k0) {
     switch (kind) {
       case ScoreKind::banded: return launch_banded_score(c, v, band_lo, band_w, p, o, sk, c->hb_scores + k0, &c->info);
       case ScoreKind::long_pairs: return launch_long_score(c, v, p, o, sk, c->hb_scores + k0, &c->info);
+      case ScoreKind::bytes: return launch_bytes_score(c, v, p, sk, c->hb_scores + k0, &c->info);
       default: return launch_batch_score(c, v, p, o, sk, c->hb_scores + k0, &c->info);
     }
   }, wave);
@@ -2223,7 +2298,7 @@ static int score_pair_on_pool(const unsigned char* seq1, long long n, const unsi
   return handled ? SWB200_OK : 1;
 }
 
-// swb200_score_batch / swb200_score_banded_batch / swb200_score_long_batch
+// swb200_score_batch / swb200_score_banded_batch / swb200_score_long_batch / swb200_score_batch_bytes
 static int score_batch_host(const HostPairs& in, long long npairs, const swb200_params* pp, const swb200_options* oo,
                             ScoreKind kind, int band_lo, int band_hi, int* scores_out) {
   if (npairs < 0 || (npairs > 0 && (!in.seq1 || !in.seq2 || !in.off1 || !in.off2 || !in.len1 || !in.len2 || !scores_out)))
@@ -2350,6 +2425,13 @@ int swb200_score_batch(const unsigned char* seq1_all, const long long* off1, con
                        const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
                        const swb200_params* p, const swb200_options* opt, int* scores_out) {
   return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, ScoreKind::batch, 0, 0,
+                          scores_out);
+}
+
+int swb200_score_batch_bytes(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                             const unsigned char* seq2_all, const long long* off2, const int* len2, long long npairs,
+                             const swb200_params* p, const swb200_options* opt, int* scores_out) {
+  return score_batch_host(HostPairs{seq1_all, off1, len1, seq2_all, off2, len2}, npairs, p, opt, ScoreKind::bytes, 0, 0,
                           scores_out);
 }
 
@@ -2572,7 +2654,8 @@ int align_rounds_locked(swb200_ctx* c, cudaStream_t s, long long npairs, size_t 
 }
 
 // Passes 1-3 and the walk over a packed range (shorter sequence first, len1 = the caller's seq1 lengths), everything on
-// stream s of c's device.  Synchronises once per trace round (the pending count decides whether another round runs).
+// stream s of c's device, with the kernels of the range's layout (v.bytes: swb_bytes_batch.cu).  Synchronises once per
+// trace round (the pending count decides whether another round runs).
 int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, const swb200_params& p, cudaStream_t s,
                         int* d_scores, int* d_spans, uint32_t* d_ops, int ops_stride, int* d_ops_count, swb200_run_info* info) {
   if (v.npairs == 0) return SWB200_OK;
@@ -2595,8 +2678,10 @@ int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, co
   P.pending = c->ab_list; P.npending = reinterpret_cast<int*>(c->ab_misc) + 1;
   P.ops = d_ops; P.ops_stride = ops_stride; P.ops_count = d_ops_count;
   P.err = reinterpret_cast<int*>(c->ab_misc); P.cells = c->ab_misc + 2;
-  swb::launch_align_span(P, (int)blocks, s);
-  swb::launch_align_trace(P, (int)blocks, s);
+  const auto span = v.bytes ? swb::launch_bytes_span : swb::launch_align_span;
+  const auto trace = v.bytes ? swb::launch_bytes_trace : swb::launch_align_trace;
+  span(P, (int)blocks, s);
+  trace(P, (int)blocks, s);
   SWB_CUDA(cudaGetLastError());
   info->engine_launches += 2;
   // rectangles larger than a slot: the pool, emptied for every round; its first taker always fits
@@ -2604,9 +2689,9 @@ int align_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len1, co
   if ((rc = align_rounds_locked(c, s, v.npairs, need, info, [&](const int* todo, int ntodo, int* pending) {
          P.pool = c->ab_pool; P.pool_words = (long long)c->ab_pool_cap;
          P.todo = todo; P.ntodo = ntodo; P.pending = pending;
-         swb::launch_align_trace(P, (int)std::max(1LL, std::min<long long>(blocks, (ntodo + 255) / 256)), s);
+         trace(P, (int)std::max(1LL, std::min<long long>(blocks, (ntodo + 255) / 256)), s);
        }))) return rc;
-  info->lanes = 32; info->config = 300; info->rows = swb::kAlignStrip;
+  info->lanes = 32; info->config = v.bytes ? 301 : 300; info->rows = swb::kAlignStrip;
   return SWB200_OK;
 }
 
@@ -2751,8 +2836,8 @@ int align_long_packed_locked(swb200_ctx* c, const BatchView& v, const int* d_len
 
 }  // namespace
 
-// which kernels a host batch alignment runs
-enum class AlignKind { batch, banded, long_pairs };
+// which kernels a host batch alignment runs (bytes: the byte layout and kernels, the limits of batch)
+enum class AlignKind { batch, banded, long_pairs, bytes };
 
 // One context's share of a host batch alignment (arguments checked by the caller): the copy/pack pipeline of the score
 // calls, then the passes over the whole range, then the outputs back.  banded: the pairs stay in caller order and the
@@ -2770,7 +2855,8 @@ static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npa
       (rc = grow(c->hb_ops, c->hb_ops_cap, np * (size_t)ops_stride, false, sc)) || (rc = grow(c->hb_opsn, c->hb_opsn_cap, np, false, sc))) return rc;
   c->info = swb200_run_info{};
   BatchView v;
-  if ((rc = stage_and_pack_locked(c, h, npairs, part, whole, kind == AlignKind::banded, &v, nullptr))) return rc;
+  if ((rc = stage_and_pack_locked(c, h, npairs, part, whole, kind == AlignKind::banded, kind == AlignKind::bytes, &v, nullptr)))
+    return rc;
   SWB_CUDA(cudaMemcpyAsync(c->h_result, c->d_result, 2 * sizeof(int), cudaMemcpyDeviceToHost, sk));
   SWB_CUDA(cudaStreamSynchronize(sk));
   SWB_CUDA(cudaStreamSynchronize(sc));
@@ -2800,12 +2886,10 @@ static int align_batch_host_ctx(swb200_ctx* c, const HostPairs& h, long long npa
   return SWB200_OK;
 }
 
-extern "C" {
-
-int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, const int* len1, const unsigned char* seq2_all,
-                       const long long* off2, const int* len2, long long npairs, const swb200_params* pp, const swb200_options* opt,
-                       int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride, int* ops_count) {
-  (void)opt;
+// swb200_align_batch / swb200_align_batch_bytes
+static int align_batch_host(const unsigned char* seq1_all, const long long* off1, const int* len1, const unsigned char* seq2_all,
+                            const long long* off2, const int* len2, long long npairs, const swb200_params* pp, AlignKind kind,
+                            int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride, int* ops_count) {
   if (npairs < 0 || ops_stride < 1 ||
       (npairs > 0 && (!seq1_all || !seq2_all || !off1 || !off2 || !len1 || !len2 || !scores_out || !spans_out || !ops_out || !ops_count)))
     return fail(SWB200_ERR_ARG, "bad batch arguments");
@@ -2821,9 +2905,28 @@ int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, con
   return run_host_batch(
       npairs, [&](long long k0, long long k1) { return scan_pairs(in, k0, k1); }, check,
       [&](swb200_ctx* c, long long k0, long long k1, const PairScan& part, const PairScan& whole) {
-        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, AlignKind::batch, 0, 0, scores_out + k0, spans_out + 4 * k0,
+        return align_batch_host_ctx(c, in.from(k0), k1 - k0, part, whole, p, kind, 0, 0, scores_out + k0, spans_out + 4 * k0,
                                     ops_out + k0 * (long long)ops_stride, ops_stride, ops_count + k0);
       });
+}
+
+extern "C" {
+
+int swb200_align_batch(const unsigned char* seq1_all, const long long* off1, const int* len1, const unsigned char* seq2_all,
+                       const long long* off2, const int* len2, long long npairs, const swb200_params* pp, const swb200_options* opt,
+                       int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride, int* ops_count) {
+  (void)opt;
+  return align_batch_host(seq1_all, off1, len1, seq2_all, off2, len2, npairs, pp, AlignKind::batch, scores_out, spans_out, ops_out,
+                          ops_stride, ops_count);
+}
+
+int swb200_align_batch_bytes(const unsigned char* seq1_all, const long long* off1, const int* len1, const unsigned char* seq2_all,
+                             const long long* off2, const int* len2, long long npairs, const swb200_params* pp,
+                             const swb200_options* opt, int* scores_out, int* spans_out, unsigned int* ops_out, int ops_stride,
+                             int* ops_count) {
+  (void)opt;
+  return align_batch_host(seq1_all, off1, len1, seq2_all, off2, len2, npairs, pp, AlignKind::bytes, scores_out, spans_out, ops_out,
+                          ops_stride, ops_count);
 }
 
 int swb200_batch_align(swb200_batch* b, const swb200_params* pp, const swb200_options* opt, void* stream, int* d_scores,
@@ -2869,7 +2972,8 @@ int swb200_batch_align_banded(swb200_batch* b, int band_lo, int band_hi, const s
     return fail(SWB200_ERR_ARG, "bad batch arguments");
   const swb200_params p = params_or_default(pp);
   int rc;
-  if ((rc = check_params(p)) || (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
+  if ((rc = refuse_bytes(b)) || (rc = check_params(p)) ||
+      (rc = check_banded_score(p, b->keep_order, band_lo, band_hi, b->max_short, b->max_long))) return rc;
   return run_device_batch(b, 0, stream, [&](swb200_ctx* c, cudaStream_t s) {
     return align_banded_packed_locked(c, whole_batch(b), band_lo, band_hi - band_lo + 1, p, s, d_scores, d_spans, d_ops, ops_stride,
                                       d_ops_count, &c->info);
@@ -2904,7 +3008,7 @@ int swb200_batch_align_long(swb200_batch* b, const swb200_params* pp, const swb2
   if (b->keep_order || !b->len1) return fail(SWB200_ERR_ARG, "batch was packed in caller order (banded); re-pack with keep_order=0");
   const swb200_params p = params_or_default(pp);
   int rc;
-  if ((rc = check_params(p)) || (rc = check_long_score(p, swb200_options{}, 0, b->max_short))) return rc;
+  if ((rc = refuse_bytes(b)) || (rc = check_params(p)) || (rc = check_long_score(p, swb200_options{}, 0, b->max_short))) return rc;
   return run_device_batch(b, 0, stream, [&](swb200_ctx* c, cudaStream_t s) {
     return align_long_packed_locked(c, whole_batch(b), b->len1, p, s, d_scores, d_spans, d_ops, ops_stride, d_ops_count, &c->info);
   });

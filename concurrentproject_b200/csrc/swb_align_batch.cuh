@@ -27,7 +27,11 @@
 // operations ("1I1I"), which re-score to the score with main.cpp's costs.  For gap_ext <= gap_init the operations are
 // exactly swb200_align's.
 //
-// Every function that runs per pair is SWB_HD, so tests/emu/align_batch_emu.cu runs the same bodies on CPU threads.
+// Symbols are 2-bit codes (A, C, G, T) by default.  With BITS = 8 the same bodies read raw bytes, 8 per 64-bit word
+// (swb_bytes_batch.cu: any byte, compared with == exactly as main.cpp does); the arithmetic does not change.
+//
+// Every function that runs per pair is SWB_HD, so tests/emu/align_batch_emu.cu and tests/emu/bytes_batch_emu.cu run the
+// same bodies on CPU threads.
 #pragma once
 #include "swb_device.cuh"
 
@@ -78,15 +82,20 @@ struct AlignBatchParams {
   unsigned long long* next;
 };
 
-// A view of 2-bit symbols: positions [0, len) of words at off (forward) or of off + len - 1 downwards (reversed).
+// A view of packed symbols: positions [0, len) of words at off (forward) or of off + len - 1 downwards (reversed).
+// align_code<2>: 2-bit codes, 32 per 64-bit word, symbol p at bits 2*(p%32) (the resident batch layout);
+// align_code<8>: bytes, 8 per 64-bit word, byte p at bits 8*(p%8) (the byte batch layout).
 struct AlignSeq {
   const uint64_t* w;
   int off, len;
   bool rev;
 };
+template <int BITS = 2>
 SWB_HD uint32_t align_code(const AlignSeq& s, int p) {
+  static_assert(BITS == 2 || BITS == 8, "2-bit codes or bytes");
   const int a = s.rev ? s.off + s.len - 1 - p : s.off + p;
-  return (uint32_t)(s.w[a >> 5] >> (2 * (a & 31))) & 3u;
+  if constexpr (BITS == 8) return (uint32_t)(s.w[a >> 3] >> (8 * (a & 7))) & 0xFFu;
+  else return (uint32_t)(s.w[a >> 5] >> (2 * (a & 31))) & 3u;
 }
 
 SWB_HD unsigned long long align_atomic_add(unsigned long long* p, unsigned long long v) {
@@ -111,13 +120,16 @@ SWB_HD long long align_dir_words(int lx, int ly) { return (long long)((lx + kAli
 
 // One recurrence over X (T side, columns x = 1..X.len) x Y (Q side, rows y = 1..Y.len).
 //   MODE 0: local (main.cpp:57-63), returns the maximum and its cell;  MODE 1: anchored, the same;
-//   MODE 2: anchored with direction nibbles, returns H at (X.len, Y.len).
+//   MODE 2: anchored with direction nibbles, returns H at (X.len, Y.len);  MODE 3: local, the maximum only (no end cell).
 //   SWP: seq1 is X (the pair was swapped); picks the tie rule's order and which gap is E (consumes seq1) and which F.
-template <int MODE, bool SWP>
+//   BITS: symbol width (align_code).  Columns past X's end read the pad code 1 << BITS, one past the largest symbol, so
+//   they match nothing: with mismatch <= 0 no pad cell exceeds the cells to its left, and MODE 3 need not mask them.
+template <int MODE, bool SWP, int BITS = 2>
 SWB_HD int align_dp(const AlignBatchParams& P, const AlignSeq& X, const AlignSeq& Y, long long tid, uint64_t* dirs,
                     long long dstride, int* bx, int* by) {
   constexpr int S = kAlignStrip;
-  constexpr bool ANCH = MODE >= 1, DIRS = MODE == 2;
+  constexpr bool ANCH = MODE == 1 || MODE == 2, DIRS = MODE == 2;
+  constexpr uint32_t kPad = 1u << BITS;
   const int LX = X.len, LY = Y.len;
   const int gi = P.gap_init, ge = P.gap_ext, gmin = gi < ge ? gi : ge;
   const int ma = P.match, mi = P.mismatch;
@@ -136,13 +148,13 @@ SWB_HD int align_dp(const AlignBatchParams& P, const AlignSeq& X, const AlignSeq
 #pragma unroll
     for (int r = 0; r < S; ++r) {
       const int x = x0 + r + 1;
-      xc[r] = x <= LX ? align_code(X, x - 1) : 4u;
+      xc[r] = x <= LX ? align_code<BITS>(X, x - 1) : kPad;
       hp[r] = ANCH ? -(gi + (x - 1) * gmin) : 0;
       gy[r] = ANCH ? kAlignNeg : 0;
     }
     int hd = col[0].x;                   // H(x0, y-1)
     for (int y = 1; y <= LY; ++y) {
-      const uint32_t yc = align_code(Y, y - 1);
+      const uint32_t yc = align_code<BITS>(Y, y - 1);
       const int2 c = col[y * cs];
       int hleft = c.x, gx = c.y;         // H(x-1, y), gap along T at (x-1, y)
       int hdiag = hd;
@@ -164,6 +176,8 @@ SWB_HD int align_dp(const AlignBatchParams& P, const AlignSeq& X, const AlignSeq
           const bool f_ext = SWP ? gy_ext > gy_open : gx_ext > gx_open;
           const uint32_t src = h == d ? 0u : (h == e ? 1u : 2u);
           dword |= (uint64_t)(src | (e_ext ? 4u : 0u) | (f_ext ? 8u : 0u)) << (4 * r);
+        } else if (MODE == 3) {
+          best = imax2(best, h);
         } else {
           const int x = x0 + r + 1;
           const int j = SWP ? x : y, i = SWP ? y : x;
@@ -187,11 +201,24 @@ SWB_HD int align_dp(const AlignBatchParams& P, const AlignSeq& X, const AlignSeq
       best = hl;
     }
   }
-  if (!DIRS) { *bx = SWP ? bj : bi; *by = SWP ? bi : bj; }
+  if (MODE <= 1) { *bx = SWP ? bj : bi; *by = SWP ? bi : bj; }
   return best;
 }
 
+// Pass 1 without the end cell for pair k: the score only.  Returns the cells computed.
+template <int BITS = 2>
+SWB_HD long long align_score_pair(const AlignBatchParams& P, long long k, long long tid) {
+  const int LQ = P.q_len[k], LT = P.t_len[k];
+  P.scores[k] = 0;
+  if (LQ == 0 || LT == 0) return 0;
+  const AlignSeq X{P.t_words + k * P.t_stride, 0, LT, false}, Y{P.q_words + k * P.q_stride, 0, LQ, false};
+  int unused0 = 0, unused1 = 0;
+  P.scores[k] = align_dp<3, false, BITS>(P, X, Y, tid, nullptr, 0, &unused0, &unused1);
+  return (long long)LQ * LT;
+}
+
 // Passes 1 and 2 for pair k: score and span.  Returns the cells computed.
+template <int BITS = 2>
 SWB_HD long long align_span_pair(const AlignBatchParams& P, long long k, long long tid) {
   const int LQ = P.q_len[k], LT = P.t_len[k];
   const bool swp = P.len1[k] != LQ;
@@ -203,12 +230,12 @@ SWB_HD long long align_span_pair(const AlignBatchParams& P, long long k, long lo
   const uint64_t* tw = P.t_words + k * P.t_stride;
   int xe = 0, ye = 0;
   const AlignSeq X{tw, 0, LT, false}, Y{qw, 0, LQ, false};
-  const int s = swp ? align_dp<0, true>(P, X, Y, tid, nullptr, 0, &xe, &ye) : align_dp<0, false>(P, X, Y, tid, nullptr, 0, &xe, &ye);
+  const int s = swp ? align_dp<0, true, BITS>(P, X, Y, tid, nullptr, 0, &xe, &ye) : align_dp<0, false, BITS>(P, X, Y, tid, nullptr, 0, &xe, &ye);
   P.scores[k] = s;
   if (s <= 0) return (long long)LQ * LT;
   int rx = 0, ry = 0;
   const AlignSeq Xr{tw, 0, xe, true}, Yr{qw, 0, ye, true};
-  const int s2 = swp ? align_dp<1, true>(P, Xr, Yr, tid, nullptr, 0, &rx, &ry) : align_dp<1, false>(P, Xr, Yr, tid, nullptr, 0, &rx, &ry);
+  const int s2 = swp ? align_dp<1, true, BITS>(P, Xr, Yr, tid, nullptr, 0, &rx, &ry) : align_dp<1, false, BITS>(P, Xr, Yr, tid, nullptr, 0, &rx, &ry);
   if (s2 != s) { atomic_or_i32(P.err, kAlignErrStart); return 0; }
   const int xs = xe - rx + 1, ys = ye - ry + 1;
   // seq1/seq2 terms: i in seq2, j in seq1
@@ -218,7 +245,7 @@ SWB_HD long long align_span_pair(const AlignBatchParams& P, long long k, long lo
 
 // The walk over the direction nibbles of a lx x ly rectangle, from its last cell back to (0, 0).  Operations come out
 // last-first; WRITE = false counts them and re-scores, WRITE = true stores them first-first (ops[n - 1 - t]).
-template <bool WRITE>
+template <bool WRITE, int BITS = 2>
 SWB_HD int align_walk(const AlignBatchParams& P, const uint64_t* dirs, long long dstride, const AlignSeq& X, const AlignSeq& Y,
                       bool swp, int n, uint32_t* ops, long long* total) {
   const int LX = X.len, LY = Y.len;
@@ -244,7 +271,7 @@ SWB_HD int align_walk(const AlignBatchParams& P, const uint64_t* dirs, long long
     const uint32_t d = (uint32_t)(dirs[((long long)((x - 1) / kAlignStrip) * LY + (y - 1)) * dstride] >> (4 * ((x - 1) % kAlignStrip))) & 0xFu;
     if (state == 0) {
       const uint32_t src = d & 3u;
-      if (src == 0) { emit(align_code(X, x - 1) == align_code(Y, y - 1) ? kOpEq : kOpX, 1); --x; --y; }
+      if (src == 0) { emit(align_code<BITS>(X, x - 1) == align_code<BITS>(Y, y - 1) ? kOpEq : kOpX, 1); --x; --y; }
       else state = (int)src;
     } else if (state == 1) {                     // E: a base of seq1 against a gap
       emit(kOpIns, 1);
@@ -270,6 +297,7 @@ SWB_HD int align_walk(const AlignBatchParams& P, const uint64_t* dirs, long long
 
 // Pass 3 and the walk for pair k (score and span from align_span_pair).  Returns the cells computed, or -1 if the pair
 // must wait for the next round (pool exhausted).
+template <int BITS = 2>
 SWB_HD long long align_trace_pair(const AlignBatchParams& P, long long k, long long tid) {
   const int s = P.scores[k];
   if (s <= 0) { P.ops_count[k] = 0; return 0; }
@@ -291,15 +319,15 @@ SWB_HD long long align_trace_pair(const AlignBatchParams& P, long long k, long l
   }
   const AlignSeq X{P.t_words + k * P.t_stride, xs - 1, lx, false}, Y{P.q_words + k * P.q_stride, ys - 1, ly, false};
   int unused0 = 0, unused1 = 0;
-  const int h = swp ? align_dp<2, true>(P, X, Y, tid, dirs, dstride, &unused0, &unused1)
-                    : align_dp<2, false>(P, X, Y, tid, dirs, dstride, &unused0, &unused1);
+  const int h = swp ? align_dp<2, true, BITS>(P, X, Y, tid, dirs, dstride, &unused0, &unused1)
+                    : align_dp<2, false, BITS>(P, X, Y, tid, dirs, dstride, &unused0, &unused1);
   const long long cells = (long long)lx * ly;
   if (h != s) { atomic_or_i32(P.err, kAlignErrTrace); P.ops_count[k] = 0; return cells; }
   long long total = 0;
-  const int n = align_walk<false>(P, dirs, dstride, X, Y, swp, 0, nullptr, &total);
+  const int n = align_walk<false, BITS>(P, dirs, dstride, X, Y, swp, 0, nullptr, &total);
   if (total != s) { atomic_or_i32(P.err, kAlignErrRescore); P.ops_count[k] = 0; return cells; }
   if (n > P.ops_stride) { P.ops_count[k] = -n; return cells; }
-  align_walk<true>(P, dirs, dstride, X, Y, swp, n, P.ops + k * (long long)P.ops_stride, &total);
+  align_walk<true, BITS>(P, dirs, dstride, X, Y, swp, n, P.ops + k * (long long)P.ops_stride, &total);
   P.ops_count[k] = n;
   return cells;
 }
@@ -325,5 +353,10 @@ __global__ void __launch_bounds__(256) align_trace_kernel(const __grid_constant_
 // host launchers (swb_align_batch.cu); blocks x 256 threads must equal P.nthreads
 void launch_align_span(const AlignBatchParams& P, int blocks, cudaStream_t s);
 void launch_align_trace(const AlignBatchParams& P, int blocks, cudaStream_t s);
+// the byte layout (swb_bytes_batch.cu): the same passes with align_code<8>, and pass 1 alone for scores
+void launch_bytes_span(const AlignBatchParams& P, int blocks, cudaStream_t s);
+void launch_bytes_trace(const AlignBatchParams& P, int blocks, cudaStream_t s);
+void launch_bytes_score(const AlignBatchParams& P, int blocks, cudaStream_t s);
+const void* bytes_score_kernel_ptr();
 
 }  // namespace swb

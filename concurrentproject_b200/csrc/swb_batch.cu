@@ -106,4 +106,42 @@ void launch_pack_batch(const uint8_t* seq1, const long long* off1, const int* le
                                            q_len, t_len, keep_order, status);
 }
 
+// Packs a byte batch (swb_bytes_batch.cu): the shorter sequence of every pair becomes Q, the longer one T, both as raw
+// bytes, 8 per 64-bit word (byte p at bits 8*(p%8)), fixed word strides per pair.  Every byte is kept as it is: no
+// check, no remapping.  One thread per output word.
+__global__ void pack_bytes_kernel(const uint8_t* __restrict__ seq1, const long long* __restrict__ off1,
+                                  const int* __restrict__ len1, const uint8_t* __restrict__ seq2,
+                                  const long long* __restrict__ off2, const int* __restrict__ len2, long long npairs,
+                                  long long q_stride, long long t_stride, uint64_t* __restrict__ q_words,
+                                  uint64_t* __restrict__ t_words, int* __restrict__ q_len, int* __restrict__ t_len) {
+  const long long per_pair = q_stride + t_stride;
+  const long long total = npairs * per_pair;
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
+       idx += (long long)gridDim.x * blockDim.x) {
+    const long long pair = idx / per_pair;
+    const long long wi = idx - pair * per_pair;
+    const int l1 = len1[pair], l2 = len2[pair];
+    const bool swap = l1 > l2;
+    const uint8_t* q = swap ? seq2 + off2[pair] : seq1 + off1[pair];
+    const uint8_t* t = swap ? seq1 + off1[pair] : seq2 + off2[pair];
+    const int lq = swap ? l2 : l1, lt = swap ? l1 : l2;
+    const bool is_q = wi < q_stride;
+    const uint8_t* src = is_q ? q : t;
+    const int len = is_q ? lq : lt;
+    const long long w = is_q ? wi : wi - q_stride;
+    uint64_t out = 0;
+    const long long base = w * 8;
+    for (int k = 0; k < 8 && base + k < len; ++k) out |= (uint64_t)src[base + k] << (8 * k);
+    if (is_q) q_words[pair * q_stride + w] = out; else t_words[pair * t_stride + w] = out;
+    if (wi == 0) { q_len[pair] = lq; t_len[pair] = lt; }
+  }
+}
+
+void launch_pack_bytes(const uint8_t* seq1, const long long* off1, const int* len1, const uint8_t* seq2,
+                       const long long* off2, const int* len2, long long npairs, long long q_stride, long long t_stride,
+                       uint64_t* q_words, uint64_t* t_words, int* q_len, int* t_len, int blocks, cudaStream_t s) {
+  pack_bytes_kernel<<<blocks, 256, 0, s>>>(seq1, off1, len1, seq2, off2, len2, npairs, q_stride, t_stride, q_words, t_words,
+                                           q_len, t_len);
+}
+
 }  // namespace swb

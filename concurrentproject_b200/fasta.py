@@ -9,14 +9,16 @@ to the GPU kernels:
                          lanes per pair, swb_batch.cuh) and orders each bucket by the longer length, so the
                          pairs a warp scores side by side stream about the same number of columns;
 * ``score_pairs``     -- scores pair k = (seqs1[k], seqs2[k]) for ragged inputs: ACGT pairs whose shorter side
-                         is <= 1024 go bucket by bucket through the batch kernel (swb200_score_batch), longer ACGT
+                         is <= 1024 go bucket by bucket through the batch kernel (swb200_score_batch), pairs with
+                         other bytes (N, IUPAC codes, amino acids) and the same limits through the byte batch
+                         (swb200_batch_pack_device_bytes), which compares bytes exactly like main.cpp:60, longer ACGT
                          pairs, when the batch beats one call per pair (long_batch_pays), through the multi-band
-                         batch kernel (swb200_batch_score_long), everything else (a few long pairs, or other
-                         alphabets such as N or amino acids) through the single-pair engine (swb200_score_ex), which compares bytes
-                         exactly like main.cpp:60;
+                         batch kernel (swb200_batch_score_long), everything else (a few long pairs, long pairs with
+                         other bytes) through the single-pair engine (swb200_score_ex);
 * ``search``          -- one query against every record of a database;
-* ``align_pairs``     -- score, span and CIGAR of (seqs1[k], seqs2[k]), each as api.align returns it: ACGT pairs whose
-                         shorter side is <= 1024 through the batch alignment (swb200_batch_align), longer ACGT pairs,
+* ``align_pairs``     -- score, span and CIGAR of (seqs1[k], seqs2[k]), each as api.align returns it: pairs whose
+                         shorter side is <= 1024 through the batch alignment (swb200_batch_align; pairs with other
+                         bytes than A,C,G,T on a byte batch), longer ACGT pairs,
                          when the batch beats one call per pair (align_long_batch_pays), through the long-pair batch
                          alignment (swb200_batch_align_long), everything else pair by pair (swb200_align_device).
 
@@ -120,8 +122,9 @@ def write_fasta(path: str, names: Sequence[str], seqs: Sequence[bytes], width: i
 @dataclass
 class Bucket:
     kind: str            # "batch": one swb200_score_batch call; "long": one swb200_batch_score_long call;
+                         # "bytes": one call on a byte batch (swb200_batch_pack_device_bytes);
                          # "single": one swb200_score_ex call per pair
-    cap: int             # capacity class of the shorter side (0 for "single")
+    cap: int             # capacity class of the shorter side (0 for "long", "bytes" and "single")
     index: np.ndarray    # pair ids, in the order they are handed to the kernel
 
 
@@ -160,13 +163,17 @@ def plan_buckets(len1: np.ndarray, len2: np.ndarray, acgt_only: np.ndarray, min_
     order, so the longest pairs start first), when that call beats the single-pair engine (long_batch_pays).  Pairs the 16-bit batch
     kernels cannot hold (match * min(len) > 32766 - match, swb200.cu: check_batch_score) go to the single-pair engine,
     which re-runs in re-based or 32-bit lanes by itself.  ``pays`` judges the "long" bucket: long_batch_pays for
-    scoring, align_long_batch_pays for alignment."""
+    scoring, align_long_batch_pays for alignment.  Pairs that are not ``acgt_only`` but within the batch limits form one
+    "bytes" bucket, ordered like a batch bucket (a byte batch has one kernel for every shorter side up to 1024)."""
     len1 = np.asarray(len1, dtype=np.int64)
     len2 = np.asarray(len2, dtype=np.int64)
     short = np.minimum(len1, len2)
     long_ = np.maximum(len1, len2)
-    in_range = np.asarray(acgt_only, dtype=bool) & (int(match) * short <= 32766 - int(match))
+    acgt = np.asarray(acgt_only, dtype=bool)
+    fits16 = int(match) * short <= 32766 - int(match)
+    in_range = acgt & fits16
     batchable = in_range & (short <= BATCH_MAX_SHORT)
+    byte_ids = np.flatnonzero(~acgt & fits16 & (short <= BATCH_MAX_SHORT))
     long_ids = np.flatnonzero(in_range & (short > BATCH_MAX_SHORT))
     if not pays(short[long_ids], long_[long_ids]):
         long_ids = long_ids[:0]
@@ -191,8 +198,11 @@ def plan_buckets(len1: np.ndarray, len2: np.ndarray, acgt_only: np.ndarray, min_
         band = 64 * 16                                             # the default band height of the tallest pairs
         padded = (-(-short[long_ids] // band) * band) * (long_[long_ids] + 63)
         out.append(Bucket("long", 0, long_ids[np.argsort(-padded, kind="stable")]))
+    if byte_ids.size:
+        out.append(Bucket("bytes", 0, byte_ids[np.argsort(-long_[byte_ids], kind="stable")]))
     routed = batchable.copy()
     routed[long_ids] = True
+    routed[byte_ids] = True
     rest = np.flatnonzero(~routed)
     if rest.size:
         out.append(Bucket("single", 0, rest))
@@ -237,7 +247,7 @@ def score_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
                   params: Sequence[int] = api.DEFAULT_PARAMS, *, min_bucket: int = 512, device: int = 0) -> np.ndarray:
     """Score pair k = (a[ia[k]], b[ib[k]]) for index arrays ia, ib.  Returns int32 scores in pair order.
     The residues go to HBM once; every bucket then only ships its offsets and lengths and is packed and scored
-    in place (swb200_batch_pack_device / swb200_batch_score)."""
+    in place (swb200_batch_pack_device / swb200_batch_score; the "bytes" bucket on a byte batch)."""
     import torch
     ia = np.asarray(ia, dtype=np.int64)
     ib = np.asarray(ib, dtype=np.int64)
@@ -259,7 +269,7 @@ def score_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
         stream = torch.cuda.current_stream(dev).cuda_stream
         for bk in buckets:
             ids = bk.index
-            if bk.kind in ("batch", "long"):
+            if bk.kind in ("batch", "long", "bytes"):
                 bl1, bl2 = l1[ids], l2[ids]
                 d_o1 = torch.from_numpy(o1[ids]).to(dev); d_o2 = torch.from_numpy(o2[ids]).to(dev)
                 d_l1 = torch.from_numpy(bl1).to(dev); d_l2 = torch.from_numpy(bl2).to(dev)
@@ -267,7 +277,8 @@ def score_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
                 short, long_ = np.minimum(bl1, bl2), np.maximum(bl1, bl2)
                 cells = int((bl1.astype(np.int64) * bl2).sum())
                 pb = api.PackedBatch(ctx, fa.data_ptr(), d_o1.data_ptr(), d_l1.data_ptr(), fb.data_ptr(), d_o2.data_ptr(),
-                                     d_l2.data_ptr(), len(ids), int(short.max()), int(long_.max()), cells, stream=stream)
+                                     d_l2.data_ptr(), len(ids), int(short.max()), int(long_.max()), cells, stream=stream,
+                                     byte_symbols=bk.kind == "bytes")
                 try:
                     if bk.kind == "long":
                         pb.score_long(d_sc.data_ptr(), params, stream=stream)
@@ -291,10 +302,10 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
                   ops_stride: int = api.OPS_STRIDE):
     """Align pair k = (a[ia[k]], b[ib[k]]): (scores int32[n], spans int32[n, 4], cigars list[str]) in pair order, each
     as api.align returns it.  The buckets of score_records, with the long bucket judged by align_long_batch_pays: batch
-    buckets are packed in place and aligned by swb200_batch_align, the long bucket by swb200_batch_align_long (pairs
-    that need more than ops_stride, or api.LONG_OPS_STRIDE, operations once more with room for len1 + len2); the rest
-    (bytes other than A,C,G,T, long pairs where the batch does not pay, pairs whose span could not get direction
-    storage) pair by pair through swb200_align_device."""
+    buckets are packed in place and aligned by swb200_batch_align, the bytes bucket on a byte batch by the same call, the
+    long bucket by swb200_batch_align_long (pairs that need more than ops_stride, or api.LONG_OPS_STRIDE, operations once
+    more with room for len1 + len2); the rest (long pairs with bytes other than A,C,G,T, long pairs where the batch does
+    not pay, pairs whose span could not get direction storage) pair by pair through swb200_align_device."""
     import torch
     ia = np.asarray(ia, dtype=np.int64)
     ib = np.asarray(ib, dtype=np.int64)
@@ -323,7 +334,7 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
         buckets = plan_buckets(l1, l2, ok_a[ia] & ok_b[ib] & fits, min_bucket, match=int(params[0]), pays=align_long_batch_pays)
         stream = torch.cuda.current_stream(dev).cuda_stream
 
-        def run(ids, stride, long_pairs=False):
+        def run(ids, stride, long_pairs=False, byte_symbols=False):
             bl1, bl2 = l1[ids], l2[ids]
             d_o1 = torch.from_numpy(o1[ids]).to(dev); d_o2 = torch.from_numpy(o2[ids]).to(dev)
             d_l1 = torch.from_numpy(bl1).to(dev); d_l2 = torch.from_numpy(bl2).to(dev)
@@ -334,7 +345,8 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
             short, long_ = np.minimum(bl1, bl2), np.maximum(bl1, bl2)
             cells = int((bl1.astype(np.int64) * bl2).sum())
             pb = api.PackedBatch(ctx, fa.data_ptr(), d_o1.data_ptr(), d_l1.data_ptr(), fb.data_ptr(), d_o2.data_ptr(),
-                                 d_l2.data_ptr(), len(ids), int(short.max()), int(long_.max()), cells, stream=stream)
+                                 d_l2.data_ptr(), len(ids), int(short.max()), int(long_.max()), cells, stream=stream,
+                                 byte_symbols=byte_symbols)
             try:
                 align = pb.align_long if long_pairs else pb.align
                 align(d_sc.data_ptr(), d_sp.data_ptr(), d_ops.data_ptr(), stride, d_cnt.data_ptr(), params, stream=stream)
@@ -344,9 +356,9 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
 
         for bk in buckets:
             ids = bk.index
-            if bk.kind in ("batch", "long"):
-                lp = bk.kind == "long"
-                sc, sp, ops, cnt = run(ids, api.LONG_OPS_STRIDE if lp else ops_stride, lp)
+            if bk.kind in ("batch", "long", "bytes"):
+                lp, by = bk.kind == "long", bk.kind == "bytes"
+                sc, sp, ops, cnt = run(ids, api.LONG_OPS_STRIDE if lp else ops_stride, lp, by)
                 scores[ids] = sc
                 spans[ids] = sp
                 for r, pid in enumerate(ids.tolist()):
@@ -354,7 +366,7 @@ def align_records(a: FastaRecords, ia: np.ndarray, b: FastaRecords, ib: np.ndarr
                         cigars[pid] = api.cigar_string(ops[r, :cnt[r]])
                 redo = ids[cnt < 0]
                 if len(redo):
-                    _, _, ops2, cnt2 = run(redo, int((l1[redo].astype(np.int64) + l2[redo]).max()), lp)
+                    _, _, ops2, cnt2 = run(redo, int((l1[redo].astype(np.int64) + l2[redo]).max()), lp, by)
                     for r, pid in enumerate(redo.tolist()):
                         cigars[pid] = api.cigar_string(ops2[r, :cnt2[r]])
             else:

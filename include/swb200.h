@@ -285,6 +285,33 @@ SWB200_API int swb200_align_batch(const unsigned char* seq1_all, const long long
 SWB200_API int swb200_batch_align(swb200_batch* batch, const swb200_params* p, const swb200_options* opt, void* stream,
                                   int* d_scores, int* d_spans, unsigned int* d_ops, int ops_stride, int* d_ops_count);
 
+/* ---- byte batches: read batches in any bytes (N, IUPAC codes, lower case, amino acids) ---------------------------------
+ * swb200_score_batch and swb200_align_batch for pairs whose bytes are not all A,C,G,T.  For every pair k the score, span
+ * and operations are exactly those swb200_score / swb200_align return for that pair alone: symbols compare as raw bytes
+ * (main.cpp:28-33), so N matches N and 'a' does not match 'A'.  The batch-alignment rules of swb200_align_batch hold as
+ * they are: ops format, ops_count = -n on overflow, the "1I1I" split when gap_ext > gap_init, the device re-score.  On
+ * A,C,G,T input the outputs equal swb200_score_batch's / swb200_align_batch's.  One thread per pair, 32-bit arithmetic
+ * (DESIGN.md section 4g).  Limits are swb200_align_batch's: min(len1,len2) <= 1024 (SWB200_ERR_ARG) and
+ * match*min(len) <= 32766 - match (SWB200_ERR_RANGE); no byte value is refused (these calls never return
+ * SWB200_ERR_ALPHABET).  All checks run before a device is touched.  The host calls copy and pack in chunks and shard
+ * over swb200_set_devices (results identical for every G).  opt is reserved (NULL).  swb200_last_run: lanes 32, config
+ * 101 for scoring and 301 for alignment. */
+SWB200_API int swb200_score_batch_bytes(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                                        const unsigned char* seq2_all, const long long* off2, const int* len2,
+                                        long long npairs, const swb200_params* p, const swb200_options* opt,
+                                        int* scores_out);
+SWB200_API int swb200_align_batch_bytes(const unsigned char* seq1_all, const long long* off1, const int* len1,
+                                        const unsigned char* seq2_all, const long long* off2, const int* len2,
+                                        long long npairs, const swb200_params* p, const swb200_options* opt, int* scores_out,
+                                        int* spans_out, unsigned int* ops_out, int ops_stride, int* ops_count);
+/* The device-resident byte batch: swb200_batch_pack_device with keep_order = 0, the bytes kept as they are (8 per 64-bit
+ * word).  swb200_batch_score and swb200_batch_align take it and run the byte kernels; swb200_batch_score_long,
+ * swb200_batch_score_banded, swb200_batch_align_banded and swb200_batch_align_long refuse it with SWB200_ERR_ARG. */
+SWB200_API int swb200_batch_pack_device_bytes(swb200_ctx* ctx, const unsigned char* d_seq1_all, const long long* d_off1,
+                                              const int* d_len1, const unsigned char* d_seq2_all, const long long* d_off2,
+                                              const int* d_len2, long long npairs, int max_short, int max_long,
+                                              long long total_cells, void* stream, swb200_batch** batch_out);
+
 /* Batch alignment without the 1024 cap: for every pair k the score, span and operations that swb200_align returns for
  * that pair alone, with swb200_align_batch's tie rules, output format, ops_stride overflow rule (ops_count = -n; the host
  * call zero-fills that slot), "1I1I" split when gap_ext > gap_init (the one documented difference from swb200_align) and
